@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the fused drone-navigation control step on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): step-only throughput, 4096 CF2X envs per GPU, DYN physics,
 240 Hz physics / 30 Hz control (S = 8 substeps fused per launch), circle track, THRUST actions with
@@ -43,6 +43,24 @@ METRIC = "env-steps/sec (fused substeps)"
 UNIT = "env-steps/s"
 BYTES_PER_ENV_STEP = 16 + 112 + 112 + 52 + 4 + 1 + 4   # action | state in | state out | obs | reward | done | found  (DESIGN.md)
 HOVER = 0.092227
+DUMP_LIMIT = 64 << 20                   # bytes, all files of --dump-outputs together
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """--dump-outputs: each [N, ...] array of `arrays` as out_dir/<name>.npy, float32 kept, every other dtype as float64
+    (exact for the integer outputs).  If they would take more than `limit` bytes together, the same fixed, seeded sample
+    of rows is written of each, and the sampled row numbers as env_index.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes > limit - 4096:                    # 4 KiB for the .npy headers
+        rows = (limit - 4096) // (row_bytes + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, size=rows, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def track_setup(track: str):
@@ -315,13 +333,13 @@ def time_flushed(env, acts, K, W, flush_buf):
     return float(per.sum()) * 1e-3, per
 
 
-def time_rotating(args, dev, N, K, W, rank, n_handles=None, on_timed=None, min_timed_s=0.02):
+def time_rotating(args, dev, N, K, W, rank, n_handles=None, on_timed=None, want_outputs=False):
     """`inputs larger than L2`: M independent N-env handles (state + actions + outputs of all of them > 126 MB L2) are
-    stepped round-robin, one launch per handle, replayed from CUDA graphs on one stream.  The unit that is timed is a
-    block of EXACTLY K launches; when K launches are shorter than `min_timed_s` the block is repeated R times inside the
-    one CUDA-event pair (successive blocks continue the rotation, so every launch still finds its state, its actions and
-    its output lines in HBM, not in L2) and the mean over the R blocks is reported.  Every graph that is replayed inside
-    the timed region has been replayed once before it (a first replay pays the graph upload)."""
+    stepped round-robin, one launch per handle, replayed from CUDA graphs on one stream.  The timed region is EXACTLY K
+    launches inside one CUDA-event pair.  Right before it the graphs that precede it in the rotation are replayed, untimed:
+    that leaves each timed launch's state, actions and output lines in HBM rather than in L2.  How often each handle has
+    been stepped depends on the arguments alone, so the outputs of the last timed launch are the same from run to run;
+    with `want_outputs` they are returned as numpy arrays (what `env.step` hands its caller)."""
     import torch
     per_handle = N * (BYTES_PER_ENV_STEP - 112)          # state planes once + actions + outputs, bytes resident per handle
     M = n_handles or max(8, int(np.ceil(160e6 / per_handle)))
@@ -334,16 +352,16 @@ def time_rotating(args, dev, N, K, W, rank, n_handles=None, on_timed=None, min_t
     s = torch.cuda.Stream(device=dev)
     s.wait_stream(torch.cuda.current_stream(dev))
     with torch.cuda.stream(s):
-        for _ in range(max(3, -(-W // M))):              # >= W untimed warm-up steps (whole rotations)
+        for _ in range(max(24, -(-W // M))):             # >= W untimed warm-up steps (whole rotations), >= 24 per handle:
+                                                         # episodes are de-phased (steady-state reset mix), as in the sweep
             for m, e in enumerate(envs):
                 e.step(acts[m])
     torch.cuda.current_stream(dev).wait_stream(s)
     torch.cuda.synchronize()
-    # the K launches of block b are handles (b*K + j) % M, j < K.  Graphs: one per distinct starting handle; the list of
-    # starting handles is periodic with period M / gcd(K, M), capped so that capture stays cheap (the cap only shortens
-    # the rotation: with >= 160 MB in flight per period it stays larger than L2 whenever n_period * K >= M)
-    period = M // int(np.gcd(K, M))
-    n_graphs = max(1, M // K) if K < M else min(period, 4)   # K < M: whole blocks of one rotation (>= 126 MB before any reuse)
+    # graph b holds the K launches of handles (b*K + j) % M, j < K: the graphs continue one rotation, so every launch of
+    # the last (timed) graph finds its handle last stepped M launches earlier (> 126 MB ago).  At least two graphs: one
+    # graph replayed twice would bring some handles back after fewer than M launches unless M divides K
+    n_graphs = max(2, -(-M // K))
     graphs = []
     for b in range(n_graphs):
         g = torch.cuda.CUDAGraph()
@@ -352,32 +370,28 @@ def time_rotating(args, dev, N, K, W, rank, n_handles=None, on_timed=None, min_t
                 m = (b * K + j) % M
                 envs[m].step(acts[m])
         graphs.append(g)
-    for g in graphs:                                     # first replay of every graph outside the timed region
-        g.replay()
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    graphs[0].replay()
-    e1.record()
-    torch.cuda.synchronize()
-    est = max(e0.elapsed_time(e1) * 1e-3, 1e-6)          # one block, to size R
-    R = int(max(1, min(100000, np.ceil(min_timed_s / est))))
     if on_timed:
         on_timed(True)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for g in graphs[:-1]:                                # untimed, not synchronised: the timed replay queues behind them
+        g.replay()
     e0.record()
-    for r in range(R):
-        graphs[r % n_graphs].replay()
+    graphs[-1].replay()
     e1.record()
     torch.cuda.synchronize()
     if on_timed:
         on_timed(False)
-    total = e0.elapsed_time(e1) * 1e-3
+    sec = e0.elapsed_time(e1) * 1e-3
+    last = None
+    if want_outputs:                                     # env.step returns views of these persistent output tensors
+        e = envs[(n_graphs * K - 1) % M]
+        last = {k: getattr(e, k).cpu().numpy() for k in ("obs", "reward", "done", "found_targets")}
     eps = sum(int(e.episode_stats()["episodes"]) for e in envs[:4])
     for e in envs:
         e.close()
     del envs, acts, graphs
     torch.cuda.empty_cache()
-    return total / R, K, M, per_handle * M, eps, R, total, n_graphs
+    return sec, K, M, per_handle * M, eps, n_graphs, last
 
 
 def time_launch_floor(env, K, flush_buf):
@@ -621,11 +635,8 @@ def run_b200(args):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    import __graft_entry__ as ge
-    if rank == 0:
-        ge.build()
-    if world > 1:
-        dist.barrier()
+    from drl_dronenavigation_b200 import _lib
+    _lib.lib()             # the library build() left in the tree: nothing is compiled here, nothing is written there
     K, W = args.steps, max(args.warmup, 3)
     N = args.envs
 
@@ -659,13 +670,14 @@ def run_b200(args):
     def around_timed(start):          # barrier + synchronize on both sides of the timed region, on every rank
         barrier()
         win["t0" if start else "t1"] = time.time()
-    sec, k_r, m_r, bytes_r, eps_r, reps, timed_s, n_graphs = time_rotating(args, dev, N, K, W, rank, n_handles=args.rotating_handles,
-                                                                           on_timed=around_timed)
+    sec, k_r, m_r, bytes_r, eps_r, n_graphs, last = time_rotating(args, dev, N, K, W, rank, n_handles=args.rotating_handles,
+                                                                  on_timed=around_timed, want_outputs=bool(args.dump_outputs))
     assert k_r == K
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     barrier()
     sec = max_over_ranks(sec)
     value = world * N * K / sec
-    launches = K * reps
     l2_note = ("PROFILING RUN with a reduced number of handles (L2-resident): " if args.rotating_handles else "") + \
               (f"inputs larger than L2: {m_r} independent {N}-env handles = {bytes_r / 1e6:.0f} MB of state + actions + outputs "
                "(> 126 MB L2) stepped round-robin from CUDA graphs on one stream, so every launch reads its inputs from HBM; "
@@ -694,13 +706,13 @@ def run_b200(args):
             "ms_per_step": 1e3 * sec / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic",
             "config": bench_config(args, world),
-            "reps": reps, "timed_region_s": timed_s,
-            "timing": {"l2": l2_note, "handles": m_r, "graphs": n_graphs, "launches_per_graph": K, "reps": reps,
-                       "timed_region_s": timed_s, "launches_in_timed_region": K * reps,
-                       "note": "ms_per_step = timed_region_s / (reps * steps): the K-launch block is repeated `reps` times inside ONE "
-                               "CUDA-event pair because K launches alone are shorter than 20 ms; every replayed graph is warmed first"},
+            "timed_region_s": sec,
+            "timing": {"l2": l2_note, "handles": m_r, "graphs": n_graphs, "launches_per_graph": K,
+                       "timed_region_s": sec, "launches_in_timed_region": K,
+                       "note": "ms_per_step = timed_region_s / steps: exactly `steps` launches (one graph replay) inside ONE "
+                               "CUDA-event pair; the graphs before it in the rotation are replayed right before it"},
             "physics_steps_per_s": value * args.substeps,
-            "clocks": clocks, "gpu_launches": int(launches), "l2_resident": resident, "flushed_event_bracket": flushed,
+            "clocks": clocks, "gpu_launches": K, "l2_resident": resident, "flushed_event_bracket": flushed,
             "episodes_finished_sample": eps_r}
 
     # ---- single-GPU extras on rank 0 only: roofline, sweep, e2e, cpu baseline --------------------
@@ -925,6 +937,7 @@ def run_b200(args):
 
 
 def main():
+    sys.dont_write_bytecode = True      # the tree may be read-only: the modules imported from it leave no __pycache__ there
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=1000)
@@ -955,7 +968,12 @@ def main():
                          "the ncu launch-list pass uses a small number so that the capture window covers the timed region)")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-BASELINE-config step-only lines")
     ap.add_argument("--cpu-budget", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write obs, reward, done and found_targets of the last timed step (the handle it stepped) as DIR/<name>.npy; "
+                         "the inputs depend on the arguments only, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs: only the GPU arm (--impl b200) writes its outputs")
     if args.impl == "reference":
         run_reference(args)
     else:

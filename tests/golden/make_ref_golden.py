@@ -1,10 +1,10 @@
-"""Mints ``tests/golden/ref_*.npz`` by stepping the REFERENCE'S OWN code (imported unmodified from
-``/root/reference``), so that the oracle restatement and the CUDA path are pinned against what the
+"""Mints ``tests/golden/ref_*.npz`` by stepping the REFERENCE'S OWN code (imported unmodified from a checkout of
+eRGiBi/DRL-DroneNavigation named by $DN_REFERENCE_ROOT), so that the oracle restatement and the CUDA path are pinned against what the
 reference computes rather than against our reading of it.
 
-Run (in the build container only -- /root/reference does not exist on the GPU box):
+Run (only the committed ``.npz`` fixtures are part of this repository, not that checkout):
 
-    python tests/golden/make_ref_golden.py
+    DN_REFERENCE_ROOT=<checkout> python tests/golden/make_ref_golden.py
 
 What executes: ``Sol.Model.Environments.PBDroneEnv.PBDroneEnv`` (``step``, ``reset``, ``rescale_action``,
 ``_preprocessAction``, ``_computeObs``, ``_clipAndNormalizeState``, ``_computeReward``, ``orientation_reward``,
@@ -41,7 +41,8 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("DN_REFERENCE_ROOT", "")          # a checkout of the original project; tests that re-run it skip without one
+HAVE_REF = bool(REF) and os.path.isdir(os.path.join(REF, "Sol"))
 HOVER = 0.092227
 
 CASES = {
@@ -441,6 +442,8 @@ def mint_forces(ref, n_rollout=40, seed=77):
 
 
 if __name__ == "__main__":
+    if not HAVE_REF:
+        sys.exit("DN_REFERENCE_ROOT must name a checkout of eRGiBi/DRL-DroneNavigation")
     ref = _import_reference()
     np.savez_compressed(os.path.join(HERE, "forces_ref.npz"), **mint_forces(ref))
     print("HoverAviary imported from the reference:", ref[-1], file=sys.stderr)

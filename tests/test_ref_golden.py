@@ -1,7 +1,7 @@
 """Fixtures minted from the REFERENCE'S OWN CODE (tests/golden/ref_*.npz; generator tests/golden/make_ref_golden.py
-imports /root/reference unmodified behind import shims for the absent third-party packages).
+imports the original project unmodified behind import shims for the absent third-party packages).
 
- - not gpu: (1) if /root/reference is present (build container), the generator still reproduces the committed
+ - not gpu: (1) if a checkout of the original project is present (make_ref_golden.REF), the generator still reproduces the committed
             fixtures bit for bit; (2) the oracle restatement matches them to FP64 round-off
             (obs: identical float32 values; reward 1e-12; done bits / found_targets / Monitor lengths exact);
             (3) the host build of the device step logic matches them within the stated FP32 tolerances.
@@ -13,11 +13,10 @@ import os
 import numpy as np
 import pytest
 
-from tests.golden.make_ref_golden import CASES
+from tests.golden.make_ref_golden import CASES, HAVE_REF
 
 GOLD = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "ref_*.npz")))
 IDS = [os.path.basename(p)[:-4] for p in GOLD]
-HAVE_REF = os.path.isdir("/root/reference/Sol")
 
 
 REWARD_IDS = {"default": 0, "dummy": 1, "thrustenv": 2, "her": 3, "reaching": 4, "progress": 5, "hover": 6, "flythrugate": 7,
@@ -41,7 +40,7 @@ def test_fixtures_exist():
     assert sorted(IDS) == sorted(CASES)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference only exists in the build container")
+@pytest.mark.skipif(not HAVE_REF, reason="needs a checkout of the original project (DN_REFERENCE_ROOT)")
 def test_reference_reproduces_fixtures():
     """Re-runs the reference for a few of the cases (each one exercises every function on the path)."""
     import subprocess

@@ -13,8 +13,10 @@ import os
 import numpy as np
 import pytest
 
+from tests.golden.make_ref_golden import HAVE_REF, REF
+
 HERE = os.path.dirname(os.path.abspath(__file__))
-HAVE_REF = os.path.isdir("/root/reference/Sol")
+ARCHIVE = os.path.join(REF, "Sol", "pyfly", "ppo_quadx_waypoints.zip")
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -58,7 +60,7 @@ def test_oracle_drag_and_ground_effect_match_the_references_functions():
         np.testing.assert_allclose(env._ground_effect(g["rpm"][i], R), g["gnd_force_z"][i], rtol=1e-12, atol=1e-18)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference only exists in the build container")
+@pytest.mark.skipif(not HAVE_REF, reason="needs a checkout of the original project (DN_REFERENCE_ROOT)")
 def test_force_fixture_is_reproduced_by_the_reference():
     import subprocess
     import sys
@@ -122,8 +124,8 @@ MANIFEST = os.path.join(HERE, "golden", "ppo_quadx_waypoints_manifest.json")
 
 
 def test_sb3_archive_manifest_loads_into_a_learner():
-    """Key / shape manifest of /root/reference/Sol/pyfly/ppo_quadx_waypoints.zip::policy.pth (committed: the archive itself
-    does not travel): a learner with that architecture accepts exactly those keys and shapes through the SB3 name map."""
+    """Key / shape manifest of the original project's Sol/pyfly/ppo_quadx_waypoints.zip::policy.pth (committed: the archive
+    itself is not part of this repository): a learner with that architecture accepts exactly those keys and shapes through the SB3 name map."""
     import torch
     from drl_dronenavigation_b200.checkpoint import policy_to_sb3_state_dict, sb3_state_dict_to_policy
     from drl_dronenavigation_b200.ppo import PPOConfig, PPOLearner
@@ -136,7 +138,7 @@ def test_sb3_archive_manifest_loads_into_a_learner():
     assert all(float(p.detach().min()) == 0.25 for p in L.policy.parameters())
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/Sol/pyfly/ppo_quadx_waypoints.zip"), reason="the archive only exists in the build container")
+@pytest.mark.skipif(not os.path.exists(ARCHIVE), reason="needs the original project's SB3 archive (DN_REFERENCE_ROOT)")
 def test_reference_sb3_archive_loads():
     """The archive SB3 itself wrote (members data, policy.pth, policy.optimizer.pth, pytorch_variables.pth, ...)."""
     import io
@@ -144,7 +146,7 @@ def test_reference_sb3_archive_loads():
     import torch
     from drl_dronenavigation_b200.checkpoint import load_sb3_zip, policy_to_sb3_state_dict
     from drl_dronenavigation_b200.ppo import PPOConfig, PPOLearner
-    path = "/root/reference/Sol/pyfly/ppo_quadx_waypoints.zip"
+    path = ARCHIVE
     man = json.load(open(MANIFEST))
     with zipfile.ZipFile(path) as zf:
         assert {"data", "policy.pth", "policy.optimizer.pth", "pytorch_variables.pth"} <= set(zf.namelist())
