@@ -194,13 +194,19 @@ class FusedUpdate:
     the eager torch path and the kernels all see the same memory."""
 
     @staticmethod
+    def shapes_ok(pi_arch, vf_arch, obs_dim: int, act_dim: int) -> bool:
+        """The shapes dn_ppo_create accepts: 1..4 hidden layers per network, every hidden width a multiple of 128 between 128
+        and 512 (the column-sum accumulator of the bias gradients holds 512 columns), 1 <= obs_dim <= 64, act_dim in (1, 3, 4)."""
+        widths = tuple(pi_arch) + tuple(vf_arch)
+        return (1 <= len(pi_arch) <= 4 and 1 <= len(vf_arch) <= 4 and all(w % 128 == 0 and 128 <= w <= 512 for w in widths)
+                and 1 <= obs_dim <= 64 and act_dim in (1, 3, 4))
+
+    @staticmethod
     def supported(cfg: "PPOConfig", obs_dim: int, act_dim: int, device) -> bool:
         dev = torch.device(device)
         if dev.type != "cuda" or torch.cuda.get_device_capability(dev)[0] != 10:
             return False
-        ok_w = all(w % 128 == 0 and w >= 128 for w in tuple(cfg.pi_arch) + tuple(cfg.vf_arch))
-        return (ok_w and 1 <= len(cfg.pi_arch) <= 4 and 1 <= len(cfg.vf_arch) <= 4 and cfg.pi_arch[-1] <= 512 and cfg.vf_arch[-1] <= 512
-                and obs_dim <= 64 and act_dim in (1, 3, 4))
+        return FusedUpdate.shapes_ok(cfg.pi_arch, cfg.vf_arch, obs_dim, act_dim)
 
     def __init__(self, learner: "PPOLearner", max_rows: int):
         from . import _lib as L
@@ -396,8 +402,8 @@ class PPOLearner:
             raise ValueError(f"update_impl={impl!r}")
         can = FusedUpdate.supported(cfg, obs_dim, act_dim, self.device)
         if impl == "fused" and not can:
-            raise RuntimeError("update_impl='fused' needs a compute-capability-10 CUDA device, hidden widths that are multiples of "
-                               "128 (last <= 512), at most 4 hidden layers, obs_dim <= 64 and act_dim in (1, 3, 4)")
+            raise RuntimeError("update_impl='fused' needs a compute-capability-10 CUDA device, 1..4 hidden layers per network whose "
+                               "widths are multiples of 128 between 128 and 512, 1 <= obs_dim <= 64 and act_dim in (1, 3, 4)")
         self.want_fused = can and impl in ("auto", "fused")
         self.fused: Optional[FusedUpdate] = None
         if self.device.type == "cuda":                  # process-wide switches: set both ways so "fp32" means FP32

@@ -50,7 +50,7 @@ typedef struct dn_ppo_config {
     int32_t obs_dim, act_dim;      /* 13 (12 without the distance entry) / 4 */
     int32_t max_rows;              /* rows of the workspaces: >= the largest minibatch and dn_ppo_forward batch */
     int32_t n_pi, n_vf;            /* hidden layers of the policy / value network (1..DN_PPO_MAX_LAYERS) */
-    int32_t pi_hidden[DN_PPO_MAX_LAYERS], vf_hidden[DN_PPO_MAX_LAYERS];   /* widths, multiples of 64, last <= 512 */
+    int32_t pi_hidden[DN_PPO_MAX_LAYERS], vf_hidden[DN_PPO_MAX_LAYERS];   /* widths: multiples of 128, 128..512 */
     int32_t precision;             /* DN_MLP_BF16X3 | DN_MLP_BF16 */
     int32_t normalize_advantage;   /* sb3_ppo.py:233-234 */
     int32_t world_size;            /* ranks whose gradients the caller sums into the bucket between grad and apply */

@@ -63,6 +63,36 @@ def test_ppo_update_rejects_bad_config_without_a_gpu(built_lib):
     assert built_lib.dn_mlp_gemm(5, 3, 128, 64, 64, 1, buf, buf, buf, 1, None, buf, None, None) == -1
 
 
+def test_fused_shape_rule_agrees_with_dn_ppo_create(built_lib):
+    """FusedUpdate.shapes_ok accepts exactly the shapes dn_ppo_create validates, so PPOConfig(update_impl="auto") never picks a
+    fused handle the library then refuses.  dn_ppo_create checks the whole configuration before it looks for a device: a shape it
+    accepts gets DN_ECUDA without a device, and with device index -1 on a machine with one it gets "bad device index" -- either
+    way it never allocates."""
+    import itertools
+    from drl_dronenavigation_b200 import _lib
+    from drl_dronenavigation_b200.ppo import FusedUpdate
+    archs = [(), (128,), (64,), (256, 128), (512, 512, 256), (512, 512, 256, 128), (128,) * 5, (1024, 512, 256), (512, 1024, 256),
+             (512, 640), (640,), (384, 256), (192, 128), (500,), (0,)]
+    buf = (C.c_float * 8)()
+    h = C.c_void_p()
+    accepted = 0
+    for pi, vf, obs, act in itertools.product(archs, [(256, 128), (512, 512), (1024,), (128, 64)], (0, 1, 12, 64, 65), range(6)):
+        cfg = _lib.dn_ppo_config()
+        cfg.abi_version, cfg.max_rows, cfg.world_size = _lib.DN_ABI_VERSION, 256, 1
+        cfg.obs_dim, cfg.act_dim, cfg.n_pi, cfg.n_vf = obs, act, len(pi), len(vf)
+        for i, w in enumerate(pi[:_lib.DN_PPO_MAX_LAYERS]):
+            cfg.pi_hidden[i] = w
+        for i, w in enumerate(vf[:_lib.DN_PPO_MAX_LAYERS]):
+            cfg.vf_hidden[i] = w
+        rc = built_lib.dn_ppo_create(C.byref(cfg), -1, buf, buf, buf, buf, buf, C.byref(h))
+        err = built_lib.dn_last_error()
+        assert rc in (-1, -2) and not h.value, (pi, vf, obs, act, rc, err)
+        lib_ok = rc == -2 or b"bad device index" in err
+        assert FusedUpdate.shapes_ok(pi, vf, obs, act) == lib_ok, (pi, vf, obs, act, err)
+        accepted += lib_ok
+    assert accepted > 0
+
+
 def test_bad_config_is_rejected_without_a_gpu(built_lib):
     from drl_dronenavigation_b200 import _lib
     h = C.c_void_p()

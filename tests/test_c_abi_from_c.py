@@ -11,16 +11,16 @@ import pytest
 from tests.conftest import ROOT
 
 SRC = os.path.join(ROOT, "tests", "c_abi", "demo.c")
-EXE = os.path.join(ROOT, "tests", "c_abi", "demo")
 
 
 @pytest.fixture(scope="module")
-def demo(built_lib):
-    if not os.path.exists(EXE) or os.path.getmtime(EXE) < max(os.path.getmtime(SRC), os.path.getmtime(os.path.join(ROOT, "include", "dronenav.h"))):
-        subprocess.run(["gcc", "-std=c99", "-pedantic", "-Wall", "-Wextra", "-Werror", "-O1", "-I", os.path.join(ROOT, "include"),
-                        "-o", EXE, SRC, "-ldl", "-lm"], check=True)
+def demo(built_lib, tmp_path_factory):
+    # compiled outside the repository tree, which may be read-only where the suite runs
+    exe = str(tmp_path_factory.mktemp("c_abi") / "demo")
+    subprocess.run(["gcc", "-std=c99", "-pedantic", "-Wall", "-Wextra", "-Werror", "-O1", "-I", os.path.join(ROOT, "include"),
+                    "-o", exe, SRC, "-ldl", "-lm"], check=True)
     from drl_dronenavigation_b200 import _lib
-    return EXE, _lib.LIB_PATH
+    return exe, _lib.LIB_PATH
 
 
 def test_header_compiles_as_c99_and_every_symbol_resolves(demo):

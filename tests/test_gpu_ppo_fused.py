@@ -196,18 +196,21 @@ def test_trainer_uses_the_fused_update_and_learns_to_reduce_value_loss():
     env.close()
 
 
-@pytest.mark.skipif(not _cc10(), reason="needs an sm_100 device")
-def test_graph_replay_of_the_fused_step_is_bit_identical():
-    """The fused minibatch step replayed from CUDA graphs (static rollout / index buffers) is the same computation as the
-    launch-by-launch path: every kernel reduces in an order fixed by its geometry, so the parameters agree BIT FOR BIT, over two
-    updates (Adam state carried across replays) and through a KL early stop."""
+def _graph_replay_outputs(batch, rollout, presize):
+    """Final parameters and the statistics of two updates, launch by launch and replayed from CUDA graphs, each followed by an
+    update that stops at once.  `presize` > 0: the handle is first sized by a forward of that many rows."""
     from drl_dronenavigation_b200.ppo import PPOConfig, PPOLearner
     outs = {}
     for graph in (False, True):
-        L = PPOLearner(13, 4, PPOConfig(batch_size=1024, n_epochs=3, target_kl=None, cuda_graph=graph, update_impl="fused"), device="cuda")
-        ro = make_rollout(L, 8192, seed=4)
+        L = PPOLearner(13, 4, PPOConfig(batch_size=batch, n_epochs=3, target_kl=None, cuda_graph=graph, update_impl="fused"), device="cuda")
+        ro = make_rollout(L, rollout, seed=4)
+        if presize:
+            L.forward(ro[0][:presize])
+            assert L.fused.max_rows == presize
         r1 = L.update(*ro, generator=torch.Generator(device="cuda").manual_seed(1))
-        ro2 = make_rollout(L, 8192, seed=5)
+        if presize:
+            assert L.fused.max_rows == presize                # the minibatches ran on the handle the forward sized
+        ro2 = make_rollout(L, rollout, seed=5)
         r2 = L.update(*ro2, generator=torch.Generator(device="cuda").manual_seed(2))
         L.cfg.target_kl = 1e-7                       # third update: stops at once, nothing applied
         L.fused.close(); L.fused = None
@@ -215,6 +218,25 @@ def test_graph_replay_of_the_fused_step_is_bit_identical():
         r3 = L.update(*ro2, generator=torch.Generator(device="cuda").manual_seed(3))
         assert r3["early_stop"] and r3["optimizer_steps"] == 0 and torch.equal(p_before, L.flat_parameters())
         outs[graph] = (L.flat_parameters().clone(), r1, r2)
+    return outs
+
+
+def _assert_bit_identical(outs):
     assert torch.equal(outs[False][0], outs[True][0])
     for k in ("policy_gradient_loss", "value_loss", "approx_kl", "clip_fraction", "minibatches", "optimizer_steps"):
         assert outs[False][1][k] == outs[True][1][k] and outs[False][2][k] == outs[True][2][k], k
+
+
+@pytest.mark.skipif(not _cc10(), reason="needs an sm_100 device")
+def test_graph_replay_of_the_fused_step_is_bit_identical():
+    """The fused minibatch step replayed from CUDA graphs (static rollout / index buffers) is the same computation as the
+    launch-by-launch path: every kernel reduces in an order fixed by its geometry, so the parameters agree BIT FOR BIT, over two
+    updates (Adam state carried across replays) and through a KL early stop."""
+    _assert_bit_identical(_graph_replay_outputs(1024, 8192, 0))
+
+
+@pytest.mark.skipif(not _cc10(), reason="needs an sm_100 device")
+def test_graph_replay_is_bit_identical_at_the_bench_line_shape():
+    """As above on the handle the trainer builds for the bench line: sized by the rollout forward over 65 536 envs, then used for
+    32 768-row minibatches (plans re-made for the smaller row count, tensor maps over the larger workspaces)."""
+    _assert_bit_identical(_graph_replay_outputs(32768, 65536, 65536))
