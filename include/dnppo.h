@@ -106,9 +106,9 @@ int dn_ppo_minibatch_apply(dn_ppo* h, void* stream);
  * between dn_ppo_minibatch_grad and dn_ppo_minibatch_apply (which divides by cfg.world_size).  The exchange runs over NVLink
  * peer memory: dn_ppo_comm_create allocates this rank's exchange region and returns its CUDA IPC handle (64 bytes); the caller
  * gathers the handles of all ranks with whatever it has (torch.distributed, MPI, a file) and passes them, rank-major, to
- * dn_ppo_comm_connect.  dn_ppo_allreduce is then three short kernels (publish, reduce-scatter + push, collect) that wait for the
- * peers through flags in the mapped regions: capturable in a CUDA graph, bit-identical results on every rank (every element is
- * summed once, in rank order, by its owner).  Every rank must call it the same number of times; a wait that is not answered
+ * dn_ppo_comm_connect.  dn_ppo_allreduce is then ONE kernel of three phases (publish, reduce-scatter + push, collect) that waits
+ * for the peers through flags in the mapped regions: capturable in a CUDA graph, bit-identical results on every rank (every
+ * element is summed once, in rank order, by its owner).  Every rank must call it the same number of times; a wait that is not answered
  * within about a minute traps (CUDA error on the host) instead of hanging the GPU.  Single node only (CUDA IPC); the Python layer falls
  * back to ncclAllReduce elsewhere.  What it replaces: nothing in the reference (its PPO is single-process, sb3_ppo.py:288-294). */
 #define DN_PPO_COMM_HANDLE_BYTES 64

@@ -63,6 +63,18 @@ def test_ppo_update_rejects_bad_config_without_a_gpu(built_lib):
     assert built_lib.dn_mlp_gemm(5, 3, 128, 64, 64, 1, buf, buf, buf, 1, None, buf, None, None) == -1
 
 
+def test_comm_entry_points_reject_null_arguments_without_a_gpu(built_lib):
+    """dn_ppo_comm_create / _connect / dn_ppo_allreduce check their pointers before they touch the handle or the device."""
+    DN_EINVAL, DN_PPO_COMM_HANDLE_BYTES = -1, 64              # include/dronenav.h, include/dnppo.h
+    buf = (C.c_ubyte * (DN_PPO_COMM_HANDLE_BYTES * 2))()
+    not_null = C.cast(buf, C.c_void_p)        # stands in for a handle: a null buffer is refused before the handle is read
+    for call in (lambda: built_lib.dn_ppo_comm_create(None, 0, 2, buf), lambda: built_lib.dn_ppo_comm_create(not_null, 0, 2, None),
+                 lambda: built_lib.dn_ppo_comm_connect(None, buf), lambda: built_lib.dn_ppo_comm_connect(not_null, None),
+                 lambda: built_lib.dn_ppo_allreduce(None, None)):
+        assert call() == DN_EINVAL
+        assert b"null" in built_lib.dn_last_error()
+
+
 def test_fused_shape_rule_agrees_with_dn_ppo_create(built_lib):
     """FusedUpdate.shapes_ok accepts exactly the shapes dn_ppo_create validates, so PPOConfig(update_impl="auto") never picks a
     fused handle the library then refuses.  dn_ppo_create checks the whole configuration before it looks for a device: a shape it
