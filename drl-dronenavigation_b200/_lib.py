@@ -100,6 +100,14 @@ class dn_ppo_stats(C.Structure):
                 ("early_stop", C.c_int32), ("last_approx_kl", C.c_float), ("last_grad_norm", C.c_float)]
 
 
+class dn_ppo_sample(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("row_id_offset", C.c_int64), ("counter", C.c_void_p), ("deterministic", C.c_int32),
+                ("low", C.c_float), ("high", C.c_float)]
+
+
+DN_PPO_ACT_TAG = 0x50504F41     # second Philox counter word of dn_ppo_act's draws
+
+
 # every symbol include/dronenav.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "dn_abi_version": (C.c_int, []),
@@ -140,6 +148,8 @@ SYMBOLS = {
     "dn_ppo_allreduce": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dn_ppo_poll": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "dn_ppo_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dn_ppo_act": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(dn_ppo_sample), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                             C.c_void_p]),
     "dn_ppo_buffer": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
 }
 

@@ -66,6 +66,7 @@ class BatchedDroneEnv:
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
         self.num_envs = int(num_envs)
+        self.env_id_offset = int(env_id_offset)     # global id of env 0 of this shard (Philox subsequences: spawn, dn_ppo_act)
         targets = np.ascontiguousarray(np.array(target_points, dtype=np.float64).reshape(-1, 3))
         self.target_points = targets
         c = L.dn_config()

@@ -16,8 +16,9 @@ LIB_PATH = os.path.join(PKG_DIR, "libdronenav.so")
 INC = os.path.join(PKG_DIR, "..", "include")
 # source -> headers it includes
 SOURCES = {
-    "dronenav.cu": ["dn_params.h", "dn_device.cuh", "dn_host.h", os.path.join(INC, "dronenav.h")],
-    "ppo_update.cu": ["dn_umma.cuh", "ppo_kernels.cuh", "ppo_comm.cuh", os.path.join(INC, "dronenav.h"), os.path.join(INC, "dnppo.h")],
+    "dronenav.cu": ["dn_params.h", "dn_device.cuh", "dn_philox.cuh", "dn_host.h", os.path.join(INC, "dronenav.h")],
+    "ppo_update.cu": ["dn_umma.cuh", "ppo_kernels.cuh", "dn_philox.cuh", "ppo_comm.cuh", os.path.join(INC, "dronenav.h"),
+                      os.path.join(INC, "dnppo.h")],
 }
 
 NVCC_FLAGS = [

@@ -7,7 +7,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "dn_philox.cuh"
 #include "dn_umma.cuh"
+#include "../../include/dnppo.h"
 
 namespace dnppo {
 
@@ -106,6 +108,11 @@ struct HeadArgs {
     __nv_bfloat16* dzv_hi; __nv_bfloat16* dzv_lo;
     float* partial;                                     // [gridDim.x][head_partial_size]
     int partial_size;
+    // sampling (dn_ppo_act, inference only): the SAMPLE instantiations write action / clipped action / log-prob
+    float* out_action; float* out_clipped; float* out_logp;
+    const long long* counter;                           // null: deterministic (action = mean, nothing drawn)
+    unsigned long long seed; long long row_id_offset;
+    float low, high;
 };
 // layout of one block's partial: dW_pi [act_dim * n_pi] | db_pi [act_dim] | dW_vf [n_vf] | db_vf [1] | dlog_std [act_dim]
 //                                | dbh_pi [n_pi] | dbh_vf [n_vf]  (bias gradients of the LAST HIDDEN layers = column sums of dz)
@@ -120,8 +127,23 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
-// NP = column pairs per lane = (widest of the two last hidden layers) / 64: sizes the per-lane register arrays
-template <int ACT, int NP>
+// Box-Muller on two Philox words: z0 = r cos(2 pi u2), z1 = r sin(2 pi u2), r = sqrt(-2 ln u1), u1 in (0, 1], u2 in [0, 1)
+__device__ __forceinline__ void box_muller(uint32_t w1, uint32_t w2, float& z0, float& z1) {
+    const float r = sqrtf(-2.0f * logf(dn::u01_open(w1)));
+    float s, c;
+    sincospif(2.0f * dn::u01(w2), &s, &c);
+    z0 = r * c;
+    z1 = r * s;
+}
+
+// the draw counter of a stochastic dn_ppo_act call advances after the head kernel has read it
+__global__ void counter_advance_kernel(long long* counter) {
+    if (threadIdx.x == 0 && blockIdx.x == 0) *counter += 1;
+}
+
+// NP = column pairs per lane = (widest of the two last hidden layers) / 64: sizes the per-lane register arrays.
+// SAMPLE: the dn_ppo_act instantiations (inference only, no training code: the Philox rounds cost the row loop no registers)
+template <int ACT, int NP, bool SAMPLE>
 __global__ void __launch_bounds__(HEAD_WARPS * 32) head_kernel(const HeadArgs g) {
     extern __shared__ float hsm[];
     float* s_wpi = hsm;                                   // [ACT][n_pi]
@@ -134,7 +156,7 @@ __global__ void __launch_bounds__(HEAD_WARPS * 32) head_kernel(const HeadArgs g)
 
     const int ip = g.n_pi / 64, iv = g.n_vf / 64;         // column pairs per lane
     float adv_mean = 0.0f, adv_rstd = 1.0f;
-    if (g.train && g.normalize_adv) {
+    if (!SAMPLE && g.train && g.normalize_adv) {
         // advantage moments: the gather blocks' (sum, sum of squares) pairs, added in a fixed order by the whole block
         __shared__ double s_adv[2][HEAD_WARPS * 32];
         double a = 0.0, b = 0.0;
@@ -221,10 +243,12 @@ __global__ void __launch_bounds__(HEAD_WARPS * 32) head_kernel(const HeadArgs g)
                 }
             value = warp_sum(acc) + bvf;
         }
-        if (!g.train) {
+        if (SAMPLE || !g.train) {
             if (lane == 0) {
+                // dn_ppo_act: the mean is staged in the action output and turned into the action after the loop
+                float* out = SAMPLE ? g.out_action : g.out_mean;
 #pragma unroll
-                for (int a = 0; a < ACT; ++a) g.out_mean[static_cast<long long>(row) * ACT + a] = mean[a];
+                for (int a = 0; a < ACT; ++a) out[static_cast<long long>(row) * ACT + a] = mean[a];
                 g.out_value[row] = value;
             }
             continue;
@@ -306,7 +330,36 @@ __global__ void __launch_bounds__(HEAD_WARPS * 32) head_kernel(const HeadArgs g)
             }
         }
     }
-    if (!g.train) return;
+    if (SAMPLE || !g.train) {
+        if (!SAMPLE) return;
+        // ---- sampling (dn_ppo_act, draw layout in include/dnppo.h): this warp's rows, one per lane (lane 0's mean stores are
+        // visible to the warp after __syncwarp) ----
+        __syncwarp();
+        const uint32_t draw = g.counter ? static_cast<uint32_t>(*g.counter) : 0u;
+        for (int row = row_first + lane * row_step; row < g.rows; row += 32 * row_step) {
+            const long long o = static_cast<long long>(row) * ACT;
+            float z[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+            if (g.counter) {
+                const unsigned long long gid = static_cast<unsigned long long>(g.row_id_offset + row);
+                const dn::U4 r = dn::philox4x32_10(dn::U4{draw, DN_PPO_ACT_TAG, static_cast<uint32_t>(gid), static_cast<uint32_t>(gid >> 32)},
+                                                   static_cast<uint32_t>(g.seed), static_cast<uint32_t>(g.seed >> 32));
+                box_muller(r.x, r.y, z[0], z[1]);
+                if (ACT > 2) box_muller(r.z, r.w, z[2], z[3]);
+            }
+            float logp = 0.0f;
+#pragma unroll
+            for (int a = 0; a < ACT; ++a) {
+                const float mean = g.out_action[o + a];
+                const float act = g.counter ? fmaf(expf(lstd[a]), z[a], mean) : mean;
+                const float diff = act - mean;
+                logp += -0.5f * diff * diff * sig2inv[a] - lstd[a] - 0.918938533204672742f;      // the training branch's expression
+                g.out_action[o + a] = act;
+                if (g.out_clipped) g.out_clipped[o + a] = fminf(fmaxf(act, g.low), g.high);
+            }
+            g.out_logp[row] = logp;
+        }
+        return;
+    }
     // ---- block reduction in warp order (deterministic), one partial vector per block ----
     const int P = g.partial_size;
     float* mine = s_red + warp * P;

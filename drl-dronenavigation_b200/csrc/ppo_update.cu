@@ -456,31 +456,33 @@ int ensure_rows(dn_ppo* h, int rows, bool train) {
     return DN_OK;
 }
 
-template <int ACT, int NP>
+template <int ACT, int NP, bool SAMPLE>
 int launch_head(dn_ppo* h, const HeadArgs& a, int blocks, cudaStream_t st) {
     static bool attr = false;
     if (!attr) {
-        PPO_CUDA(cudaFuncSetAttribute(head_kernel<ACT, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        PPO_CUDA(cudaFuncSetAttribute(head_kernel<ACT, NP, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         attr = true;
     }
-    head_kernel<ACT, NP><<<blocks, HEAD_WARPS * 32, h->head_smem, st>>>(a);
+    head_kernel<ACT, NP, SAMPLE><<<blocks, HEAD_WARPS * 32, h->head_smem, st>>>(a);
     PPO_CUDA(cudaGetLastError());
     return DN_OK;
 }
 
-template <int ACT>
+template <int ACT, bool SAMPLE>
 int run_head_np(dn_ppo* h, HeadArgs& a, int blocks, cudaStream_t st) {
     const int np = std::max(a.n_pi, a.n_vf) / 64;       // widths are multiples of 128
-    if (np <= 2) return launch_head<ACT, 2>(h, a, blocks, st);
-    if (np <= 4) return launch_head<ACT, 4>(h, a, blocks, st);
-    return launch_head<ACT, 8>(h, a, blocks, st);
+    if (np <= 2) return launch_head<ACT, 2, SAMPLE>(h, a, blocks, st);
+    if (np <= 4) return launch_head<ACT, 4, SAMPLE>(h, a, blocks, st);
+    return launch_head<ACT, 8, SAMPLE>(h, a, blocks, st);
 }
 
+// a.out_action set: the sampling instantiations (dn_ppo_act)
 int run_head(dn_ppo* h, HeadArgs& a, int blocks, cudaStream_t st) {
+    const bool s = a.out_action != nullptr;
     switch (h->cfg.act_dim) {
-        case 1: return run_head_np<1>(h, a, blocks, st);
-        case 3: return run_head_np<3>(h, a, blocks, st);
-        case 4: return run_head_np<4>(h, a, blocks, st);
+        case 1: return s ? run_head_np<1, true>(h, a, blocks, st) : run_head_np<1, false>(h, a, blocks, st);
+        case 3: return s ? run_head_np<3, true>(h, a, blocks, st) : run_head_np<3, false>(h, a, blocks, st);
+        case 4: return s ? run_head_np<4, true>(h, a, blocks, st) : run_head_np<4, false>(h, a, blocks, st);
         default: return dn_internal_fail(DN_EINVAL, "dn_ppo: act_dim must be 1, 3 or 4");
     }
 }
@@ -834,6 +836,36 @@ int dn_ppo_forward(dn_ppo* h, const float* obs, int32_t rows, float* mean, float
     a.train = 0; a.out_mean = mean; a.out_value = value;
     const int head_blocks = std::min(std::max((rows + HEAD_WARPS - 1) / HEAD_WARPS, 1), h->head_blocks_max);
     return run_head(h, a, head_blocks, st);
+}
+
+int dn_ppo_act(dn_ppo* h, const float* obs, int32_t rows, const dn_ppo_sample* s, float* action, float* clipped_action, float* log_prob,
+               float* value, void* stream) {
+    if (!h || !obs || !s || !action || !log_prob || !value) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: null argument");
+    if (s->deterministic != 0 && s->deterministic != 1) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: deterministic must be 0 or 1");
+    if (!s->deterministic && !s->counter) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: a sampling call needs the device counter (null counter)");
+    if (s->row_id_offset < 0) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: row_id_offset must be >= 0");
+    if (!(s->low <= s->high)) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: low must not exceed high (and neither may be NaN)");
+    if (rows < 1) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: rows must be within max_rows");
+    if (rows > h->max_rows) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: rows must be within max_rows");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int rows_pad = (rows + BM - 1) / BM * BM;
+    int rc;
+    if ((rc = ensure_rows(h, rows_pad, false))) return rc;
+    if ((rc = run_gather(h, obs, nullptr, nullptr, rows, false, st))) return rc;
+    if ((rc = run_forward_chain(h, st))) return rc;
+    HeadArgs a;
+    fill_head_common(h, a, rows);
+    a.train = 0; a.out_value = value;
+    a.out_action = action; a.out_clipped = clipped_action; a.out_logp = log_prob;
+    a.counter = s->deterministic ? nullptr : reinterpret_cast<const long long*>(s->counter);
+    a.seed = s->seed; a.row_id_offset = s->row_id_offset; a.low = s->low; a.high = s->high;
+    const int head_blocks = std::min(std::max((rows + HEAD_WARPS - 1) / HEAD_WARPS, 1), h->head_blocks_max);
+    if ((rc = run_head(h, a, head_blocks, st))) return rc;
+    if (!s->deterministic) {
+        counter_advance_kernel<<<1, 32, 0, st>>>(reinterpret_cast<long long*>(s->counter));
+        PPO_CUDA(cudaGetLastError());
+    }
+    return DN_OK;
 }
 
 int dn_ppo_buffer(dn_ppo* h, const char* name, void** ptr, int64_t* elems) {

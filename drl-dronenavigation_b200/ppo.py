@@ -50,6 +50,8 @@ class PPOConfig:
     update_impl: str = "auto"           # "fused": hand-written sm_100a kernels (include/dnppo.h); "torch": eager PyTorch;
                                         # "auto": fused on a compute-capability-10 device when the shapes allow it
     mlp_precision: str = "bf16x3"       # fused path: "bf16x3" (FP32-faithful hi/lo split, default) | "bf16" (labelled option)
+    rollout_impl: str = "torch"         # "torch": per-step host loop, torch.Generator noise; "fused": dn_ppo_act (Philox noise keyed by
+                                        # the global env id) and the T-step loop replayed from a CUDA graph (needs the fused handle)
 
 
 _ONES: Dict[tuple, torch.Tensor] = {}
@@ -295,6 +297,30 @@ class FusedUpdate:
             self.L.check(self.lib.dn_ppo_sync_weights(self.handle, self._stream()), "dn_ppo_sync_weights")
             self.L.check(self.lib.dn_ppo_forward(self.handle, obs.data_ptr(), n, mean.data_ptr(), value.data_ptr(), self._stream()), "dn_ppo_forward")
         return mean, value
+
+    def act(self, obs: torch.Tensor, sample, action: torch.Tensor = None, clipped_action: torch.Tensor = None,
+            log_prob: torch.Tensor = None, value: torch.Tensor = None, sync: bool = True):
+        """ActorCriticPolicy.forward with the sampler of the library (dn_ppo_act): (action, clipped_action, log_prob, value).
+        `sample` is an ``_lib.dn_ppo_sample`` (seed, global id of row 0, device int64 draw counter, deterministic, Box bounds).
+        Outputs may be passed in (graph capture: fixed pointers); `clipped_action` is only written when given or allocated here.
+        ``sync=False`` skips the FP32 -> BF16 weight refresh (the caller knows the parameters did not change)."""
+        n = obs.shape[0]
+        A = self.cfg_c.act_dim
+        f = dict(dtype=torch.float32, device=self.device)
+        action = torch.empty(n, A, **f) if action is None else action
+        clipped_action = torch.empty(n, A, **f) if clipped_action is None else clipped_action
+        log_prob = torch.empty(n, **f) if log_prob is None else log_prob
+        value = torch.empty(n, **f) if value is None else value
+        dev = torch.device("cuda", torch.cuda.current_device() if self.device.index is None else self.device.index)
+        for t, shape in ((obs, (n, self.cfg_c.obs_dim)), (action, (n, A)), (clipped_action, (n, A)), (log_prob, (n,)), (value, (n,))):
+            if t.dtype != torch.float32 or t.device != dev or not t.is_contiguous() or tuple(t.shape) != shape:
+                raise ValueError(f"dn_ppo_act: expected a contiguous float32 tensor of shape {shape} on {self.device}")
+        with torch.cuda.device(self.device):
+            if sync:
+                self.L.check(self.lib.dn_ppo_sync_weights(self.handle, self._stream()), "dn_ppo_sync_weights")
+            self.L.check(self.lib.dn_ppo_act(self.handle, obs.data_ptr(), n, C.byref(sample), action.data_ptr(), clipped_action.data_ptr(),
+                                             log_prob.data_ptr(), value.data_ptr(), self._stream()), "dn_ppo_act")
+        return action, clipped_action, log_prob, value
 
     def begin_update(self):
         with torch.cuda.device(self.device):
@@ -788,9 +814,30 @@ class PPOTrainer:
         self.obs = env.reset().clone()
         self.total_steps = 0
         self.low, self.high = -1.0, 1.0           # Box(-1, 1) with normalize_actions (PBDroneEnv.py:230-236)
+        if cfg.rollout_impl not in ("torch", "fused"):
+            raise ValueError(f"rollout_impl={cfg.rollout_impl!r}")
+        self.rollout_graph = bool(cfg.cuda_graph)
+        self._rollout_graph = None
+        if cfg.rollout_impl == "fused":
+            if self.learner.fused is None:
+                raise RuntimeError("rollout_impl='fused' needs the fused PPO handle (update_impl 'fused' or 'auto' on a compute-capability-10 "
+                                   "CUDA device, 1..4 hidden layers per network whose widths are multiples of 128 between 128 and 512, "
+                                   "1 <= obs_dim <= 64, act_dim in (1, 3, 4), minibatches that are multiples of 128 and divide the rollout)")
+            from . import _lib as L
+            # Philox draw counter on the device (advanced by every dn_ppo_act call, also inside graph replays); the key is the
+            # seed shared by all ranks and the subsequence the GLOBAL env id, so the noise does not depend on the sharding
+            self.draw_counter = torch.zeros(1, dtype=torch.int64, device=self.dev)
+            self.sample = L.dn_ppo_sample()
+            self.sample.seed, self.sample.row_id_offset = int(cfg.seed), int(getattr(env, "env_id_offset", 0))
+            self.sample.counter, self.sample.deterministic = self.draw_counter.data_ptr(), 0
+            self.sample.low, self.sample.high = self.low, self.high
+            self.b_clip = torch.empty(T, N, 4, **f)       # what env.step received
+            self.b_term = torch.zeros(T, N, D, **f)       # terminal observations (meaningful where b_done == truncated)
 
     @torch.no_grad()
     def collect_rollouts(self):
+        if self.cfg.rollout_impl == "fused":
+            return self._collect_rollouts_fused()
         env, pol = self.env, self.learner
         for t in range(self.T):
             action, logp, value = pol.act(self.obs, generator=self.gen)
@@ -806,6 +853,57 @@ class PPOTrainer:
         last_values = pol.value(self.obs)
         adv, ret = compute_gae(self.b_rew, self.b_val, self.b_done, last_values, self.cfg.gamma, self.cfg.gae_lambda)
         self.total_steps += self.T * env.num_envs * _world()      # global count: every rank collects its own shard
+        return adv, ret
+
+    def _rollout_step(self, fu, t: int):
+        """Control step t of a fused rollout: act on the current observation, record, step the env (nothing here waits for the host)."""
+        env = self.env
+        self.b_obs[t].copy_(self.obs)
+        fu.act(self.b_obs[t], self.sample, self.b_act[t], self.b_clip[t], self.b_logp[t], self.b_val[t], sync=False)
+        env.step(self.b_clip[t])
+        self.b_rew[t].copy_(env.reward)
+        self.b_done[t].copy_(env.done)
+        self.b_term[t].copy_(env.terminal_obs)
+        self.obs.copy_(env.obs)
+
+    def _collect_rollouts_fused(self, graph: Optional[bool] = None):
+        """collect_rollouts on dn_ppo_act.  The T-step loop is one CUDA graph, captured at the second rollout (the first one, launched
+        step by step, loads every kernel) and replayed from then on; between its first and last step the host does not wait.  The
+        policy is fixed during a rollout, so the truncation bootstrap of SB3's collect_rollouts (V(terminal_obs) of episodes that
+        were truncated, not terminated) is deferred to one pass after the loop: the recorded terminal rows are compacted (the one
+        host synchronisation of the rollout), their values computed by dn_ppo_forward in chunks of at most max_rows, and
+        b_rew[t, i] += gamma V added as the per-step path adds it."""
+        from . import _lib as L
+        env, pol, cfg = self.env, self.learner, self.cfg
+        fu = pol.fused
+        graph = self.rollout_graph if graph is None else graph
+        fu.sync_weights()                       # the planes the loop reads (the loop itself does not refresh them)
+        g = self._rollout_graph
+        if graph and g is not None and g[0] is fu:
+            g[1].replay()
+        elif graph and getattr(self, "_rollout_warm", False):
+            cg = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(cg):
+                for t in range(self.T):
+                    self._rollout_step(fu, t)
+            self._rollout_graph = (fu, cg)
+            cg.replay()
+        else:
+            for t in range(self.T):
+                self._rollout_step(fu, t)
+            self._rollout_warm = True
+        # deferred bootstrap of truncated episodes
+        D = env.obs_dim
+        idx = (self.b_done.reshape(-1) == L.DN_DONE_TRUNCATED).nonzero().squeeze(1)
+        if idx.numel():
+            rows = self.b_term.reshape(-1, D).index_select(0, idx)
+            tv = torch.cat([fu.forward(rows[i:i + fu.max_rows])[1] for i in range(0, rows.shape[0], fu.max_rows)])
+            rew = self.b_rew.view(-1)
+            rew[idx] += cfg.gamma * tv
+        self.truncated_steps = int(idx.numel())
+        last_values = fu.forward(self.obs)[1]
+        adv, ret = compute_gae(self.b_rew, self.b_val, self.b_done, last_values, cfg.gamma, cfg.gae_lambda)
+        self.total_steps += self.T * env.num_envs * _world()
         return adv, ret
 
     def train_iteration(self) -> Dict[str, float]:

@@ -94,7 +94,7 @@ class PBDroneSimulator:
         n = train_env.num_envs
         T = getattr(self.args, "rollout_steps", None) or max(16, min(4096, (12 * 4096 * 8) // max(n, 1)))
         cfg = PPOConfig(n_steps=T, batch_size=getattr(self.args, "minibatch", None) or max(512, (T * n) // 32),
-                        n_epochs=getattr(self.args, "n_epochs", 10))
+                        n_epochs=getattr(self.args, "n_epochs", 10), rollout_impl=getattr(self.args, "rollout_impl", "torch"))
         return PPOTrainer(train_env, cfg, rollout_steps=T)
 
     # ------------------------------------------------------------------ runs

@@ -123,6 +123,41 @@ int dn_ppo_poll(dn_ppo* h, int32_t* early_stop, int32_t* minibatches, int32_t* o
 /* ActorCriticPolicy.forward without sampling: mean [rows, act_dim] and value [rows] for obs [rows, obs_dim] with the
  * same kernels and arithmetic as the update (rollout collection, evaluation).  rows <= max_rows. */
 int dn_ppo_forward(dn_ppo* h, const float* obs, int32_t rows, float* mean, float* value, void* stream);
+
+/* ActorCriticPolicy.forward with sampling (rollout collection): dn_ppo_forward's kernels and arithmetic for mean and value,
+ * then, per row, in the same kernel:
+ *   action[a]          = fmaf(exp(log_std[a]), z[a], mean[a])         (deterministic: action = mean, nothing is drawn)
+ *   log_prob           = sum_a -0.5 diff_a^2 exp(-2 log_std[a]) - log_std[a] - 0.5 log(2 pi),   diff = action - mean
+ *                        (the expression of the gradient half, which therefore recomputes the same old_log_prob)
+ *   clipped_action[a]  = min(max(action[a], low), high)                 (SB3 clips to the Box before env.step)
+ *
+ * Draw layout (bit-exact, restated in numpy by tests/ppo_act_reference.py).  Row r of a call with counter value c takes ONE
+ * Philox4x32-10 block (dn_philox.cuh, the generator of the random spawn):
+ *   key     = (seed lo, seed hi)
+ *   counter = (c mod 2^32, DN_PPO_ACT_TAG, g lo, g hi),   g = row_id_offset + r   (global row id: shard-invariant)
+ *   -> words (x, y, z, w).  The spawn draws use 0 and 1 in the second counter word, so the two streams never meet.
+ * Box-Muller on two pairs (x, y) and (z, w), 24-bit uniforms u01(v) = (v >> 8) 2^-24 in [0, 1),
+ * u01_open(v) = ((v >> 8) + 1) 2^-24 in (0, 1]:
+ *   r  = sqrt(-2 ln u01_open(x)),  z[0] = r cos(2 pi u01(y)),  z[1] = r sin(2 pi u01(y))
+ *   r' = sqrt(-2 ln u01_open(z)),  z[2] = r' cos(2 pi u01(w)), z[3] = r' sin(2 pi u01(w))
+ * act_dim 1 uses z[0], act_dim 3 z[0..2], act_dim 4 z[0..3].  The smallest u01_open is 2^-24, so |z| <= sqrt(48 ln 2) ~= 5.77:
+ * the tails beyond 5.77 sigma (probability ~8e-9 per component) are never drawn.  In FP32: logf, sqrtf and sincospif.
+ *
+ * `counter` is a DEVICE int64: a stochastic call reads *counter when its kernel runs and adds 1 after it (stream-ordered), so
+ * a captured CUDA graph replays draw after draw without host involvement.  `seed` is the same on every rank and
+ * `row_id_offset` is the shard's env_id_offset (dn_config): the env with global id g then draws the same noise on any split. */
+#define DN_PPO_ACT_TAG 0x50504F41u   /* "PPOA": second counter word of the sampler's draws */
+typedef struct dn_ppo_sample {
+    uint64_t seed;                 /* Philox key */
+    int64_t  row_id_offset;        /* global id of row 0 (>= 0) */
+    int64_t* counter;              /* device; this call draws at *counter, then *counter += 1.  May be NULL when deterministic */
+    int32_t  deterministic;        /* 1: action = mean, no draw, counter untouched; 0: sample */
+    float    low, high;            /* Box bounds of clipped_action, low <= high */
+} dn_ppo_sample;
+/* obs [rows, obs_dim]; action, clipped_action (nullable) [rows, act_dim]; log_prob, value [rows]; rows <= max_rows.
+ * Capturable, no host synchronisation; the arguments are checked before the handle is read. */
+int dn_ppo_act(dn_ppo* h, const float* obs, int32_t rows, const dn_ppo_sample* s, float* action, float* clipped_action,
+               float* log_prob, float* value, void* stream);
 /* Test hook: device pointer / element count of an internal buffer: "x", "pi.h1".."pi.h4", "pi.dz1".., "pi.w1".. (BF16
  * planes, lo plane at + elems / 2), and the same with "vf.". */
 int dn_ppo_buffer(dn_ppo* h, const char* name, void** ptr, int64_t* elems);
