@@ -107,8 +107,28 @@ class dn_ppo_sample(C.Structure):
 
 DN_PPO_ACT_TAG = 0x50504F41     # second Philox counter word of dn_ppo_act's draws
 
+# ---- include/dnsac.h ------------------------------------------------------------------------------------------
+DN_SAC_MAX_LAYERS = 4
+DN_SAC_SAMPLE, DN_SAC_DETERMINISTIC, DN_SAC_UNIFORM = 0, 1, 2
+DN_SAC_ACT_TAG = 0x53414341     # "SACA": second Philox counter word of dn_sac_act's draws
 
-# every symbol include/dronenav.h declares: name -> (restype, argtypes)
+
+class dn_sac_actor_config(C.Structure):
+    _fields_ = [
+        ("abi_version", C.c_int32), ("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("max_rows", C.c_int32),
+        ("n_hidden", C.c_int32), ("hidden", C.c_int32 * DN_SAC_MAX_LAYERS), ("precision", C.c_int32),
+        ("w_off", C.c_int64 * DN_SAC_MAX_LAYERS), ("b_off", C.c_int64 * DN_SAC_MAX_LAYERS),
+        ("mu_w_off", C.c_int64), ("mu_b_off", C.c_int64), ("log_std_w_off", C.c_int64), ("log_std_b_off", C.c_int64),
+        ("n_params", C.c_int64),
+    ]
+
+
+class dn_sac_sample(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("row_id_offset", C.c_int64), ("counter", C.c_void_p), ("mode", C.c_int32),
+                ("reserved0", C.c_int32)]
+
+
+# every symbol include/dronenav.h and include/dnppo.h declare: name -> (restype, argtypes)
 SYMBOLS = {
     "dn_abi_version": (C.c_int, []),
     "dn_last_error": (C.c_char_p, []),
@@ -153,6 +173,15 @@ SYMBOLS = {
     "dn_ppo_buffer": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
 }
 
+# every symbol include/dnsac.h declares
+SAC_SYMBOLS = {
+    "dn_sac_actor_create": (C.c_int, [C.POINTER(dn_sac_actor_config), C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "dn_sac_actor_destroy": (C.c_int, [C.c_void_p]),
+    "dn_sac_actor_sync_weights": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "dn_sac_act": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(dn_sac_sample), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dn_sac_actor_buffer": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
+}
+
 _lib = None
 
 
@@ -169,7 +198,7 @@ def lib() -> C.CDLL:
                 f"{LIB_PATH} is missing: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
                 "(nvcc, sm_100a).  drl_dronenavigation_b200 has no CPU fallback.")
         handle = C.CDLL(LIB_PATH)
-        for name, (restype, argtypes) in SYMBOLS.items():
+        for name, (restype, argtypes) in (SYMBOLS | SAC_SYMBOLS).items():
             fn = getattr(handle, name)          # AttributeError if the symbol is not exported
             fn.restype = restype
             fn.argtypes = argtypes

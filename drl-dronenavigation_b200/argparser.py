@@ -68,8 +68,9 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--tensorboard", type=str, default=None, help="directory for TensorBoard scalars (SB3 tag names)")
     p.add_argument("--rollout_steps", type=int, default=None, help="steps per env per PPO rollout (default: n_steps=4096 / scaled)")
     p.add_argument("--rollout_impl", type=str, default="torch", choices=["torch", "fused"],
-                   help="PPO rollout collection: torch (per-step host loop, torch.Generator noise) or fused (dn_ppo_act: Philox noise "
-                        "keyed by the global env id, the rollout replayed from a CUDA graph; needs the fused PPO handle)")
+                   help="rollout collection: torch (per-step host loop, torch.Generator noise) or fused (Philox noise keyed by the "
+                        "global env id, collection replayed from a CUDA graph). PPO: dn_ppo_act, needs the fused PPO handle; SAC: "
+                        "dn_sac_act, needs a compute-capability-10 device (the SAC gradient step stays on torch)")
     return p
 
 

@@ -17,8 +17,8 @@ INC = os.path.join(PKG_DIR, "..", "include")
 # source -> headers it includes
 SOURCES = {
     "dronenav.cu": ["dn_params.h", "dn_device.cuh", "dn_philox.cuh", "dn_host.h", os.path.join(INC, "dronenav.h")],
-    "ppo_update.cu": ["dn_umma.cuh", "ppo_kernels.cuh", "dn_philox.cuh", "ppo_comm.cuh", os.path.join(INC, "dronenav.h"),
-                      os.path.join(INC, "dnppo.h")],
+    "ppo_update.cu": ["dn_umma.cuh", "ppo_kernels.cuh", "dn_philox.cuh", "ppo_comm.cuh", "sac_kernels.cuh", os.path.join(INC, "dronenav.h"),
+                      os.path.join(INC, "dnppo.h"), os.path.join(INC, "dnsac.h")],
 }
 
 NVCC_FLAGS = [

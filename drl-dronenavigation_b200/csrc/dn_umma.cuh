@@ -3,7 +3,7 @@
 // FP32 accumulation in TMEM) issued by one thread, tcgen05.ld epilogues fused with the elementwise work of the layer.
 //
 // One persistent, warp-specialised kernel template `umma_gemm<KIND, BN>` serves the three contractions of an MLP layer
-//   FWD    Y  = tanh(X W^T + b)            A = X  [M,K]   K-major, B = W  [N,K]    K-major
+//   FWD    Y  = tanh(X W^T + b)            A = X  [M,K]   K-major, B = W  [N,K]    K-major   (FWD_RELU: max(X W^T + b, 0))
 //   DGRAD  dX = (dY W) * (1 - H^2)         A = dY [M,N]   K-major, B = W  [N,K]    MN-major (reduction over W's rows)
 //   WGRAD  dW = dY^T X  (split over rows)  A = dY [m,N]   MN-major, B = X [m,K]    MN-major (reduction over the batch rows)
 // so that no transposed copy of an activation, a gradient or a weight is ever written.
@@ -51,7 +51,9 @@ constexpr uint32_t BAR_BYTES = 512;
 constexpr uint32_t SMEM_BYTES = 1024 /* alignment slack */ + RING_BYTES + EPI_BYTES + COLSUM_BYTES + BAR_BYTES;
 constexpr uint32_t PEER_BIT_MASK = 0xFEFFFFFFu;      // shared::cluster address of the same offset in the even CTA of a pair
 
-enum Kind { K_FWD = 0, K_DGRAD = 1, K_WGRAD = 2 };
+// K_FWD_RELU: the forward contraction with max(x, 0) as a compile-time epilogue (the SAC actor's latent layers).  A kind of
+// its own rather than a third runtime value of GemmArgs::act, so that the K_FWD instantiations keep their code.
+enum Kind { K_FWD = 0, K_DGRAD = 1, K_WGRAD = 2, K_FWD_RELU = 3 };
 
 struct GemmArgs {
     int m_tiles, n_tiles, slices;   // tile grid: accumulator rows / (128 CG), accumulator columns / BN, split of the reduction
@@ -331,7 +333,7 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
     constexpr int BNL = BN / CG;                          // rows (K-major) / columns (MN-major) of B this CTA loads
     constexpr uint32_t A_BYTES = BM * BK * 2;             // one plane of the A tile: 16 KB
     constexpr uint32_t B_BYTES = BNL * BK * 2;            // one plane of this CTA's share of the B tile
-    constexpr uint32_t IDESC = instr_desc(BM * CG, BN, KIND == K_WGRAD, KIND != K_FWD);
+    constexpr uint32_t IDESC = instr_desc(BM * CG, BN, KIND == K_WGRAD, KIND != K_FWD && KIND != K_FWD_RELU);
     constexpr uint32_t TMEM_COLS = (2 * BN <= 32) ? 32 : (2 * BN <= 64) ? 64 : (2 * BN <= 128) ? 128 : (2 * BN <= 256) ? 256 : 512;
 
     extern __shared__ uint8_t smem_raw[];
@@ -391,7 +393,7 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
             for (int gi = 0; gi < g.groups; ++gi)
                 for (int i = threadIdx.x; i < 4 * g.ld_out; i += NUM_THREADS) colsum_s[gi * GROUP_FLOATS + i] = 0.0f;
     }
-    if constexpr (KIND == K_FWD) {                       // the layer's bias vector (<= 512 entries) next to the epilogue warps
+    if constexpr (KIND == K_FWD || KIND == K_FWD_RELU) {   // the layer's bias vector (<= 512 entries) next to the epilogue warps
         for (int gi = 0; gi < g.groups; ++gi)
             for (int i = threadIdx.x; i < g.ld_out; i += NUM_THREADS) colsum_s[gi * GROUP_FLOATS + i] = __ldg((gi ? g.bias2 : g.bias) + i);
     }
@@ -426,7 +428,7 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                         const int a_row = p ? g.a_lo_row : 0, b_row = p ? g.b_lo_row : 0;
                         uint8_t* da = sa + p * A_BYTES;
                         uint8_t* db = sb + p * B_BYTES;
-                        if constexpr (KIND == K_FWD) {
+                        if constexpr (KIND == K_FWD || KIND == K_FWD_RELU) {
                             tma_load_2d<CG>(mA, &full_bar[stage], da, kb * BK, a_row + m0);                         // X rows, K slice
                             tma_load_2d<CG>(mB, &full_bar[stage], db, kb * BK, b_row + n0);                         // W rows, K slice
                         } else if constexpr (KIND == K_DGRAD) {
@@ -472,11 +474,11 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                     for (int k = 0; k < BK / UK; ++k) {
                         if (g.dbg & 4) break;
                         const uint64_t a_hi = (KIND == K_WGRAD) ? desc_mnmajor(sa, k) : desc_kmajor(sa, k);
-                        const uint64_t b_hi = (KIND == K_FWD) ? desc_kmajor(sb, k) : desc_mnmajor(sb, k);
+                        const uint64_t b_hi = (KIND == K_FWD || KIND == K_FWD_RELU) ? desc_kmajor(sb, k) : desc_mnmajor(sb, k);
                         umma_bf16<CG>(d_tmem, a_hi, b_hi, IDESC, (kb | k) != 0);
                         if (planes == 2) {
                             const uint64_t a_lo = (KIND == K_WGRAD) ? desc_mnmajor(sa + A_BYTES, k) : desc_kmajor(sa + A_BYTES, k);
-                            const uint64_t b_lo = (KIND == K_FWD) ? desc_kmajor(sb + B_BYTES, k) : desc_mnmajor(sb + B_BYTES, k);
+                            const uint64_t b_lo = (KIND == K_FWD || KIND == K_FWD_RELU) ? desc_kmajor(sb + B_BYTES, k) : desc_mnmajor(sb + B_BYTES, k);
                             umma_bf16<CG>(d_tmem, a_hi, b_lo, IDESC, 1);
                             umma_bf16<CG>(d_tmem, a_lo, b_hi, IDESC, 1);
                         }
@@ -552,14 +554,19 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
 #pragma unroll
                     for (int qd = 0; qd < 8; ++qd) dst[qd] = make_float4(v[4 * qd], v[4 * qd + 1], v[4 * qd + 2], v[4 * qd + 3]);
                 } else {
-                    if constexpr (KIND == K_FWD) {
+                    if constexpr (KIND == K_FWD || KIND == K_FWD_RELU) {
                         const float4* sbias = reinterpret_cast<const float4*>(gsm + col);
 #pragma unroll
                         for (int j4 = 0; j4 < 8; ++j4) {
                             const float4 bb = sbias[j4];
                             v[4 * j4] += bb.x; v[4 * j4 + 1] += bb.y; v[4 * j4 + 2] += bb.z; v[4 * j4 + 3] += bb.w;
                         }
-                        if (g.act && !(g.dbg & 1)) {
+                        if constexpr (KIND == K_FWD_RELU) {
+                            if (!(g.dbg & 1)) {
+#pragma unroll
+                                for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.0f);
+                            }
+                        } else if (g.act && !(g.dbg & 1)) {
 #pragma unroll
                             for (int j = 0; j < 32; ++j) v[j] = tanh_fast(v[j]);
                         }

@@ -1,5 +1,5 @@
-// ppo_update.cu -- the PPO minibatch update (include/dnppo.h) on sm_100a: tensor-map construction, launchers of the
-// tcgen05 contraction kernel (dn_umma.cuh) and the CUDA-core kernels around it.
+// ppo_update.cu -- the PPO minibatch update (include/dnppo.h) and the SAC actor (include/dnsac.h) on sm_100a: tensor-map
+// construction, launchers of the tcgen05 contraction kernel (dn_umma.cuh) and the CUDA-core kernels around it.
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -13,10 +13,12 @@
 #include <vector>
 
 #include "../../include/dnppo.h"
+#include "../../include/dnsac.h"
 #include "../../include/dronenav.h"
 #include "dn_umma.cuh"
 #include "ppo_kernels.cuh"
 #include "ppo_comm.cuh"
+#include "sac_kernels.cuh"
 
 int dn_internal_fail(int code, const std::string& msg);   // dronenav.cu: sets the thread-local dn_last_error message
 
@@ -143,6 +145,7 @@ int launch_gemm(const GemmPlan& p, cudaStream_t st) {
     DN_CASE(K_FWD, 256, 2) DN_CASE(K_FWD, 128, 2) DN_CASE(K_FWD, 128, 1) DN_CASE(K_FWD, 64, 1)
     DN_CASE(K_DGRAD, 256, 2) DN_CASE(K_DGRAD, 128, 2) DN_CASE(K_DGRAD, 128, 1) DN_CASE(K_DGRAD, 64, 1)
     DN_CASE(K_WGRAD, 256, 2) DN_CASE(K_WGRAD, 128, 2) DN_CASE(K_WGRAD, 128, 1) DN_CASE(K_WGRAD, 64, 1)
+    DN_CASE(K_FWD_RELU, 256, 2) DN_CASE(K_FWD_RELU, 128, 2) DN_CASE(K_FWD_RELU, 128, 1) DN_CASE(K_FWD_RELU, 64, 1)
 #undef DN_CASE
     return dn_internal_fail(DN_EINVAL, "launch_gemm: no such kernel instantiation");
 }
@@ -153,12 +156,12 @@ void set_grid(GemmPlan* p) {
     const GemmArgs& g = p->args;
     p->grid = grid_for(g.m_tiles * g.n_tiles * g.slices, p->cg);
 }
-// forward: out[M,N] = act(A[M,K] W[N,K]^T + bias)
+// forward: out[M,N] = act(A[M,K] W[N,K]^T + bias); act 0 identity, 1 tanh, 2 ReLU (the K_FWD_RELU instantiations)
 int plan_fwd(GemmPlan* p, int passes, int M, int N, int K, const void* a, const void* w, const float* bias, int act, void* out,
              int rows_now = 0) {
     if (!rows_now) rows_now = M;
     if (M % BM || rows_now % BM || N % 64 || K % 64) return dn_internal_fail(DN_EINVAL, "mlp forward: M % 128, N % 64, K % 64 must be 0");
-    p->kind = K_FWD;
+    p->kind = (act == 2) ? K_FWD_RELU : K_FWD;
     pick_tile(rows_now, N, &p->cg, &p->bn);
     int rc;
     if ((rc = make_map(&p->ma, a, 2LL * M, K, BM, MAP_KMAJOR)) || (rc = make_map(&p->mb, w, 2LL * N, K, p->bn / p->cg, MAP_KMAJOR)) ||
@@ -288,8 +291,8 @@ int wgrad_slices(int rows, int tiles, int units) {
     return std::max(1, std::min(target, rows / 256));
 }
 
-template <typename T>
-int dev_alloc(dn_ppo* h, T** p, size_t count) {
+template <typename H, typename T>
+int dev_alloc(H* h, T** p, size_t count) {
     void* q = nullptr;
     PPO_CUDA(cudaMalloc(&q, std::max<size_t>(count, 1) * sizeof(T)));
     PPO_CUDA(cudaMemset(q, 0, std::max<size_t>(count, 1) * sizeof(T)));
@@ -403,15 +406,17 @@ int build_reduce_table(dn_ppo* h, int rows) {
     return DN_OK;
 }
 
-int build_plane_table(dn_ppo* h) {
+// the table planes_kernel walks: every hidden weight of `nets` -> its BF16 planes
+template <typename H>
+int build_plane_table(H* h, const Net* const* nets, int n_nets, int obs_dim) {
     std::vector<PlaneSeg> v;
     std::vector<int> sob;
-    Net* nets[2] = {&h->pi, &h->vf};
-    for (Net* net : nets)
+    for (int k = 0; k < n_nets; ++k) {
+        const Net* net = nets[k];
         for (int l = 1; l <= net->L; ++l) {
             PlaneSeg s;
             s.param_off = net->w_off[l - 1]; s.rows = net->n[l]; s.ld = net->n[l - 1];
-            s.cols = (l == 1) ? h->cfg.obs_dim : net->n[l - 1];
+            s.cols = (l == 1) ? obs_dim : net->n[l - 1];
             s.planes = net->w[l];
             const long long count = static_cast<long long>(s.rows) * s.ld / 2;
             s.first_block = static_cast<int>(sob.size());
@@ -419,6 +424,7 @@ int build_plane_table(dn_ppo* h) {
             for (int b = 0; b < s.n_blocks; ++b) sob.push_back(static_cast<int>(v.size()));
             v.push_back(s);
         }
+    }
     PPO_CUDA(cudaMalloc(&h->psegs_dev, v.size() * sizeof(PlaneSeg)));
     PPO_CUDA(cudaMalloc(&h->pseg_of_block_dev, sob.size() * sizeof(int)));
     PPO_CUDA(cudaMemcpy(h->psegs_dev, v.data(), v.size() * sizeof(PlaneSeg), cudaMemcpyHostToDevice));
@@ -487,20 +493,29 @@ int run_head(dn_ppo* h, HeadArgs& a, int blocks, cudaStream_t st) {
     }
 }
 
+// observation rows -> the padded BF16 planes `x` [2][max_rows][XPAD] the first layer reads
+void gather_obs_args(GatherArgs& g, const float* obs, int rows, int obs_dim, __nv_bfloat16* x, int max_rows, int passes) {
+    memset(&g, 0, sizeof(g));
+    g.obs = obs; g.rows = rows; g.obs_dim = obs_dim;
+    g.x_hi = x; g.x_lo = (passes > 1) ? x + static_cast<long long>(max_rows) * XPAD : nullptr;
+}
+int launch_gather(const GatherArgs& g, cudaStream_t st) {
+    const int blocks = (g.rows * 8 + 255) / 256;
+    gather_kernel<<<blocks, 256, 0, st>>>(g);
+    PPO_CUDA(cudaGetLastError());
+    return DN_OK;
+}
+
 int run_gather(dn_ppo* h, const float* obs, const dn_ppo_rollout* r, const long long* idx, int rows, bool train, cudaStream_t st) {
     GatherArgs g;
-    memset(&g, 0, sizeof(g));
-    g.obs = obs; g.idx = idx; g.rows = rows; g.obs_dim = h->cfg.obs_dim; g.act_dim = h->cfg.act_dim;
-    g.x_hi = h->x; g.x_lo = (h->passes > 1) ? h->x + static_cast<long long>(h->max_rows) * XPAD : nullptr;
+    gather_obs_args(g, obs, rows, h->cfg.obs_dim, h->x, h->max_rows, h->passes);
+    g.idx = idx; g.act_dim = h->cfg.act_dim;
     if (train) {
         g.act = r->actions; g.logp = r->old_log_prob; g.val = r->old_values; g.adv = r->advantages; g.ret = r->returns;
         g.m_act = h->m_act; g.m_logp = h->m_logp; g.m_val = h->m_val; g.m_adv = h->m_adv; g.m_ret = h->m_ret;
         g.adv_partial = h->adv_partial;
     }
-    const int blocks = (rows * 8 + 255) / 256;
-    gather_kernel<<<blocks, 256, 0, st>>>(g);
-    PPO_CUDA(cudaGetLastError());
-    return DN_OK;
+    return launch_gather(g, st);
 }
 
 int run_forward_chain(dn_ppo* h, cudaStream_t st) {
@@ -624,7 +639,10 @@ int dn_ppo_create(const dn_ppo_config* cfg, int device, float* params, float* gr
         if (e != cudaSuccess) return bail(dn_internal_fail(DN_ECUDA, std::string("cudaHostGetDevicePointer: ") + cudaGetErrorString(e)));
         h->mirror_dev = static_cast<int*>(d);
     }
-    if ((rc = build_plane_table(h))) return bail(rc);
+    {
+        const Net* nets[2] = {&h->pi, &h->vf};
+        if ((rc = build_plane_table(h, nets, 2, cfg->obs_dim))) return bail(rc);
+    }
     if ((rc = ensure_rows(h, h->max_rows, true))) return bail(rc);
     if ((rc = dn_ppo_sync_weights(h, nullptr))) return bail(rc);
     PPO_CUDA(cudaStreamSynchronize(nullptr));
@@ -884,6 +902,211 @@ int dn_ppo_buffer(dn_ppo* h, const char* name, void** ptr, int64_t* elems) {
         }
     }
     return dn_internal_fail(DN_EINVAL, "dn_ppo_buffer: unknown buffer name");
+}
+
+}  // extern "C"
+
+// ====================================================================================================================
+// the SAC actor (include/dnsac.h): the latent ReLU layers on the forward contraction above, then sac_head_kernel
+// ====================================================================================================================
+struct dn_sac_actor {
+    dn_sac_actor_config cfg;
+    int device = 0, passes = 3, sms = 148;
+    int max_rows = 0, cur_rows = -1;
+    const float* params = nullptr;
+    __nv_bfloat16* x = nullptr;
+    Net net;                          // h, w and fwd of the latent layers (the training buffers stay unallocated)
+    float *mu = nullptr, *log_std = nullptr;
+    PlaneSeg* psegs_dev = nullptr; int* pseg_of_block_dev = nullptr; int plane_blocks = 0;
+    std::vector<void*> allocs;
+};
+
+namespace {
+
+int sac_check_config(const dn_sac_actor_config* c) {
+    if (c->abi_version != DN_ABI_VERSION) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: abi_version mismatch");
+    if (c->obs_dim < 1 || c->obs_dim > XPAD) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: obs_dim must be 1..64");
+    if (c->act_dim < 1 || c->act_dim > 4) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: act_dim must be 1..4");
+    if (c->max_rows < BM || c->max_rows % BM) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: max_rows must be a positive multiple of 128");
+    if (c->n_hidden < 1 || c->n_hidden > DN_SAC_MAX_LAYERS) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: 1..4 hidden layers");
+    for (int l = 0; l < c->n_hidden; ++l)
+        if (c->hidden[l] < 128 || c->hidden[l] > 512 || c->hidden[l] % 128)
+            return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: hidden widths must be multiples of 128 between 128 and 512");
+    if (c->precision != DN_MLP_BF16X3 && c->precision != DN_MLP_BF16) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: unknown precision");
+    const long long A = c->act_dim, last = c->hidden[c->n_hidden - 1];
+    auto inside = [&](long long off, long long count) { return off >= 0 && count <= c->n_params && off <= c->n_params - count; };
+    bool ok = c->n_params > 0;
+    for (int l = 0; l < c->n_hidden; ++l) {
+        const long long in = l ? c->hidden[l - 1] : c->obs_dim;
+        ok = ok && inside(c->w_off[l], c->hidden[l] * in) && inside(c->b_off[l], c->hidden[l]);
+    }
+    ok = ok && inside(c->mu_w_off, A * last) && inside(c->mu_b_off, A) && inside(c->log_std_w_off, A * last) && inside(c->log_std_b_off, A);
+    if (!ok) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: a parameter tensor lies outside [0, n_params)");
+    return DN_OK;
+}
+
+int sac_ensure_rows(dn_sac_actor* h, int rows_pad) {
+    if (rows_pad == h->cur_rows) return DN_OK;
+    Net& net = h->net;
+    int rc;
+    for (int l = 1; l <= net.L; ++l)
+        if ((rc = plan_fwd(&net.fwd[l], h->passes, h->max_rows, net.n[l], net.n[l - 1], net.h[l - 1], net.w[l], h->params + net.b_off[l - 1], 2,
+                           net.h[l], rows_pad)))
+            return rc;
+    h->cur_rows = rows_pad;
+    return DN_OK;
+}
+
+template <int ACT, int NP>
+int launch_sac_head(const dnsac::SacHeadArgs& a, int blocks, cudaStream_t st) {
+    dnsac::sac_head_kernel<ACT, NP><<<blocks, HEAD_WARPS * 32, 2 * ACT * a.n * sizeof(float), st>>>(a);
+    PPO_CUDA(cudaGetLastError());
+    return DN_OK;
+}
+
+template <int ACT>
+int run_sac_head_np(const dnsac::SacHeadArgs& a, int blocks, cudaStream_t st) {
+    const int np = a.n / 64;                              // widths are multiples of 128
+    if (np <= 2) return launch_sac_head<ACT, 2>(a, blocks, st);
+    if (np <= 4) return launch_sac_head<ACT, 4>(a, blocks, st);
+    return launch_sac_head<ACT, 8>(a, blocks, st);
+}
+
+int run_sac_head(int act_dim, const dnsac::SacHeadArgs& a, int blocks, cudaStream_t st) {
+    switch (act_dim) {
+        case 1: return run_sac_head_np<1>(a, blocks, st);
+        case 2: return run_sac_head_np<2>(a, blocks, st);
+        case 3: return run_sac_head_np<3>(a, blocks, st);
+        case 4: return run_sac_head_np<4>(a, blocks, st);
+        default: return dn_internal_fail(DN_EINVAL, "dn_sac_act: act_dim must be 1..4");
+    }
+}
+
+}  // namespace
+
+extern "C" {
+
+int dn_sac_actor_create(const dn_sac_actor_config* cfg, int device, const float* params, dn_sac_actor** out) {
+    if (!cfg || !params || !out) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: null argument");
+    *out = nullptr;
+    int rc;
+    if ((rc = sac_check_config(cfg))) return rc;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return dn_internal_fail(DN_ECUDA, "dn_sac_actor_create: no CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: bad device index");
+    PPO_CUDA(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    PPO_CUDA(cudaGetDeviceProperties(&prop, device));
+    if (prop.major != 10) return dn_internal_fail(DN_ECUDA, "dn_sac_actor_create: the kernels are sm_100a only (tcgen05 / TMEM / TMA)");
+
+    dn_sac_actor* h = new dn_sac_actor();
+    h->cfg = *cfg;
+    h->device = device;
+    h->passes = (cfg->precision == DN_MLP_BF16X3) ? 3 : 1;
+    h->sms = prop.multiProcessorCount;
+    g_num_sms = h->sms;
+    h->max_rows = cfg->max_rows;
+    h->params = params;
+    const long long R = h->max_rows;
+    auto bail = [&](int code) { dn_sac_actor_destroy(h); return code; };
+    Net& net = h->net;
+    net.L = cfg->n_hidden;
+    net.n[0] = XPAD;
+    if ((rc = dev_alloc(h, &h->x, 2 * R * XPAD))) return bail(rc);
+    net.h[0] = h->x;
+    for (int l = 1; l <= net.L; ++l) {
+        net.n[l] = cfg->hidden[l - 1];
+        net.w_off[l - 1] = cfg->w_off[l - 1];
+        net.b_off[l - 1] = cfg->b_off[l - 1];
+        if ((rc = dev_alloc(h, &net.h[l], 2 * R * net.n[l])) || (rc = dev_alloc(h, &net.w[l], 2LL * net.n[l] * net.n[l - 1]))) return bail(rc);
+    }
+    if ((rc = dev_alloc(h, &h->mu, R * cfg->act_dim)) || (rc = dev_alloc(h, &h->log_std, R * cfg->act_dim))) return bail(rc);
+    const Net* nets[1] = {&net};
+    if ((rc = build_plane_table(h, nets, 1, cfg->obs_dim))) return bail(rc);
+    if ((rc = sac_ensure_rows(h, h->max_rows))) return bail(rc);
+    if ((rc = dn_sac_actor_sync_weights(h, nullptr))) return bail(rc);
+    PPO_CUDA(cudaStreamSynchronize(nullptr));
+    *out = h;
+    return DN_OK;
+}
+
+int dn_sac_actor_destroy(dn_sac_actor* h) {
+    if (!h) return DN_OK;
+    cudaSetDevice(h->device);
+    for (void* p : h->allocs) cudaFree(p);
+    if (h->psegs_dev) cudaFree(h->psegs_dev);
+    if (h->pseg_of_block_dev) cudaFree(h->pseg_of_block_dev);
+    delete h;
+    return DN_OK;
+}
+
+int dn_sac_actor_sync_weights(dn_sac_actor* h, void* stream) {
+    if (!h) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_sync_weights: null handle");
+    planes_kernel<<<h->plane_blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(h->psegs_dev, h->pseg_of_block_dev, h->params, h->passes > 1);
+    PPO_CUDA(cudaGetLastError());
+    return DN_OK;
+}
+
+int dn_sac_act(dn_sac_actor* h, const float* obs, int32_t rows, const dn_sac_sample* s, float* action, float* log_prob, void* stream) {
+    if (!h || !obs || !s || !action) return dn_internal_fail(DN_EINVAL, "dn_sac_act: null argument");
+    if (s->mode != DN_SAC_SAMPLE && s->mode != DN_SAC_DETERMINISTIC && s->mode != DN_SAC_UNIFORM)
+        return dn_internal_fail(DN_EINVAL, "dn_sac_act: mode must be DN_SAC_SAMPLE, DN_SAC_DETERMINISTIC or DN_SAC_UNIFORM");
+    if (s->mode != DN_SAC_DETERMINISTIC && !s->counter) return dn_internal_fail(DN_EINVAL, "dn_sac_act: a drawing call needs the device counter (null counter)");
+    if (s->row_id_offset < 0) return dn_internal_fail(DN_EINVAL, "dn_sac_act: row_id_offset must be >= 0");
+    if (rows < 1) return dn_internal_fail(DN_EINVAL, "dn_sac_act: rows must be within max_rows");
+    if (rows > h->max_rows) return dn_internal_fail(DN_EINVAL, "dn_sac_act: rows must be within max_rows");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const long long* counter = reinterpret_cast<const long long*>(s->counter);
+    int rc;
+    if (s->mode == DN_SAC_UNIFORM) {
+        dnsac::sac_uniform_kernel<<<(rows + 255) / 256, 256, 0, st>>>(rows, h->cfg.act_dim, counter, s->seed, s->row_id_offset, action, log_prob);
+        PPO_CUDA(cudaGetLastError());
+    } else {
+        if ((rc = sac_ensure_rows(h, (rows + BM - 1) / BM * BM))) return rc;
+        GatherArgs g;
+        gather_obs_args(g, obs, rows, h->cfg.obs_dim, h->x, h->max_rows, h->passes);
+        if ((rc = launch_gather(g, st))) return rc;
+        for (int l = 1; l <= h->net.L; ++l)
+            if ((rc = launch_gemm(h->net.fwd[l], st))) return rc;
+        const Net& net = h->net;
+        const int n = net.n[net.L];
+        dnsac::SacHeadArgs a;
+        memset(&a, 0, sizeof(a));
+        a.rows = rows; a.n = n; a.mode = s->mode;
+        a.h_hi = net.h[net.L]; a.h_lo = (h->passes > 1) ? a.h_hi + static_cast<long long>(h->max_rows) * n : nullptr;
+        const dn_sac_actor_config& c = h->cfg;
+        a.w_mu = h->params + c.mu_w_off; a.b_mu = h->params + c.mu_b_off;
+        a.w_ls = h->params + c.log_std_w_off; a.b_ls = h->params + c.log_std_b_off;
+        a.mu = h->mu; a.log_std = h->log_std; a.action = action; a.log_prob = log_prob;
+        a.counter = (s->mode == DN_SAC_SAMPLE) ? counter : nullptr;
+        a.seed = s->seed; a.row_id_offset = s->row_id_offset;
+        const int blocks = std::min((rows + HEAD_WARPS - 1) / HEAD_WARPS, 3 * h->sms);
+        if ((rc = run_sac_head(c.act_dim, a, blocks, st))) return rc;
+    }
+    if (s->mode != DN_SAC_DETERMINISTIC) {
+        counter_advance_kernel<<<1, 32, 0, st>>>(reinterpret_cast<long long*>(s->counter));
+        PPO_CUDA(cudaGetLastError());
+    }
+    return DN_OK;
+}
+
+int dn_sac_actor_buffer(dn_sac_actor* h, const char* name, void** ptr, int64_t* elems) {
+    if (!h || !name || !ptr || !elems) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_buffer: null argument");
+    const long long R = h->max_rows;
+    const Net& net = h->net;
+    std::string s(name);
+    if (s == "x") { *ptr = h->x; *elems = 2 * R * XPAD; return DN_OK; }
+    if (s == "mu") { *ptr = h->mu; *elems = R * h->cfg.act_dim; return DN_OK; }
+    if (s == "log_std") { *ptr = h->log_std; *elems = R * h->cfg.act_dim; return DN_OK; }
+    if (s.size() == 2 && (s[0] == 'h' || s[0] == 'w')) {
+        const int l = s[1] - '0';
+        if (l >= 1 && l <= net.L) {
+            if (s[0] == 'h') { *ptr = net.h[l]; *elems = 2 * R * net.n[l]; }
+            else { *ptr = net.w[l]; *elems = 2LL * net.n[l] * net.n[l - 1]; }
+            return DN_OK;
+        }
+    }
+    return dn_internal_fail(DN_EINVAL, "dn_sac_actor_buffer: unknown buffer name");
 }
 
 }  // extern "C"

@@ -9,9 +9,13 @@ truncations not treated as terminal, next observation of a finished episode = it
 What changes is where the data lives: the replay buffer is a set of device tensors filled straight from the fused
 step kernel's outputs (no numpy hop, no per-env Python), and under ``torchrun`` every gradient step all-reduces two
 flat buckets (critics + log-alpha, actor) over NCCL -- the environment shards need no collective.
+With ``rollout_impl="fused"`` the collection phase samples the actor with the library's kernels (``dn_sac_act``,
+include/dnsac.h: Philox noise keyed by the global env id) and is replayed from one CUDA graph per phase; the gradient
+step is the same torch code either way.
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
 import time
 from dataclasses import dataclass
@@ -44,6 +48,12 @@ class SACConfig:
     seed: int = 42
     matmul_precision: str = "tf32"
     cuda_graph: bool = True        # replay each gradient step from three captured CUDA graphs (CUDA devices only)
+    rollout_impl: str = "torch"    # "torch": torch.Generator noise, one launch at a time; "fused": dn_sac_act (Philox noise keyed
+                                   # by the global env id), every collection phase after learning_starts replayed from a CUDA graph
+
+    def __post_init__(self):
+        if self.rollout_impl not in ("torch", "fused"):
+            raise ValueError(f"rollout_impl={self.rollout_impl!r}: 'torch' or 'fused'")
 
 
 def _relu_mlp(sizes, out_dim=None):
@@ -208,6 +218,121 @@ class ReplayBuffer:
         return flat(self.obs)[idx], flat(self.act)[idx], flat(self.rew)[idx], flat(self.next_obs)[idx], flat(self.done)[idx]
 
 
+class FusedSACActor:
+    """ctypes face of the dn_sac_actor handle (include/dnsac.h): SB3's Actor.forward with sampling as sm_100a kernels (the
+    latent ReLU layers on the tcgen05 contraction, heads and sampler in one CUDA-core kernel) on ONE flat FP32 parameter
+    vector.  The actor's ``Parameter`` s are views into that vector (:meth:`flatten`, before the optimisers are built), so
+    the torch gradient step, state dicts and checkpoints all see the memory the kernels read."""
+
+    @staticmethod
+    def shapes_ok(arch, obs_dim: int, act_dim: int) -> bool:
+        """The shapes dn_sac_actor_create accepts: 1..4 hidden layers, every width a multiple of 128 between 128 and 512,
+        1 <= obs_dim <= 64, 1 <= act_dim <= 4."""
+        arch = tuple(arch)
+        return 1 <= len(arch) <= 4 and all(w % 128 == 0 and 128 <= w <= 512 for w in arch) and 1 <= obs_dim <= 64 and 1 <= act_dim <= 4
+
+    @staticmethod
+    def check_supported(arch, obs_dim: int, act_dim: int, device) -> None:
+        dev = torch.device(device)
+        if dev.type != "cuda" or torch.cuda.get_device_capability(dev)[0] != 10:
+            raise RuntimeError(f"rollout_impl='fused' runs the SAC actor on sm_100a kernels: needs a compute-capability-10 CUDA device, "
+                               f"got {dev}")
+        if not FusedSACActor.shapes_ok(arch, obs_dim, act_dim):
+            raise RuntimeError(f"rollout_impl='fused': pi_arch={tuple(arch)}, obs_dim={obs_dim}, act_dim={act_dim} is not a shape "
+                               "dn_sac_actor_create accepts (1..4 hidden layers, widths multiples of 128 between 128 and 512, "
+                               "1 <= obs_dim <= 64, 1 <= act_dim <= 4)")
+
+    @staticmethod
+    def flatten(actor: "Actor") -> torch.Tensor:
+        """Re-seats the actor's parameters (latent layers, mu, log_std, SB3's order) as views of one new flat vector, values unchanged."""
+        ps = list(actor.parameters())
+        flat = torch.cat([p.detach().reshape(-1) for p in ps])
+        off = 0
+        for p in ps:
+            p.data = flat[off:off + p.numel()].view_as(p)
+            off += p.numel()
+        return flat
+
+    def __init__(self, actor: "Actor", flat: torch.Tensor, max_rows: int):
+        from . import _lib as L
+        self.L, self.lib = L, L.lib()
+        self.device, self.flat = flat.device, flat
+        self.max_rows = int(-(-max_rows // 128) * 128)
+        offs, off = {}, 0
+        for name, p in actor.named_parameters():
+            if p.data_ptr() != flat.data_ptr() + 4 * off:
+                raise RuntimeError(f"FusedSACActor: {name} is not a view of the flat parameter vector (FusedSACActor.flatten first)")
+            offs[name] = off
+            off += p.numel()
+        arch = [m.out_features for m in actor.latent if isinstance(m, nn.Linear)]
+        c = L.dn_sac_actor_config()
+        c.abi_version = L.DN_ABI_VERSION
+        c.obs_dim, c.act_dim, c.max_rows = actor.latent[0].in_features, actor.mu.out_features, self.max_rows
+        c.n_hidden = len(arch)
+        for l, w in enumerate(arch):            # nn.Sequential indices: Linear at 0, 2, 4, ... (ReLU in between)
+            c.hidden[l] = w
+            c.w_off[l], c.b_off[l] = offs[f"latent.{2 * l}.weight"], offs[f"latent.{2 * l}.bias"]
+        c.precision = L.DN_MLP_BF16X3
+        c.mu_w_off, c.mu_b_off = offs["mu.weight"], offs["mu.bias"]
+        c.log_std_w_off, c.log_std_b_off = offs["log_std.weight"], offs["log_std.bias"]
+        c.n_params = flat.numel()
+        self.cfg_c = c
+        self.handle = C.c_void_p()
+        with torch.cuda.device(self.device):
+            torch.cuda.synchronize(self.device)
+            L.check(self.lib.dn_sac_actor_create(C.byref(c), self.device.index or 0, flat.data_ptr(), C.byref(self.handle)),
+                    "dn_sac_actor_create")
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def close(self):
+        if getattr(self, "handle", None):
+            self.lib.dn_sac_actor_destroy(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:  # noqa: BLE001
+            pass
+
+    def sync_weights(self):
+        with torch.cuda.device(self.device):
+            self.L.check(self.lib.dn_sac_actor_sync_weights(self.handle, self._stream()), "dn_sac_actor_sync_weights")
+
+    def act(self, obs: torch.Tensor, sample, action: torch.Tensor = None, log_prob: torch.Tensor = None):
+        """dn_sac_act on `obs` [n, obs_dim]: action [n, act_dim] (and log_prob [n] when given).  `sample` is an
+        ``_lib.dn_sac_sample`` (seed, global id of row 0, device int64 draw counter, mode).  The BF16 planes are NOT refreshed
+        here: call :meth:`sync_weights` after the parameters change."""
+        n, A = obs.shape[0], self.cfg_c.act_dim
+        action = torch.empty(n, A, dtype=torch.float32, device=self.device) if action is None else action
+        for t, shape in ((obs, (n, self.cfg_c.obs_dim)), (action, (n, A))) + (((log_prob, (n,)),) if log_prob is not None else ()):
+            if t.dtype != torch.float32 or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape:
+                raise ValueError(f"dn_sac_act: expected a contiguous float32 tensor of shape {shape} on {self.device}")
+        with torch.cuda.device(self.device):
+            self.L.check(self.lib.dn_sac_act(self.handle, obs.data_ptr(), n, C.byref(sample), action.data_ptr(),
+                                             None if log_prob is None else log_prob.data_ptr(), self._stream()), "dn_sac_act")
+        return action
+
+    def buffer(self, name: str, rows: int) -> torch.Tensor:
+        """Test hook: the first `rows` rows of an internal buffer in FP32: "h1".."h4" (hi + lo of the BF16 planes of that
+        hidden layer), "mu", "log_std" (as the last non-uniform dn_sac_act left them)."""
+        ptr, elems = C.c_void_p(), C.c_int64()
+        self.L.check(self.lib.dn_sac_actor_buffer(self.handle, name.encode(), C.byref(ptr), C.byref(elems)), "dn_sac_actor_buffer")
+        n, planes = elems.value, name not in ("mu", "log_std")
+
+        class _Arr:      # __cuda_array_interface__ view of the library's allocation
+            pass
+        a = _Arr()
+        a.__cuda_array_interface__ = {"shape": (n,), "typestr": "<i2" if planes else "<f4", "data": (ptr.value, False), "version": 2}
+        raw = torch.as_tensor(a, device=self.device)
+        if not planes:
+            return raw.view(self.max_rows, -1)[:rows].clone()
+        p = raw.view(torch.bfloat16).view(2, self.max_rows, -1)[:, :rows]
+        return p[0].float() + p[1].float()
+
+
 class SACLearner:
     """Actor, twin critics + targets, log-alpha and the SAC update; independent of the environment."""
 
@@ -215,6 +340,10 @@ class SACLearner:
         self.cfg, self.device = cfg, torch.device(device)
         torch.manual_seed(cfg.seed)                         # same seed on every rank -> identical initial parameters
         self.actor = Actor(obs_dim, act_dim, cfg.pi_arch).to(self.device)
+        self.actor_flat, self.fused_actor = None, None
+        if cfg.rollout_impl == "fused":                     # before the optimisers: they hold the re-seated Parameters
+            FusedSACActor.check_supported(cfg.pi_arch, obs_dim, act_dim, self.device)
+            self.actor_flat = FusedSACActor.flatten(self.actor)
         self.critic = Critics(obs_dim, act_dim, cfg.qf_arch, cfg.n_critics).to(self.device)
         self.critic_target = Critics(obs_dim, act_dim, cfg.qf_arch, cfg.n_critics).to(self.device)
         self.critic_target.load_state_dict(self.critic.state_dict())
@@ -239,6 +368,16 @@ class SACLearner:
     @torch.no_grad()
     def act(self, obs, generator=None, deterministic=False):
         return self.actor(obs, generator=generator, deterministic=deterministic)[0]
+
+    def ensure_fused_actor(self, max_rows: int) -> FusedSACActor:
+        """The dn_sac_actor handle on this learner's actor (rollout_impl="fused"), created for at least `max_rows` rows."""
+        if self.actor_flat is None:
+            raise RuntimeError("ensure_fused_actor needs SACConfig(rollout_impl='fused')")
+        if self.fused_actor is None or self.fused_actor.max_rows < max_rows:
+            if self.fused_actor is not None:
+                self.fused_actor.close()
+            self.fused_actor = FusedSACActor(self.actor, self.actor_flat, max_rows)
+        return self.fused_actor
 
     # ---- one gradient step of SB3's SAC.train, in three stages around the two gradient all-reduces -----------------
     def _stage_critic(self, obs, act, rew, next_obs, done, eps_pi, eps_next, out):
@@ -369,9 +508,26 @@ class SACTrainer:
         self.buffer = ReplayBuffer(cfg.buffer_size, env.num_envs, env.obs_dim, 4, self.dev)
         self.obs = env.reset().clone()
         self.total_steps = 0
+        self.collect_graph = bool(cfg.cuda_graph)
+        self._collect_graph, self._collect_warm = None, False
+        if cfg.rollout_impl == "fused":
+            from . import _lib as L
+            self.fused = self.learner.ensure_fused_actor(env.num_envs)
+            # Philox draw counter on the device (advanced by every drawing dn_sac_act call, also inside graph replays); the key is
+            # the seed shared by all ranks and the subsequence the GLOBAL env id, so the noise does not depend on the sharding
+            self.draw_counter = torch.zeros(1, dtype=torch.int64, device=self.dev)
+            self.samplers = {}
+            for mode in (L.DN_SAC_SAMPLE, L.DN_SAC_UNIFORM):
+                s = L.dn_sac_sample()
+                s.seed, s.row_id_offset, s.counter, s.mode = int(cfg.seed), int(getattr(env, "env_id_offset", 0)), self.draw_counter.data_ptr(), mode
+                self.samplers[mode] = s
+            self.slot = torch.zeros(1, dtype=torch.int64, device=self.dev)     # replay-buffer row the next step writes (= buffer.pos)
+            self.action = torch.empty(env.num_envs, 4, dtype=torch.float32, device=self.dev)
 
     @torch.no_grad()
     def collect(self, n_steps: int):
+        if self.cfg.rollout_impl == "fused":
+            return self._collect_fused(n_steps)
         env, N = self.env, self.env.num_envs
         for _ in range(n_steps):
             if self.total_steps < self.cfg.learning_starts:      # SB3: uniform random actions before learning_starts
@@ -384,10 +540,67 @@ class SACTrainer:
             self.obs = obs.clone()
             self.total_steps += N * _world()
 
+    def _collect_step(self, mode: int):
+        """One env step of a fused phase: dn_sac_act on the current observation, env.step, the replay write at the device-side
+        slot (ReplayBuffer.add's arithmetic with torch ops), slot + 1.  Nothing here waits for the host."""
+        env, buf, s = self.env, self.buffer, self.slot
+        self.fused.act(self.obs, self.samplers[mode], self.action)
+        env.step(self.action)
+        buf.obs.index_copy_(0, s, self.obs.unsqueeze(0))
+        buf.next_obs.index_copy_(0, s, torch.where((env.done != 0).unsqueeze(-1), env.terminal_obs, env.obs).unsqueeze(0))
+        buf.act.index_copy_(0, s, self.action.unsqueeze(0))
+        buf.rew.index_copy_(0, s, env.reward.unsqueeze(0))
+        buf.done.index_copy_(0, s, ((env.done & 1) != 0).to(torch.float32).unsqueeze(0))
+        s.add_(1).remainder_(buf.cap)
+        self.obs.copy_(env.obs)
+
+    def _collect_fused(self, n_steps: int, graph: Optional[bool] = None):
+        """collect() on dn_sac_act.  A phase with a step before learning_starts runs launch by launch (uniform actions for those
+        steps, as SB3's action_space.sample()).  Every later phase is ONE CUDA graph -- weight refresh, then n_steps x (act,
+        env.step, replay write) -- captured at the second such phase (the first, launched, loads every kernel) and replayed from
+        then on.  The host keeps ReplayBuffer.pos / full by arithmetic; the slot tensor is set from pos before every phase."""
+        from . import _lib as L
+        cfg, buf = self.cfg, self.buffer
+        graph = self.collect_graph if graph is None else graph
+        per_step = self.env.num_envs * _world()
+        self.slot.fill_(buf.pos)
+        if self.total_steps < cfg.learning_starts:
+            self.fused.sync_weights()
+            for k in range(n_steps):
+                self._collect_step(L.DN_SAC_UNIFORM if self.total_steps + k * per_step < cfg.learning_starts else L.DN_SAC_SAMPLE)
+        else:
+            g = self._collect_graph
+            if graph and g is not None and g[0] == n_steps:
+                g[1].replay()
+            elif graph and self._collect_warm:
+                cg = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(cg):
+                    self.fused.sync_weights()
+                    for _ in range(n_steps):
+                        self._collect_step(L.DN_SAC_SAMPLE)
+                self._collect_graph = (n_steps, cg)
+                cg.replay()
+            else:
+                self.fused.sync_weights()
+                for _ in range(n_steps):
+                    self._collect_step(L.DN_SAC_SAMPLE)
+                self._collect_warm = True
+        for _ in range(n_steps):
+            buf.pos = (buf.pos + 1) % buf.cap
+            buf.full = buf.full or buf.pos == 0
+        self.total_steps += n_steps * per_step
+
     def train_iteration(self) -> Dict[str, float]:
         cfg = self.cfg
         t0 = time.perf_counter()
+        cuda = self.dev.type == "cuda"
+        if cuda:                     # device events: timing the collection needs no host synchronisation inside the iteration
+            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+            ev[0].record()
         self.collect(cfg.train_freq)
+        if cuda:
+            ev[1].record()
+        t_collect = time.perf_counter()
         out = {}
         grad_steps = 0
         if self.total_steps >= cfg.learning_starts and len(self.buffer) >= cfg.batch_size:
@@ -399,5 +612,6 @@ class SACTrainer:
         dt = time.perf_counter() - t0
         res = {k: float(v) for k, v in out.items()}
         res.update(samples=cfg.train_freq * self.env.num_envs * _world(), gradient_steps=grad_steps, seconds=dt,
-                   sps=cfg.train_freq * self.env.num_envs * _world() / dt)
+                   sps=cfg.train_freq * self.env.num_envs * _world() / dt,
+                   collect_s=ev[0].elapsed_time(ev[1]) / 1000.0 if cuda else t_collect - t0)
         return res

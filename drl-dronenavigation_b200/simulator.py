@@ -88,7 +88,8 @@ class PBDroneSimulator:
         same 12 x 4096 x (a few) samples per update unless --rollout_steps says otherwise."""
         if self.args.agent == "SAC":            # :290-331
             from .sac import SACConfig, SACTrainer
-            return SACTrainer(train_env, SACConfig())
+            impl = getattr(self.args, "rollout_impl", "torch")
+            return SACTrainer(train_env, SACConfig(rollout_impl=impl) if impl != "torch" else SACConfig())
         if self.args.agent != "PPO":
             raise NotImplementedError(f"{self.args.agent}: the PPO and SAC branches are built on the device path")
         n = train_env.num_envs
