@@ -76,8 +76,6 @@ struct GemmArgs {
     const float* bias2;
     float* partial2;
     float* colsum2;
-    int dbg;                        // DN_MLP_DBG (tools/micro/epilogue_probe.py only): 1 no activation math, 2 no staging / stores,
-                                    // 4 no MMAs (epilogue cost alone), 8 no epilogue TMEM loads
 };
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -472,7 +470,6 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                     const uint32_t sa = smem_u32(smem + stage * stage_bytes), sb = sa + planes * A_BYTES;
 #pragma unroll
                     for (int k = 0; k < BK / UK; ++k) {
-                        if (g.dbg & 4) break;
                         const uint64_t a_hi = (KIND == K_WGRAD) ? desc_mnmajor(sa, k) : desc_kmajor(sa, k);
                         const uint64_t b_hi = (KIND == K_FWD || KIND == K_FWD_RELU) ? desc_kmajor(sb, k) : desc_mnmajor(sb, k);
                         umma_bf16<CG>(d_tmem, a_hi, b_hi, IDESC, (kb | k) != 0);
@@ -536,7 +533,7 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                 const int col = tile_col(t, ci);
                 tmem_ld_wait(cur);
                 if (ci + 1 < CHUNKS) {
-                    if (!(g.dbg & 8)) tmem_ld32_issue(t_row + (ci + 1) * 32, nxt);   // in flight while this chunk is worked on
+                    tmem_ld32_issue(t_row + (ci + 1) * 32, nxt);    // in flight while this chunk is worked on
                 } else {
                     // the whole accumulator stage is in registers: hand it back to the MMA issuer before the last chunk's work
                     tc_fence_before();
@@ -562,11 +559,9 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                             v[4 * j4] += bb.x; v[4 * j4 + 1] += bb.y; v[4 * j4 + 2] += bb.z; v[4 * j4 + 3] += bb.w;
                         }
                         if constexpr (KIND == K_FWD_RELU) {
-                            if (!(g.dbg & 1)) {
 #pragma unroll
-                                for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.0f);
-                            }
-                        } else if (g.act && !(g.dbg & 1)) {
+                            for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.0f);
+                        } else if (g.act) {
 #pragma unroll
                             for (int j = 0; j < 32; ++j) v[j] = tanh_fast(v[j]);
                         }
@@ -610,17 +605,13 @@ umma_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                             v[2 * j + 1] *= fmaf(-h1, h1, 1.0f);
                         }
                     }
-                    if (!(g.dbg & 2)) {
-                        stage_split32(v, buf, lane, write_lo);
-                        fence_proxy_async();                 // generic-proxy writes -> visible to the TMA (async proxy)
-                        __syncwarp();
-                        if (lane == 0) {
-                            tma_store_2d(mC, buf, col, row0);
-                            if (write_lo) tma_store_2d(mC, buf + 2048, col, g.c_lo_row + row0);
-                            bulk_commit();
-                        }
-                    } else if (v[0] == 1.2345e-30f) {        // keeps the values alive
-                        *reinterpret_cast<volatile float*>(buf) = v[1];
+                    stage_split32(v, buf, lane, write_lo);
+                    fence_proxy_async();                     // generic-proxy writes -> visible to the TMA (async proxy)
+                    __syncwarp();
+                    if (lane == 0) {
+                        tma_store_2d(mC, buf, col, row0);
+                        if (write_lo) tma_store_2d(mC, buf + 2048, col, g.c_lo_row + row0);
+                        bulk_commit();
                     }
                     if constexpr (KIND == K_DGRAD) {
                         if (g.colsum != nullptr) {

@@ -366,147 +366,6 @@ step_kernel(const __grid_constant__ Params P, const __grid_constant__ StepIO io,
     if ((tid & 31) == 0) bulk_store_wait_read();   // shared memory must outlive the bulk read
 }
 
-// ---------------------------------------------------------------------------
-// EXPERIMENTAL (opt-in with DN_PIPE=1; measured SLOWER than step_kernel so far: 4 Mi envs, S = 8: 297 vs 235 us,
-// S = 1: 231 vs 196 us -- ncu: 15 % of SMSP time without a resident warp and 53 % DRAM utilisation, i.e. the
-// statically scheduled persistent CTAs stay phase-locked and leave a tail; DN_PIPE=k > 1 runs k contiguous tiles per
-// CTA on a normal grid instead: k = 2 is 1-3 % faster than step_kernel, k >= 4 slower; see DESIGN.md section 4).
-// Persistent, software-pipelined variant of the single-step kernel for large batches (>= 2 tiles per resident CTA).
-// In step_kernel all CTAs of an SM start together, load together, compute together and retire together, so the
-// load phase of every wave is exposed (ncu, 4 Mi envs, S = 8: no eligible warp in 20 % of the cycles although HBM is
-// at 69 % and the issue slots at 80 %).  Here each CTA walks tiles blockIdx.x, + gridDim.x, ... and keeps the NEXT
-// tile's inputs in flight with cp.async (LDGSTS) while it computes the current one:
-//   group C(t): actions + physics planes 0..3 of tile t  -> core_stage   (consumed at the top of iteration t)
-//   group A(t): bookkeeping planes 4..6 of tile t        -> aux_stage    (consumed after the last substep)
-// Every thread only ever touches its own 16-byte slots, so the pipeline needs no barrier: cp.async.wait_group 1
-// always leaves exactly the younger group in flight (order of commits: C(t0) A(t0) | C(t1) A(t1) | ...).
-// ---------------------------------------------------------------------------
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
-    const uint32_t dst = static_cast<uint32_t>(__cvta_generic_to_shared(smem_dst));
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(dst), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-
-template <int PHYS>
-__global__ void __launch_bounds__(kBlock, (kCtasPerSm * 7) / 8)
-step_kernel_pipe(const __grid_constant__ Params P, const __grid_constant__ StepIO io, const int num_tiles, const int tiles_per_cta) {
-    __shared__ __align__(128) float tile2[2][kBlock * kMaxObs];   // observation rows, double-buffered across iterations
-    __shared__ __align__(16) float4 core_stage[5 * kBlock];     // action | planes 0..3
-    __shared__ __align__(16) float4 aux_stage[3 * kBlock];      // planes 4..6
-    __shared__ __align__(16) float4 entry_stage[kBlock];        // plane 0 at step entry (the reset path needs the old position)
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    const int tid = threadIdx.x;
-    const int D = P.obs_dim;
-    int parity = 0;
-    BlockAcc acc = {0.f, 0, 0, 0, 0};
-
-    // tiles_per_cta > 0: this CTA owns the contiguous tiles [blockIdx.x * tiles_per_cta, +tiles_per_cta) and the grid is
-    // ceil(num_tiles / tiles_per_cta) (CTAs come and go, the hardware balances them); 0: persistent grid-stride walk
-    const int t_first = tiles_per_cta > 0 ? blockIdx.x * tiles_per_cta : blockIdx.x;
-    const int t_step = tiles_per_cta > 0 ? 1 : static_cast<int>(gridDim.x);
-    const int t_end = tiles_per_cta > 0 ? min(num_tiles, t_first + tiles_per_cta) : num_tiles;
-
-    auto issue_core = [&](int t) {
-        const int j = t * kBlock + tid;
-        if (t < t_end && j < P.n) {
-            cp_async16(&core_stage[tid], io.actions + j);
-#pragma unroll
-            for (int p = 0; p < 4; ++p) cp_async16(&core_stage[(p + 1) * kBlock + tid], &P.s[p][j]);
-        }
-        cp_async_commit();                                  // committed even when empty: keeps the group count uniform
-    };
-    auto issue_aux = [&](int t) {
-        const int j = t * kBlock + tid;
-        if (t < t_end && j < P.n) {
-#pragma unroll
-            for (int p = 0; p < 3; ++p) cp_async16(&aux_stage[p * kBlock + tid], &P.s[4 + p][j]);
-        }
-        cp_async_commit();
-    };
-    issue_core(t_first);
-    issue_aux(t_first);
-
-    for (int t = t_first; t < t_end; t += t_step) {
-        const int base = t * kBlock;
-        const int i = base + tid;
-        const bool active = i < P.n;
-        float* const tile = tile2[parity];
-        float* const obs_row = tile + tid * D;
-        parity ^= 1;
-        asm volatile("cp.async.wait_group 1;" ::: "memory");            // C(t) has landed; A(t) may still be in flight
-        EnvState s;
-        float last_rpm_sum = 0.0f;
-        if (active) {
-            const float4 act = core_stage[tid];
-            const float4 a = core_stage[kBlock + tid], b = core_stage[2 * kBlock + tid];
-            const float4 c = core_stage[3 * kBlock + tid], d = core_stage[4 * kBlock + tid];
-            s.px = a.x; s.py = a.y; s.pz = a.z; s.dist = a.w;
-            s.qx = b.x; s.qy = b.y; s.qz = b.z; s.qw = b.w;
-            s.vx = c.x; s.vy = c.y; s.vz = c.z; s.prev_dist = c.w;
-            s.wx = d.x; s.wy = d.y; s.wz = d.z; s.ep_ret = d.w;
-            if (PHYS & 1) last_rpm_sum = P.last_rpm_sum[i];
-            entry_stage[tid] = a;
-            issue_core(t + t_step);                                     // this thread's slots are free again
-            const StepResult r = env_step<PHYS>(P, i, s, act, last_rpm_sum, obs_row, &aux_stage[tid], kBlock, 1, &entry_stage[tid]);
-            issue_aux(t + t_step);                                      // A(t) was consumed inside env_step
-            store_state(P, i, s);
-            if (PHYS & 1) P.last_rpm_sum[i] = last_rpm_sum;
-            if (r.finished) {
-                if (io.terminal_obs) {
-                    float* term_out = io.terminal_obs + static_cast<size_t>(i) * D;
-#pragma unroll
-                    for (int k = 0; k < 12; ++k) term_out[k] = obs_row[k];
-                    if (D == 13) term_out[12] = obs_row[12];
-                }
-#pragma unroll
-                for (int k = 3; k < 12; ++k) obs_row[k] = P.init_obs[k];
-                obs_row[0] = r.spawn_obs[0]; obs_row[1] = r.spawn_obs[1]; obs_row[2] = r.spawn_obs[2];
-                if (D == 13) obs_row[12] = r.reset_obs_dist;
-                if (io.episode_return) io.episode_return[i] = r.ep_ret;
-                if (io.episode_length) io.episode_length[i] = r.ep_len;
-                acc.ret += r.ep_ret; acc.len += r.ep_len; acc.fnd += r.found;
-                acc.eps_suc += 1 + (r.success ? 0x10000 : 0);
-                acc.cra_tru += (r.crash ? 1 : 0) + ((r.done == DN_DONE_TRUNCATED) ? 0x10000 : 0);
-            }
-            io.reward[i] = r.reward;
-            io.done[i] = r.done;
-            if (io.found_targets) io.found_targets[i] = r.found;
-        } else {                                                        // keep the group accounting of idle lanes uniform
-            issue_core(t + t_step);
-            asm volatile("cp.async.wait_group 1;" ::: "memory");
-            issue_aux(t + t_step);
-        }
-        // observation rows of this warp: one TMA bulk store.  The two row buffers alternate, so before the next
-        // iteration only the store issued ONE ITERATION AGO must have been read by the bulk engine (wait_group.read 1):
-        // the warp never waits for the store it has just issued
-        const int wbase = base + (tid & ~31);
-        const int n_here = min(32, P.n - wbase);
-        if (n_here > 0) {
-            float* gdst = io.obs + static_cast<size_t>(wbase) * D;
-            const float* wsrc = tile + (tid & ~31) * D;
-            const uint32_t bytes = static_cast<uint32_t>(n_here) * D * 4u;
-            const bool bulk_ok = ((reinterpret_cast<uintptr_t>(gdst) & 15u) == 0) && ((bytes & 15u) == 0);
-            if (bulk_ok) {
-                fence_proxy_async_smem();
-                __syncwarp();
-                if ((tid & 31) == 0) {
-                    bulk_store_g2s_commit(gdst, wsrc, bytes);
-                    asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-                }
-                __syncwarp();
-            } else {
-                __syncwarp();
-                for (int j = (tid & 31); j < n_here * D; j += 32) gdst[j] = wsrc[j];
-                __syncwarp();
-            }
-        }
-    }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    flush_stats(P, acc, tid);
-    if ((tid & 31) == 0) bulk_store_wait_read();   // shared memory must outlive the bulk reads
-}
-
 // reduces the per-CTA slots into one Stats record (dn_episode_stats); optionally clears the slots
 __global__ void stats_reduce_kernel(BlockStats* slots, int n_slots, Stats* out, int clear) {
     __shared__ double s_ret[256];
@@ -737,10 +596,8 @@ struct dn_env {
     dn::BlockStats* d_block_stats; // one slot per CTA of the step grid
     int n_slots;
     int64_t launches;
-    int pipe_ctas;          // grid of the persistent pipelined kernel: SMs x resident CTAs per SM
     int sms;                // multiprocessor count of the device
     int full;               // 1: any optional feature is on (random spawn, another reward family, reward wrappers) -> FULL kernels
-    int use_pipe;           // DN_PIPE=1 at dn_create: opt into step_kernel_pipe for large batches (experimental, see DESIGN.md)
     float d0;
     // dn_step_host staging (allocated on first use)
     cudaStream_t host_stream;
@@ -760,7 +617,6 @@ struct dn_env {
     // zero-copy host call: completion word in pinned host memory, written by the last CTA of the step kernel
     unsigned int* zc_flag_h; unsigned int* zc_flag_d; unsigned int* zc_counter; unsigned int zc_seq;
     int zc_signal;          // launch_step: pass the completion word to the kernel (set around the zero-copy launch only)
-    int zc_signalled;       // the launch in flight announces completion through the word (else: poll the stream)
     // resident step server (dn_host_server): a dn_step_many kernel that stays on the GPU and takes one host command per step
     int srv_idle_us;        // > 0: dn_step_host on pinned + mapped buffers goes through the server
     int srv_alive;          // a server kernel has been launched on srv_stream and has not been seen to finish
@@ -797,15 +653,6 @@ struct DeviceGuard {   // switches the calling thread to the handle's device onl
     }
     ~DeviceGuard() { if (switched) cudaSetDevice(prev); }
 };
-
-// Lowest-latency completion wait for the host-buffer call: poll the stream instead of blocking in
-// cudaStreamSynchronize (the caller is a single-threaded step loop that has nothing else to do).
-inline cudaError_t spin_until_done(cudaStream_t st) {
-    cudaError_t e;
-    while ((e = cudaStreamQuery(st)) == cudaErrorNotReady) {}
-    return e;
-}
-
 }  // namespace
 
 extern "C" {
@@ -907,8 +754,6 @@ int dn_create(const dn_config* cfg, int device, dn_env** out) {
         if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) sms = prop.multiProcessorCount;
         P.prefetch_ctas = sms * dn::kCtasPerSm;  // 1024 resident threads per SM at 64 registers
         e->sms = sms;
-        e->pipe_ctas = sms * ((dn::kCtasPerSm * 7) / 8);   // step_kernel_pipe's launch bounds
-        e->use_pipe = getenv("DN_PIPE") ? std::max(1, atoi(getenv("DN_PIPE"))) : 0;
     }
     P.targets = e->d_targets; P.segs = e->d_segs; P.block_stats = e->d_block_stats;
 
@@ -984,8 +829,7 @@ static int launch_step(dn_env* env, const dn_step_io* io, int num_steps, int per
     // Programmatic dependent launch: the step kernel may be scheduled while the previous kernel of the stream is still
     // running (its CTAs trigger at entry); it then waits (griddepcontrol.wait, before its first global access) until that
     // kernel has completed and flushed.  Back-to-back steps -- plain or replayed from a CUDA graph -- thereby hide
-    // the launch / CTA-scheduling latency, which is a third of a 4096-env step.  DN_NO_PDL=1 disables it.
-    static const bool use_pdl = (getenv("DN_NO_PDL") == nullptr);
+    // the launch / CTA-scheduling latency, which is a third of a 4096-env step.
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -995,25 +839,9 @@ static int launch_step(dn_env* env, const dn_step_io* io, int num_steps, int per
     // two consecutive small grids each get SMs of their own.  With mid-size grids (0.3 - 1 wave) the early-resident
     // CTAs of the next step pile up on the SMs that had free slots, and the step then runs unbalanced (measured:
     // 65 536 envs 7.7 -> 9.8 us, 16 384 envs with drag / ground effect 7.4 -> 9.1 us per replayed step).
-    lc.attrs = attr; lc.numAttrs = (use_pdl && !env->no_pdl && !env->srv_launch && static_cast<int>(grid.x) * 2 <= env->sms) ? 1 : 0;
+    lc.attrs = attr; lc.numAttrs = (!env->no_pdl && !env->srv_launch && static_cast<int>(grid.x) * 2 <= env->sms) ? 1 : 0;
     k.pdl_prefetch = static_cast<int>(lc.numAttrs);
     cudaError_t lerr = cudaSuccess;
-    // large batches: persistent software-pipelined kernel (>= 2 tiles per resident CTA, single step, no fused obs-RMS)
-    const int tiles = (N + dn::kBlock - 1) / dn::kBlock;
-    if (env->use_pipe && num_steps == 1 && !env->normalize_obs && tiles >= 2 * env->pipe_ctas) {
-        const int tpc = env->use_pipe > 1 ? env->use_pipe : 0;       // DN_PIPE=1: persistent grid; DN_PIPE=k>1: k tiles per CTA
-        lc.gridDim = dim3(tpc ? (tiles + tpc - 1) / tpc : env->pipe_ctas);
-        switch (phys) {
-            case 0: lerr = cudaLaunchKernelEx(&lc, dn::step_kernel_pipe<0>, env->P, k, tiles, tpc); break;
-            case 1: lerr = cudaLaunchKernelEx(&lc, dn::step_kernel_pipe<1>, env->P, k, tiles, tpc); break;
-            case 2: lerr = cudaLaunchKernelEx(&lc, dn::step_kernel_pipe<2>, env->P, k, tiles, tpc); break;
-            default: lerr = cudaLaunchKernelEx(&lc, dn::step_kernel_pipe<3>, env->P, k, tiles, tpc); break;
-        }
-        DN_CUDA(lerr);
-        DN_CUDA(cudaGetLastError());
-        env->launches += 1;
-        return DN_OK;
-    }
 #define DN_LAUNCH(PH, NO)                                                                                              \
     do {                                                                                                               \
         if (env->full) {                                                                                               \
@@ -1054,7 +882,7 @@ int dn_step_many(dn_env* env, const dn_step_io* io, int num_steps, int per_step_
 static int host_classify(dn_env* env, const dn_step_io* h) {
     if (std::memcmp(&env->host_seen, h, sizeof(*h)) == 0) return DN_OK;
     env->host_seen = *h;
-    env->host_direct = getenv("DN_HOST_STAGED") ? 0 : 1;
+    env->host_direct = 1;
     const void* src[8] = {h->actions, h->obs, h->reward, h->done, h->terminal_obs, h->found_targets, h->episode_return, h->episode_length};
     void* dst[8] = {nullptr};
     for (int k = 0; k < 8 && env->host_direct; ++k) {
@@ -1082,35 +910,33 @@ static int host_classify(dn_env* env, const dn_step_io* h) {
     return DN_OK;
 }
 
-// One launch of the step kernel on the mapped host buffers.  Completion is announced through a pinned word that the last CTA
-// of the kernel writes after a system-scope fence (DN_HOST_POLL_STREAM=1: poll the stream instead, the first version).
+// The completion word of the zero-copy call and of the resident server: a pinned, device-mapped word that the last CTA of
+// the step kernel writes after a system-scope fence, and the device counter through which the CTAs find the last one.
+static int ensure_completion_word(dn_env* env) {
+    if (env->zc_flag_h) return DN_OK;
+    void* hp = nullptr; void* dp = nullptr;
+    DN_CUDA(cudaHostAlloc(&hp, 64, cudaHostAllocMapped));
+    DN_CUDA(cudaHostGetDevicePointer(&dp, hp, 0));
+    std::memset(hp, 0, 64);
+    env->zc_flag_h = static_cast<unsigned int*>(hp); env->zc_flag_d = static_cast<unsigned int*>(dp);
+    DN_CUDA(cudaMalloc(reinterpret_cast<void**>(&env->zc_counter), 64));
+    DN_CUDA(cudaMemset(env->zc_counter, 0, 64));
+    return DN_OK;
+}
+
+// One launch of the step kernel on the mapped host buffers; the kernel announces completion through the completion word.
 static int zero_copy_launch(dn_env* env) {
-    if (!env->zc_flag_h && !env->use_pipe) {
-        void* hp = nullptr; void* dp = nullptr;
-        DN_CUDA(cudaHostAlloc(&hp, 64, cudaHostAllocMapped));
-        DN_CUDA(cudaHostGetDevicePointer(&dp, hp, 0));
-        std::memset(hp, 0, 64);
-        env->zc_flag_h = static_cast<unsigned int*>(hp); env->zc_flag_d = static_cast<unsigned int*>(dp);
-        DN_CUDA(cudaMalloc(reinterpret_cast<void**>(&env->zc_counter), 64));
-        DN_CUDA(cudaMemset(env->zc_counter, 0, 64));
-    }
-    const bool signal = env->zc_flag_h != nullptr && getenv("DN_HOST_POLL_STREAM") == nullptr;
-    env->zc_signalled = signal ? 1 : 0;
-    if (signal) {
-        env->zc_seq += 1; if (env->zc_seq == 0u) env->zc_seq = 1u; env->zc_signal = 1;
-        // the word is shared with the resident server (its own sequence numbers): never start a wait on a stale equal value
-        if (*reinterpret_cast<volatile unsigned int*>(env->zc_flag_h) == env->zc_seq) *reinterpret_cast<volatile unsigned int*>(env->zc_flag_h) = 0u;
-    }
+    const int rw = ensure_completion_word(env);
+    if (rw != DN_OK) return rw;
+    env->zc_seq += 1; if (env->zc_seq == 0u) env->zc_seq = 1u; env->zc_signal = 1;
+    // the word is shared with the resident server (its own sequence numbers): never start a wait on a stale equal value
+    if (*reinterpret_cast<volatile unsigned int*>(env->zc_flag_h) == env->zc_seq) *reinterpret_cast<volatile unsigned int*>(env->zc_flag_h) = 0u;
     const int rc = launch_step(env, &env->host_mapped, 1, 1, env->host_stream);
     env->zc_signal = 0;
     return rc;
 }
 
 static int zero_copy_wait(dn_env* env) {
-    if (!env->zc_signalled) {
-        DN_CUDA(spin_until_done(env->host_stream));
-        return DN_OK;
-    }
     volatile unsigned int* flag = env->zc_flag_h;
     const unsigned int want = env->zc_seq;
     uint32_t spins = 0;
@@ -1177,15 +1003,8 @@ static int srv_step(dn_env* env) {
         const int rq = srv_quiesce(env);
         if (rq != DN_OK) return rq;
     }
-    if (!env->zc_flag_h) {
-        void* hp = nullptr; void* dp = nullptr;
-        DN_CUDA(cudaHostAlloc(&hp, 64, cudaHostAllocMapped));
-        DN_CUDA(cudaHostGetDevicePointer(&dp, hp, 0));
-        std::memset(hp, 0, 64);
-        env->zc_flag_h = static_cast<unsigned int*>(hp); env->zc_flag_d = static_cast<unsigned int*>(dp);
-        DN_CUDA(cudaMalloc(reinterpret_cast<void**>(&env->zc_counter), 64));
-        DN_CUDA(cudaMemset(env->zc_counter, 0, 64));
-    }
+    const int rw = ensure_completion_word(env);
+    if (rw != DN_OK) return rw;
     const unsigned int prev = env->srv_seq;
     const unsigned int seq = (prev % 0xFFFFu) + 1u;
     if (!env->srv_alive) {
@@ -1225,7 +1044,6 @@ int dn_host_server(dn_env* env, int idle_us) {
     // every CTA of the resident grid must fit on the device at once (they wait for each other's commands)
     const int grid = (env->P.n + dn::kBlock - 1) / dn::kBlock;
     if (idle_us > 0 && grid > 4 * env->sms) return fail(DN_EINVAL, "dn_host_server: more environments than a resident grid can hold (4 CTAs per SM)");
-    if (idle_us > 0 && env->use_pipe) return fail(DN_EINVAL, "dn_host_server: not with DN_PIPE");
     env->srv_idle_us = idle_us;
     return DN_OK;
 }

@@ -68,23 +68,12 @@ int make_map(CUtensorMap* m, const void* base, long long rows, long long cols, i
     return DN_OK;
 }
 
-int env_int(const char* name) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : 0;
-}
-
 // Tile shape of a contraction whose accumulator is `rows` x `n`: CTA pairs (CG = 2, 256 x BN tiles) whenever the row count
-// allows it, else single CTAs (128 x BN).  DN_MLP_CG=1 forces single CTAs, DN_MLP_BN=64|128|256 the tile width (experiments).
+// allows it, else single CTAs (128 x BN).
 void pick_tile(int rows, int n, int* cg, int* bn) {
-    static int forced_cg = -1, forced_bn = -1;
-    if (forced_cg < 0) { forced_cg = env_int("DN_MLP_CG"); forced_bn = env_int("DN_MLP_BN"); }
-    *cg = (rows % 256 == 0 && n % 128 == 0 && forced_cg != 1) ? 2 : 1;
+    *cg = (rows % 256 == 0 && n % 128 == 0) ? 2 : 1;
     if (*cg == 2) *bn = (n % 256 == 0) ? 256 : 128;
     else *bn = (n % 128 == 0) ? 128 : 64;
-    if (forced_bn == 64 || forced_bn == 128 || forced_bn == 256) {
-        const bool ok = n % forced_bn == 0 && ((*cg == 2) ? forced_bn >= 128 : forced_bn <= 128);
-        if (ok) *bn = forced_bn;
-    }
 }
 
 struct GemmPlan {       // one contraction, ready to launch
@@ -128,12 +117,11 @@ int launch_one(const GemmPlan& p, cudaStream_t st) {
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     // programmatic dependent launch: the kernel's set-up overlaps the tail of its predecessor in the stream (umma_gemm waits
-    // with griddepcontrol.wait before its first global access); DN_MLP_NO_PDL=1 launches normally (A/B measurements)
-    static const bool use_pdl = (getenv("DN_MLP_NO_PDL") == nullptr);
+    // with griddepcontrol.wait before its first global access)
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = use_pdl ? 2 : 1;
+    cfg.numAttrs = 2;
     if (p.args.groups == 2) PPO_CUDA(cudaLaunchKernelEx(&cfg, kern, p.ma, p.mb, p.mc, p.mh, p.ma2, p.mb2, p.mc2, p.mh2, p.args));
     else PPO_CUDA(cudaLaunchKernelEx(&cfg, kern, p.ma, p.mb, p.mc, p.mh, p.ma, p.mb, p.mc, p.mh, p.args));
     return DN_OK;
@@ -172,7 +160,6 @@ int plan_fwd(GemmPlan* p, int passes, int M, int N, int K, const void* a, const 
     memset(&g, 0, sizeof(g));
     g.m_tiles = rows_now / (BM * p->cg); g.n_tiles = N / p->bn; g.slices = 1; g.k_blocks = K / BK; g.passes = passes;
     g.a_lo_row = M; g.b_lo_row = N; g.c_lo_row = M; g.act = act; g.bias = bias; g.ld_out = N; g.groups = 1;
-    g.dbg = env_int("DN_MLP_DBG");
     set_grid(p);
     return DN_OK;
 }
@@ -190,7 +177,6 @@ int plan_dgrad(GemmPlan* p, int passes, int M, int N, int K, const void* a, cons
     memset(&g, 0, sizeof(g));
     g.m_tiles = rows_now / (BM * p->cg); g.n_tiles = N / p->bn; g.slices = 1; g.k_blocks = K / BK; g.passes = passes;
     g.a_lo_row = M; g.b_lo_row = K; g.c_lo_row = M; g.ld_out = N; g.groups = 1;
-    g.dbg = env_int("DN_MLP_DBG");
     set_grid(p);
     return DN_OK;
 }
@@ -437,7 +423,7 @@ int build_plane_table(H* h, const Net* const* nets, int n_nets, int obs_dim) {
 int ensure_rows(dn_ppo* h, int rows, bool train) {
     int rc;
     if (rows != h->cur_rows) {
-        bool same = h->pi.L == h->vf.L && getenv("DN_MLP_NO_GROUP") == nullptr;
+        bool same = h->pi.L == h->vf.L;
         for (int l = 1; same && l <= h->pi.L; ++l) same = h->pi.n[l] == h->vf.n[l];
         if ((rc = build_plans(h, h->pi, rows, same ? 2 : 1)) || (rc = build_plans(h, h->vf, rows, same ? 2 : 1))) return rc;
         for (int l = 1; same && l <= h->pi.L; ++l) {
@@ -448,7 +434,7 @@ int ensure_rows(dn_ppo* h, int rows, bool train) {
                 h->pi.dgrad[l].grid = h->vf.dgrad[l].grid = h->gdgrad[l].grid;
             }
         }
-        if (!same && h->pi.L == h->vf.L && getenv("DN_MLP_NO_GROUP") == nullptr) {
+        if (!same && h->pi.L == h->vf.L) {
             // shapes differ after all: plans with per-net slice counts
             if ((rc = build_plans(h, h->pi, rows, 1)) || (rc = build_plans(h, h->vf, rows, 1))) return rc;
         }

@@ -27,10 +27,7 @@
  *   - dn_step / dn_step_many launch small grids (at most half the SMs) with programmatic stream serialization
  *     (PDL): the grid may be scheduled
  *     while the previous kernel of the stream is still running, but it executes griddepcontrol.wait before
- *     its first global memory access, so stream-order semantics of all buffers are unchanged;
- *   - environment variables read by the library: DN_NO_PDL=1 (plain launches), DN_HOST_STAGED=1 (dn_step_host
- *     always stages through device buffers), DN_PIPE=1 at dn_create (experimental persistent pipelined kernel for
- *     batches of >= 2 tiles per resident CTA; slower than the default in all measurements so far).
+ *     its first global memory access, so stream-order semantics of all buffers are unchanged.
  */
 #ifndef DRONENAV_H_
 #define DRONENAV_H_
@@ -225,10 +222,10 @@ int dn_step_many(dn_env* env, const dn_step_io* io, int num_steps, int per_step_
 
 /* dn_step with HOST buffers (caller-owned; same shapes as dn_step_io).  Returns when the results are in
  * the host buffers.  Pinned, device-mapped buffers (cudaHostAlloc / cudaHostRegister / torch pin_memory)
- * are read and written by the fused kernel directly over PCIe (zero copy: one launch + one stream
- * synchronise); pageable buffers are staged (H2D actions -> kernel -> D2H outputs).  This is the call an
- * out-of-process / numpy caller such as SB3's VecEnv.step_wait makes; staging buffers and the stream
- * belong to the handle.  Set DN_HOST_STAGED=1 to force the staged path. */
+ * are read and written by the fused kernel directly over PCIe (zero copy: one launch, whose last CTA
+ * announces completion through a pinned word the call polls); pageable buffers are staged (H2D actions ->
+ * kernel -> D2H outputs).  This is the call an out-of-process / numpy caller such as SB3's VecEnv.step_wait
+ * makes; staging buffers and the stream belong to the handle. */
 int dn_step_host(dn_env* env, const dn_step_io* host_io);
 
 /* The lowest-latency form of the host-buffer call: the HANDLE owns one pinned host slab laid out

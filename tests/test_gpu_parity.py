@@ -608,47 +608,6 @@ def test_vec_env_collect_rollouts_text_format(tmp_path):
             assert all("e" not in c.lower() for c in cells[:13])      # positional notation, as the reference writes it
 
 
-def test_pipelined_kernel_matches_single_step_kernel(monkeypatch):
-    """With DN_PIPE=1, batches of >= 2 tiles per resident CTA take the (experimental) persistent cp.async-pipelined
-    kernel step_kernel_pipe; its rows must be bit-identical to the single-step kernel's on the same actions (head and
-    ragged tail of the batch), over enough steps for resets, and the Monitor statistics must add up."""
-    from drl_dronenavigation_b200.batched_env import BatchedDroneEnv
-    from oracle.dyn_oracle import make_reference_env
-    monkeypatch.setenv("DN_PIPE", "1")
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    N = 2 * sms * 1024 + 12345                          # above the switch-over (2 tiles per resident CTA), not a multiple of 128
-    M = 4096
-    ref = make_reference_env("reaching", pyb_freq=240, ctrl_freq=30)
-    mk = lambda n: BatchedDroneEnv(n, ref._target_points, aviary_dim=ref._aviary_dim, initial_xyzs=ref.INIT_XYZS, pyb_freq=240,
-                                   ctrl_freq=30, circle=False, include_distance=True, normalize_actions=True)
-    big = mk(N)
-    monkeypatch.delenv("DN_PIPE")
-    head, tail = mk(M), mk(M)
-    for e in (big, head, tail):
-        e.reset()
-    g = torch.Generator(device="cuda").manual_seed(7)
-    n_done = 0
-    for t in range(20):
-        a = torch.rand(N, 4, device="cuda", generator=g) * 2 - 1
-        if t % 2:
-            a = HOVER + 0.006 * a
-        o, r, d, f = big.step(a)
-        n_done += int((d != 0).sum())
-        for small, sl in ((head, slice(0, M)), (tail, slice(N - M, N))):
-            o2, r2, d2, f2 = small.step(a[sl].contiguous())
-            assert torch.equal(o[sl], o2) and torch.equal(r[sl], r2) and torch.equal(d[sl], d2) and torch.equal(f[sl], f2), t
-            done = d2 != 0
-            assert torch.equal(big.terminal_obs[sl][done], small.terminal_obs[done])
-            assert torch.equal(big.episode_return[sl][done], small.episode_return[done])
-    sb, sh = big.get_state(), head.get_state()
-    for k in sb:
-        assert torch.equal(sb[k][:M], sh[k]), k
-    st = big.episode_stats()
-    assert st["episodes"] == n_done > 0 and st["crashes"] + st["truncations"] + st["successes"] == n_done
-    for e in (big, head, tail):
-        e.close()
-
-
 def test_vec_env_save_and_load_running_stats(tmp_path):
     """eval_env.save(path) (PBDroneSimulator.py:746) and its counterpart: the per-env obs / reward statistics survive a
     round trip, so a restored env normalises the next observation exactly like the one that was saved."""

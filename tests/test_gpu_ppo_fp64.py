@@ -62,7 +62,6 @@ CONFIGS = {
                 dict(clip_range_vf=None, normalize_advantage=False, ent_coef=0.0, max_grad_norm=1e9), {}),
     "world2": (13, 4, (256, 128), (256, 128), 1024, 1024, {}, dict(world=2)),
     "bf16": (13, 4, A3, A3, 4096, 4096, dict(mlp_precision="bf16"), {}),
-    "nogroup": (13, 4, A3, A3, 4096, 4096, {}, dict(nogroup=True)),
 }
 
 
@@ -81,8 +80,6 @@ def _build(cid, monkeypatch):
                 p.add_(0.1 * torch.randn(p.shape, device="cuda", generator=g))
     spec = R.Spec(obs_dim, act_dim, pi, vf)
     ro = R.make_rollout(L.flat_parameters(), spec, max(max_rows, 2 * B), seed=B + act_dim, device="cuda")
-    if opt.get("nogroup"):
-        monkeypatch.setenv("DN_MLP_NO_GROUP", "1")          # read whenever the handle plans a row count
     with monkeypatch.context() as m:
         if opt.get("world"):
             m.setattr(ppo, "_world", lambda: opt["world"])     # the handle is configured for world_size ranks
