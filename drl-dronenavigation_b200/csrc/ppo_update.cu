@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <string>
 #include <vector>
 
@@ -84,28 +85,38 @@ struct GemmPlan {       // one contraction, ready to launch
     GemmArgs args;
 };
 
-int g_num_sms = 0;
-int num_sms() {
-    if (!g_num_sms) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (g_num_sms <= 0) g_num_sms = 148;
-    }
-    return g_num_sms;
+// persistent grid: one CTA (pair) per SM (pair) of a device with `sms` SMs, never more than there are tiles
+int grid_for(int tiles, int cg, int sms) { return std::max(1, std::min(tiles, sms / cg)) * cg; }
+
+typedef void (*GemmKernel)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap,
+                           GemmArgs);
+
+// the instantiation of umma_gemm for a kind and tile shape; nullptr if there is none
+GemmKernel gemm_kernel(int kind, int bn, int cg) {
+#define DN_CASE(K, B, G) \
+    if (kind == K && bn == B && cg == G) return umma_gemm<K, B, G>;
+    DN_CASE(K_FWD, 256, 2) DN_CASE(K_FWD, 128, 2) DN_CASE(K_FWD, 128, 1) DN_CASE(K_FWD, 64, 1)
+    DN_CASE(K_DGRAD, 256, 2) DN_CASE(K_DGRAD, 128, 2) DN_CASE(K_DGRAD, 128, 1) DN_CASE(K_DGRAD, 64, 1)
+    DN_CASE(K_WGRAD, 256, 2) DN_CASE(K_WGRAD, 128, 2) DN_CASE(K_WGRAD, 128, 1) DN_CASE(K_WGRAD, 64, 1)
+    DN_CASE(K_FWD_RELU, 256, 2) DN_CASE(K_FWD_RELU, 128, 2) DN_CASE(K_FWD_RELU, 128, 1) DN_CASE(K_FWD_RELU, 64, 1)
+#undef DN_CASE
+    return nullptr;
 }
 
-// persistent grid: one CTA (pair) per SM (pair), never more than there are tiles
-int grid_for(int tiles, int cg) { return std::max(1, std::min(tiles, num_sms() / cg)) * cg; }
+// umma_gemm needs more than the default 48 KB of dynamic shared memory.  That limit belongs to the function on the device that is
+// current when it is set, so it is set on every device that launches the kernel: by each handle on its own device at create time,
+// for every tile shape pick_tile can return.
+int allow_gemm_smem(std::initializer_list<int> kinds) {
+    const int tiles[4][2] = {{256, 2}, {128, 2}, {128, 1}, {64, 1}};
+    for (int kind : kinds)
+        for (const auto& t : tiles)
+            PPO_CUDA(cudaFuncSetAttribute(gemm_kernel(kind, t[0], t[1]), cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SMEM_BYTES)));
+    return DN_OK;
+}
 
-template <int KIND, int BN, int CG>
-int launch_one(const GemmPlan& p, cudaStream_t st) {
-    auto kern = umma_gemm<KIND, BN, CG>;
-    static bool attr_set = false;
-    if (!attr_set) {
-        PPO_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SMEM_BYTES)));
-        attr_set = true;
-    }
+int launch_gemm(const GemmPlan& p, cudaStream_t st) {
+    const GemmKernel kern = gemm_kernel(p.kind, p.bn, p.cg);
+    if (!kern) return dn_internal_fail(DN_EINVAL, "launch_gemm: no such kernel instantiation");
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(p.grid);
     cfg.blockDim = dim3(NUM_THREADS);
@@ -113,7 +124,7 @@ int launch_one(const GemmPlan& p, cudaStream_t st) {
     cfg.stream = st;
     cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CG;
+    attr[0].val.clusterDim.x = p.cg;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     // programmatic dependent launch: the kernel's set-up overlaps the tail of its predecessor in the stream (umma_gemm waits
@@ -127,25 +138,15 @@ int launch_one(const GemmPlan& p, cudaStream_t st) {
     return DN_OK;
 }
 
-int launch_gemm(const GemmPlan& p, cudaStream_t st) {
-#define DN_CASE(K, B, G) \
-    if (p.kind == K && p.bn == B && p.cg == G) return launch_one<K, B, G>(p, st);
-    DN_CASE(K_FWD, 256, 2) DN_CASE(K_FWD, 128, 2) DN_CASE(K_FWD, 128, 1) DN_CASE(K_FWD, 64, 1)
-    DN_CASE(K_DGRAD, 256, 2) DN_CASE(K_DGRAD, 128, 2) DN_CASE(K_DGRAD, 128, 1) DN_CASE(K_DGRAD, 64, 1)
-    DN_CASE(K_WGRAD, 256, 2) DN_CASE(K_WGRAD, 128, 2) DN_CASE(K_WGRAD, 128, 1) DN_CASE(K_WGRAD, 64, 1)
-    DN_CASE(K_FWD_RELU, 256, 2) DN_CASE(K_FWD_RELU, 128, 2) DN_CASE(K_FWD_RELU, 128, 1) DN_CASE(K_FWD_RELU, 64, 1)
-#undef DN_CASE
-    return dn_internal_fail(DN_EINVAL, "launch_gemm: no such kernel instantiation");
-}
-
 // Plans.  `*_planes` point at the hi plane; the lo plane starts `plane_rows * cols` elements later.  `rows_now` <= plane_rows
-// is the number of rows the launch covers (tile counts); the tensor maps always span the whole planes.
-void set_grid(GemmPlan* p) {
+// is the number of rows the launch covers (tile counts); the tensor maps always span the whole planes.  `sms`: SMs of the
+// device the plan launches on.
+void set_grid(GemmPlan* p, int sms) {
     const GemmArgs& g = p->args;
-    p->grid = grid_for(g.m_tiles * g.n_tiles * g.slices, p->cg);
+    p->grid = grid_for(g.m_tiles * g.n_tiles * g.slices, p->cg, sms);
 }
 // forward: out[M,N] = act(A[M,K] W[N,K]^T + bias); act 0 identity, 1 tanh, 2 ReLU (the K_FWD_RELU instantiations)
-int plan_fwd(GemmPlan* p, int passes, int M, int N, int K, const void* a, const void* w, const float* bias, int act, void* out,
+int plan_fwd(GemmPlan* p, int sms, int passes, int M, int N, int K, const void* a, const void* w, const float* bias, int act, void* out,
              int rows_now = 0) {
     if (!rows_now) rows_now = M;
     if (M % BM || rows_now % BM || N % 64 || K % 64) return dn_internal_fail(DN_EINVAL, "mlp forward: M % 128, N % 64, K % 64 must be 0");
@@ -160,11 +161,11 @@ int plan_fwd(GemmPlan* p, int passes, int M, int N, int K, const void* a, const 
     memset(&g, 0, sizeof(g));
     g.m_tiles = rows_now / (BM * p->cg); g.n_tiles = N / p->bn; g.slices = 1; g.k_blocks = K / BK; g.passes = passes;
     g.a_lo_row = M; g.b_lo_row = N; g.c_lo_row = M; g.act = act; g.bias = bias; g.ld_out = N; g.groups = 1;
-    set_grid(p);
+    set_grid(p, sms);
     return DN_OK;
 }
 // dgrad: out[M,N] = (A[M,K] W[K,N]) * (1 - H[M,N]^2)
-int plan_dgrad(GemmPlan* p, int passes, int M, int N, int K, const void* a, const void* w, const void* h, void* out, int rows_now = 0) {
+int plan_dgrad(GemmPlan* p, int sms, int passes, int M, int N, int K, const void* a, const void* w, const void* h, void* out, int rows_now = 0) {
     if (!rows_now) rows_now = M;
     if (M % BM || rows_now % BM || N % 64 || K % 64) return dn_internal_fail(DN_EINVAL, "mlp dgrad: M % 128, N % 64, K % 64 must be 0");
     p->kind = K_DGRAD;
@@ -177,11 +178,11 @@ int plan_dgrad(GemmPlan* p, int passes, int M, int N, int K, const void* a, cons
     memset(&g, 0, sizeof(g));
     g.m_tiles = rows_now / (BM * p->cg); g.n_tiles = N / p->bn; g.slices = 1; g.k_blocks = K / BK; g.passes = passes;
     g.a_lo_row = M; g.b_lo_row = K; g.c_lo_row = M; g.ld_out = N; g.groups = 1;
-    set_grid(p);
+    set_grid(p, sms);
     return DN_OK;
 }
 // wgrad: partial[s][Mo][No] = A[rows_s, Mo]^T B[rows_s, No], rows split into `slices`
-int plan_wgrad(GemmPlan* p, int passes, int Mo, int No, int rows, int slices, const void* a, const void* b, float* partial, int rows_now = 0) {
+int plan_wgrad(GemmPlan* p, int sms, int passes, int Mo, int No, int rows, int slices, const void* a, const void* b, float* partial, int rows_now = 0) {
     if (!rows_now) rows_now = rows;
     if (Mo % BM || No % 64 || slices < 1 || rows_now % 64 || rows_now / BK < slices)
         return dn_internal_fail(DN_EINVAL, "mlp wgrad: Mo % 128, No % 64, rows % 64 must be 0 and every slice needs at least one k-block");
@@ -196,13 +197,13 @@ int plan_wgrad(GemmPlan* p, int passes, int Mo, int No, int rows, int slices, co
     g.m_tiles = Mo / (BM * p->cg); g.n_tiles = No / p->bn; g.slices = slices; g.k_blocks = rows_now / BK; g.passes = passes;
     g.a_lo_row = rows; g.b_lo_row = rows;
     g.partial = partial; g.ld_partial = No; g.slice_stride = static_cast<long long>(Mo) * No; g.groups = 1;
-    set_grid(p);
+    set_grid(p, sms);
     return DN_OK;
 }
 
 // One launch for two problems of identical shape (layer l of the policy and of the value net): `out` = a's problem + b's.
 // false if the two plans differ in anything but their pointers.
-bool merge_plans(GemmPlan* out, const GemmPlan& a, const GemmPlan& b) {
+bool merge_plans(GemmPlan* out, const GemmPlan& a, const GemmPlan& b, int sms) {
     const GemmArgs &x = a.args, &y = b.args;
     if (a.kind != b.kind || a.bn != b.bn || a.cg != b.cg || x.m_tiles != y.m_tiles || x.n_tiles != y.n_tiles || x.slices != y.slices ||
         x.k_blocks != y.k_blocks || x.passes != y.passes || x.a_lo_row != y.a_lo_row || x.b_lo_row != y.b_lo_row || x.c_lo_row != y.c_lo_row ||
@@ -212,7 +213,7 @@ bool merge_plans(GemmPlan* out, const GemmPlan& a, const GemmPlan& b) {
     *out = a;
     out->ma2 = b.ma; out->mb2 = b.mb; out->mc2 = b.mc; out->mh2 = b.mh;
     out->args.groups = 2; out->args.bias2 = y.bias; out->args.partial2 = y.partial; out->args.colsum2 = y.colsum;
-    out->grid = grid_for(2 * x.m_tiles * x.n_tiles * x.slices, a.cg);
+    out->grid = grid_for(2 * x.m_tiles * x.n_tiles * x.slices, a.cg, sms);
     return true;
 }
 
@@ -234,15 +235,32 @@ struct Net {                      // one MLP (pi or vf)
     GemmPlan fwd[MAX_LAYERS + 1], dgrad[MAX_LAYERS + 1], wgrad[MAX_LAYERS + 1];
 };
 
+// What the PPO handle and the SAC actor share: the device, the observation planes the first layer reads, the table that
+// refreshes the BF16 weight planes from the flat FP32 parameters, and the device allocations, which go with the handle.
+struct MlpCore {
+    int device = 0, passes = 3, sms = 148;
+    int max_rows = 0, cur_rows = -1;   // cur_rows: the (padded) row count the forward plans were built for
+    float* params = nullptr;
+    __nv_bfloat16* x = nullptr;
+    PlaneSeg* psegs_dev = nullptr; int* pseg_of_block_dev = nullptr; int plane_blocks = 0;
+    std::vector<void*> allocs;
+    ~MlpCore() {                        // the handle's device is current
+        for (void* p : allocs) cudaFree(p);
+        if (psegs_dev) cudaFree(psegs_dev);
+        if (pseg_of_block_dev) cudaFree(pseg_of_block_dev);
+    }
+};
+
+typedef void (*HeadKernel)(HeadArgs);
+typedef void (*SacHeadKernel)(dnsac::SacHeadArgs);
+
 }  // namespace
 
-struct dn_ppo {
+struct dn_ppo : MlpCore {
     dn_ppo_config cfg;
-    int device = 0, passes = 3, sms = 148;
-    int max_rows = 0;
-    float *params = nullptr, *grads = nullptr, *exp_avg = nullptr, *exp_avg_sq = nullptr, *step = nullptr;
+    float *grads = nullptr, *exp_avg = nullptr, *exp_avg_sq = nullptr, *step = nullptr;
     Net pi, vf;
-    __nv_bfloat16* x = nullptr;
+    HeadKernel head[2] = {};        // head_kernel for this act_dim and width: [0] dn_ppo_forward / training, [1] sampling
     float *m_act = nullptr, *m_logp = nullptr, *m_val = nullptr, *m_adv = nullptr, *m_ret = nullptr;
     double *adv_partial = nullptr, *norm_partial = nullptr;
     float* head_partial = nullptr;
@@ -253,8 +271,7 @@ struct dn_ppo {
     int* mirror_dev = nullptr;
     Seg* segs_dev = nullptr; int* seg_of_block_dev = nullptr; int n_segs = 0, reduce_blocks = 0;
     std::vector<Seg> segs_host;
-    PlaneSeg* psegs_dev = nullptr; int* pseg_of_block_dev = nullptr; int plane_blocks = 0;
-    int cur_rows = -1, table_rows = -1;
+    int table_rows = -1;
     // the policy and the value net have the same hidden widths (PBDroneSimulator.py:251-258): layer l of both runs as ONE launch
     // gradient all-reduce over NVLink peer memory (ppo_comm.cuh); comm_base == nullptr: not set up
     char* comm_base = nullptr;
@@ -264,7 +281,14 @@ struct dn_ppo {
     std::vector<void*> comm_opened;
     bool grouped = false;
     GemmPlan gfwd[MAX_LAYERS + 1], gdgrad[MAX_LAYERS + 1], gwgrad[MAX_LAYERS + 1];
-    std::vector<void*> allocs;
+};
+
+// the SAC actor (include/dnsac.h): the latent ReLU layers on the forward contraction, then sac_head_kernel
+struct dn_sac_actor : MlpCore {
+    dn_sac_actor_config cfg;
+    Net net;                          // h, w and fwd of the latent layers (the training buffers stay unallocated)
+    SacHeadKernel head = nullptr;     // sac_head_kernel for this act_dim and width
+    float *mu = nullptr, *log_std = nullptr;
 };
 
 namespace {
@@ -277,14 +301,39 @@ int wgrad_slices(int rows, int tiles, int units) {
     return std::max(1, std::min(target, rows / 256));
 }
 
-template <typename H, typename T>
-int dev_alloc(H* h, T** p, size_t count) {
+template <typename T>
+int dev_alloc(MlpCore* h, T** p, size_t count) {
     void* q = nullptr;
     PPO_CUDA(cudaMalloc(&q, std::max<size_t>(count, 1) * sizeof(T)));
     PPO_CUDA(cudaMemset(q, 0, std::max<size_t>(count, 1) * sizeof(T)));
     h->allocs.push_back(q);
     *p = static_cast<T*>(q);
     return DN_OK;
+}
+
+// Makes `device` current after checking that it exists and is an sm_100 part; *sms = its SM count.  `who` (the entry point) and
+// `kernels` word the messages.
+int open_device(const char* who, const char* kernels, int device, int* sms) {
+    const std::string w(who);
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return dn_internal_fail(DN_ECUDA, w + ": no CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) return dn_internal_fail(DN_EINVAL, w + ": bad device index");
+    PPO_CUDA(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    PPO_CUDA(cudaGetDeviceProperties(&prop, device));
+    if (prop.major != 10) return dn_internal_fail(DN_ECUDA, w + ": " + kernels + " are sm_100a only (tcgen05 / TMEM / TMA)");
+    *sms = prop.multiProcessorCount;
+    return DN_OK;
+}
+
+// the shared part of a new handle on the device open_device made current, with its observation planes [2][max_rows][XPAD]
+int init_core(MlpCore* h, int device, int sms, int precision, int max_rows, float* params) {
+    h->device = device;
+    h->sms = sms;
+    h->passes = (precision == DN_MLP_BF16X3) ? 3 : 1;
+    h->max_rows = max_rows;
+    h->params = params;
+    return dev_alloc(h, &h->x, 2LL * max_rows * XPAD);
 }
 
 // tiles of the weight-gradient contraction of a layer [N, K] (accumulator N x K) and the CTAs (pairs) available for them
@@ -295,19 +344,23 @@ int wgrad_tiles(int N, int K, int sms, int* units) {
     return (N / (BM * cg)) * (K / bn);
 }
 
-int setup_net(dn_ppo* h, Net& net, int L, const int32_t* hidden, const int64_t* w_off, const int64_t* b_off) {
+// The hidden layers of one MLP: widths, flat offsets, activation and weight planes.  `train` adds the buffers of the backward
+// pass: pre-activation gradient planes and the partials of the weight and bias gradients.
+int setup_net(MlpCore* h, Net& net, int L, const int32_t* hidden, const int64_t* w_off, const int64_t* b_off, bool train) {
     net.L = L;
     net.n[0] = XPAD;
+    net.h[0] = h->x;
     const long long R = h->max_rows;
     int rc;
-    for (int l = 1; l <= L; ++l) net.n[l] = hidden[l - 1];
-    for (int l = 0; l <= L; ++l) { net.w_off[l] = w_off[l]; net.b_off[l] = b_off[l]; }
-    net.h[0] = h->x;
     for (int l = 1; l <= L; ++l) {
-        const int N = net.n[l], K = net.n[l - 1];
-        if ((rc = dev_alloc(h, &net.h[l], 2 * R * N)) || (rc = dev_alloc(h, &net.dz[l], 2 * R * N)) ||
+        const int N = hidden[l - 1], K = net.n[l - 1];
+        net.n[l] = N;
+        net.w_off[l - 1] = w_off[l - 1];
+        net.b_off[l - 1] = b_off[l - 1];
+        if ((rc = dev_alloc(h, &net.h[l], 2 * R * N)) || (train && (rc = dev_alloc(h, &net.dz[l], 2 * R * N))) ||
             (rc = dev_alloc(h, &net.w[l], 2LL * N * K)))
             return rc;
+        if (!train) continue;
         int units = 0;
         const int wt = wgrad_tiles(N, K, h->sms, &units);
         net.slices_max[l] = wgrad_slices(h->max_rows, wt, units);
@@ -319,21 +372,32 @@ int setup_net(dn_ppo* h, Net& net, int L, const int32_t* hidden, const int64_t* 
 }
 
 // Plans for `rows` rows: tensor maps over the full workspaces (lo plane max_rows rows after the hi plane), tile shapes and
-// counts for this row count (CTA pairs need multiples of 256 rows).
+// counts for this row count (CTA pairs need multiples of 256 rows).  plan_forward: the forward contractions of `net`, act 1 tanh
+// (the PPO nets) or 2 ReLU (the SAC actor); build_plans adds the backward contractions of a PPO net.
+int plan_forward(const MlpCore* h, Net& net, int rows, int act) {
+    int rc;
+    for (int l = 1; l <= net.L; ++l)
+        if ((rc = plan_fwd(&net.fwd[l], h->sms, h->passes, h->max_rows, net.n[l], net.n[l - 1], net.h[l - 1], net.w[l],
+                           h->params + net.b_off[l - 1], act, net.h[l], rows)))
+            return rc;
+    return DN_OK;
+}
+
 int build_plans(dn_ppo* h, Net& net, int rows, int groups) {
     int rc;
+    if ((rc = plan_forward(h, net, rows, 1))) return rc;
     for (int l = 1; l <= net.L; ++l) {
         const int N = net.n[l], K = net.n[l - 1];
-        const float* bias = h->params + net.b_off[l - 1];
-        if ((rc = plan_fwd(&net.fwd[l], h->passes, h->max_rows, N, K, net.h[l - 1], net.w[l], bias, 1, net.h[l], rows))) return rc;
         if (l > 1) {
-            if ((rc = plan_dgrad(&net.dgrad[l], h->passes, h->max_rows, K, N, net.dz[l], net.w[l], net.h[l - 1], net.dz[l - 1], rows))) return rc;
+            if ((rc = plan_dgrad(&net.dgrad[l], h->sms, h->passes, h->max_rows, K, N, net.dz[l], net.w[l], net.h[l - 1], net.dz[l - 1], rows)))
+                return rc;
             net.dgrad[l].args.colsum = net.bpart[l - 1];      // bias gradient of layer l-1 = column sums of dz[l-1], per CTA
         }
         int units = 0;
         const int wt = wgrad_tiles(N, K, h->sms, &units);
         const int slices = std::min(wgrad_slices(rows, wt * groups, units), net.slices_max[l]);   // one work item per CTA (pair) per launch
-        if ((rc = plan_wgrad(&net.wgrad[l], h->passes, N, K, h->max_rows, slices, net.dz[l], net.h[l - 1], net.wpart[l], rows))) return rc;
+        if ((rc = plan_wgrad(&net.wgrad[l], h->sms, h->passes, N, K, h->max_rows, slices, net.dz[l], net.h[l - 1], net.wpart[l], rows)))
+            return rc;
     }
     return DN_OK;
 }
@@ -393,8 +457,7 @@ int build_reduce_table(dn_ppo* h, int rows) {
 }
 
 // the table planes_kernel walks: every hidden weight of `nets` -> its BF16 planes
-template <typename H>
-int build_plane_table(H* h, const Net* const* nets, int n_nets, int obs_dim) {
+int build_plane_table(MlpCore* h, const Net* const* nets, int n_nets, int obs_dim) {
     std::vector<PlaneSeg> v;
     std::vector<int> sob;
     for (int k = 0; k < n_nets; ++k) {
@@ -419,6 +482,25 @@ int build_plane_table(H* h, const Net* const* nets, int n_nets, int obs_dim) {
     return DN_OK;
 }
 
+// FP32 parameters -> the BF16 weight planes the contractions read
+int refresh_planes(const MlpCore* h, cudaStream_t st) {
+    planes_kernel<<<h->plane_blocks, 256, 0, st>>>(h->psegs_dev, h->pseg_of_block_dev, h->params, h->passes > 1);
+    PPO_CUDA(cudaGetLastError());
+    return DN_OK;
+}
+
+int check_rows(const MlpCore* h, const char* who, int rows) {
+    if (rows < 1 || rows > h->max_rows) return dn_internal_fail(DN_EINVAL, std::string(who) + ": rows must be within max_rows");
+    return DN_OK;
+}
+
+// a drawing call's one step of the device draw counter (enqueued, so graph replays advance it too)
+int advance_counter(void* counter, cudaStream_t st) {
+    counter_advance_kernel<<<1, 32, 0, st>>>(static_cast<long long*>(counter));
+    PPO_CUDA(cudaGetLastError());
+    return DN_OK;
+}
+
 // (re)plans the contractions for `rows` rows; the reduction table of the partial gradients only when training with a new row count
 int ensure_rows(dn_ppo* h, int rows, bool train) {
     int rc;
@@ -427,9 +509,10 @@ int ensure_rows(dn_ppo* h, int rows, bool train) {
         for (int l = 1; same && l <= h->pi.L; ++l) same = h->pi.n[l] == h->vf.n[l];
         if ((rc = build_plans(h, h->pi, rows, same ? 2 : 1)) || (rc = build_plans(h, h->vf, rows, same ? 2 : 1))) return rc;
         for (int l = 1; same && l <= h->pi.L; ++l) {
-            same = merge_plans(&h->gfwd[l], h->pi.fwd[l], h->vf.fwd[l]) && merge_plans(&h->gwgrad[l], h->pi.wgrad[l], h->vf.wgrad[l]);
+            same = merge_plans(&h->gfwd[l], h->pi.fwd[l], h->vf.fwd[l], h->sms) &&
+                   merge_plans(&h->gwgrad[l], h->pi.wgrad[l], h->vf.wgrad[l], h->sms);
             if (same && l > 1) {
-                same = merge_plans(&h->gdgrad[l], h->pi.dgrad[l], h->vf.dgrad[l]);
+                same = merge_plans(&h->gdgrad[l], h->pi.dgrad[l], h->vf.dgrad[l], h->sms);
                 // the reduction table sums one column-sum row per CTA of the launch that wrote them
                 h->pi.dgrad[l].grid = h->vf.dgrad[l].grid = h->gdgrad[l].grid;
             }
@@ -448,42 +531,51 @@ int ensure_rows(dn_ppo* h, int rows, bool train) {
     return DN_OK;
 }
 
-template <int ACT, int NP, bool SAMPLE>
-int launch_head(dn_ppo* h, const HeadArgs& a, int blocks, cudaStream_t st) {
-    static bool attr = false;
-    if (!attr) {
-        PPO_CUDA(cudaFuncSetAttribute(head_kernel<ACT, NP, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        attr = true;
+// f(NP) for the head kernels' NP = column pairs per lane = width / 64, rounded up to the instantiated 2, 4 or 8 (widths are
+// multiples of 128, at most 512)
+template <typename F>
+auto with_np(int width, F&& f) {
+    const int np = width / 64;
+    if (np <= 2) return f(std::integral_constant<int, 2>());
+    if (np <= 4) return f(std::integral_constant<int, 4>());
+    return f(std::integral_constant<int, 8>());
+}
+
+// the PPO head for act_dim 1, 3 or 4 and the wider of the two last hidden layers; `sample`: dn_ppo_act's instantiation
+HeadKernel ppo_head_for(int act_dim, int width, bool sample) {
+    return with_np(width, [&](auto np) -> HeadKernel {
+        constexpr int NP = decltype(np)::value;
+        switch (act_dim) {
+            case 1: return sample ? head_kernel<1, NP, true> : head_kernel<1, NP, false>;
+            case 3: return sample ? head_kernel<3, NP, true> : head_kernel<3, NP, false>;
+            case 4: return sample ? head_kernel<4, NP, true> : head_kernel<4, NP, false>;
+            default: return nullptr;
+        }
+    });
+}
+
+// h->head: the two instantiations for this handle's act_dim and width, allowed the dynamic shared memory head_smem may take (at
+// most 200 KB) on the handle's device
+int setup_heads(dn_ppo* h, int width) {
+    for (int s = 0; s < 2; ++s) {
+        h->head[s] = ppo_head_for(h->cfg.act_dim, width, s);
+        PPO_CUDA(cudaFuncSetAttribute(h->head[s], cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     }
-    head_kernel<ACT, NP, SAMPLE><<<blocks, HEAD_WARPS * 32, h->head_smem, st>>>(a);
+    return DN_OK;
+}
+
+// a.out_action set: the sampling instantiation (dn_ppo_act)
+int run_head(dn_ppo* h, const HeadArgs& a, int blocks, cudaStream_t st) {
+    h->head[a.out_action != nullptr]<<<blocks, HEAD_WARPS * 32, h->head_smem, st>>>(a);
     PPO_CUDA(cudaGetLastError());
     return DN_OK;
 }
 
-template <int ACT, bool SAMPLE>
-int run_head_np(dn_ppo* h, HeadArgs& a, int blocks, cudaStream_t st) {
-    const int np = std::max(a.n_pi, a.n_vf) / 64;       // widths are multiples of 128
-    if (np <= 2) return launch_head<ACT, 2, SAMPLE>(h, a, blocks, st);
-    if (np <= 4) return launch_head<ACT, 4, SAMPLE>(h, a, blocks, st);
-    return launch_head<ACT, 8, SAMPLE>(h, a, blocks, st);
-}
-
-// a.out_action set: the sampling instantiations (dn_ppo_act)
-int run_head(dn_ppo* h, HeadArgs& a, int blocks, cudaStream_t st) {
-    const bool s = a.out_action != nullptr;
-    switch (h->cfg.act_dim) {
-        case 1: return s ? run_head_np<1, true>(h, a, blocks, st) : run_head_np<1, false>(h, a, blocks, st);
-        case 3: return s ? run_head_np<3, true>(h, a, blocks, st) : run_head_np<3, false>(h, a, blocks, st);
-        case 4: return s ? run_head_np<4, true>(h, a, blocks, st) : run_head_np<4, false>(h, a, blocks, st);
-        default: return dn_internal_fail(DN_EINVAL, "dn_ppo: act_dim must be 1, 3 or 4");
-    }
-}
-
 // observation rows -> the padded BF16 planes `x` [2][max_rows][XPAD] the first layer reads
-void gather_obs_args(GatherArgs& g, const float* obs, int rows, int obs_dim, __nv_bfloat16* x, int max_rows, int passes) {
+void gather_obs_args(GatherArgs& g, const MlpCore* h, const float* obs, int rows, int obs_dim) {
     memset(&g, 0, sizeof(g));
     g.obs = obs; g.rows = rows; g.obs_dim = obs_dim;
-    g.x_hi = x; g.x_lo = (passes > 1) ? x + static_cast<long long>(max_rows) * XPAD : nullptr;
+    g.x_hi = h->x; g.x_lo = (h->passes > 1) ? h->x + static_cast<long long>(h->max_rows) * XPAD : nullptr;
 }
 int launch_gather(const GatherArgs& g, cudaStream_t st) {
     const int blocks = (g.rows * 8 + 255) / 256;
@@ -494,7 +586,7 @@ int launch_gather(const GatherArgs& g, cudaStream_t st) {
 
 int run_gather(dn_ppo* h, const float* obs, const dn_ppo_rollout* r, const long long* idx, int rows, bool train, cudaStream_t st) {
     GatherArgs g;
-    gather_obs_args(g, obs, rows, h->cfg.obs_dim, h->x, h->max_rows, h->passes);
+    gather_obs_args(g, h, obs, rows, h->cfg.obs_dim);
     g.idx = idx; g.act_dim = h->cfg.act_dim;
     if (train) {
         g.act = r->actions; g.logp = r->old_log_prob; g.val = r->old_values; g.adv = r->advantages; g.ret = r->returns;
@@ -504,6 +596,13 @@ int run_gather(dn_ppo* h, const float* obs, const dn_ppo_rollout* r, const long 
     return launch_gather(g, st);
 }
 
+int launch_forward(const Net& net, cudaStream_t st) {
+    int rc;
+    for (int l = 1; l <= net.L; ++l)
+        if ((rc = launch_gemm(net.fwd[l], st))) return rc;
+    return DN_OK;
+}
+
 int run_forward_chain(dn_ppo* h, cudaStream_t st) {
     int rc;
     if (h->grouped) {
@@ -511,11 +610,8 @@ int run_forward_chain(dn_ppo* h, cudaStream_t st) {
             if ((rc = launch_gemm(h->gfwd[l], st))) return rc;
         return DN_OK;
     }
-    Net* nets[2] = {&h->pi, &h->vf};
-    for (Net* net : nets)
-        for (int l = 1; l <= net->L; ++l)
-            if ((rc = launch_gemm(net->fwd[l], st))) return rc;
-    return DN_OK;
+    if ((rc = launch_forward(h->pi, st))) return rc;
+    return launch_forward(h->vf, st);
 }
 
 void fill_head_common(dn_ppo* h, HeadArgs& a, int rows) {
@@ -531,6 +627,19 @@ void fill_head_common(dn_ppo* h, HeadArgs& a, int rows) {
     a.partial_size = h->head_psize;
 }
 
+// the BF16 plane pairs of `net` the buffer entry points expose: "h<l>", "w<l>" and, of a training net, "dz<l>"
+bool find_planes(const MlpCore* h, const Net& net, const std::string& s, void** ptr, int64_t* elems) {
+    const int l = s.empty() ? 0 : s.back() - '0';
+    if (l < 1 || l > net.L) return false;
+    const std::string kind = s.substr(0, s.size() - 1);
+    const long long R = h->max_rows;
+    if (kind == "h") { *ptr = net.h[l]; *elems = 2 * R * net.n[l]; }
+    else if (kind == "w") { *ptr = net.w[l]; *elems = 2LL * net.n[l] * net.n[l - 1]; }
+    else if (kind == "dz" && net.dz[l]) { *ptr = net.dz[l]; *elems = 2 * R * net.n[l]; }
+    else return false;
+    return true;
+}
+
 }  // namespace
 
 extern "C" {
@@ -539,24 +648,21 @@ int dn_mlp_gemm(int kind, int passes, int M, int N, int K, int slices, const voi
                 const void* h, void* out, float* partial, void* stream) {
     if (passes != 1 && passes != 3) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: passes must be 1 or 3");
     if (!a || !b) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: null operand");
+    if (kind == 0 && (!bias || !out)) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: forward needs bias and out");
+    if (kind == 1 && (!h || !out)) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: dgrad needs h and out");
+    if (kind == 2 && !partial) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: wgrad needs partial");
+    if (kind < 0 || kind > 2) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: kind must be 0, 1 or 2");
+    // the contraction runs on the caller's current device: its SM count sizes the grid, and the kernel gets its shared memory there
+    int dev = 0, sms = 0;
+    PPO_CUDA(cudaGetDevice(&dev));
+    PPO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     GemmPlan p;
-    int rc;
-    if (kind == 0) {
-        if (!bias || !out) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: forward needs bias and out");
-        rc = plan_fwd(&p, passes, M, N, K, a, b, bias, act, out);
-    } else if (kind == 1) {
-        if (!h || !out) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: dgrad needs h and out");
-        rc = plan_dgrad(&p, passes, M, N, K, a, b, h, out);
-    } else if (kind == 2) {
-        if (!partial) return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: wgrad needs partial");
-        rc = plan_wgrad(&p, passes, M, N, K, slices, a, b, partial);
-    } else {
-        return dn_internal_fail(DN_EINVAL, "dn_mlp_gemm: kind must be 0, 1 or 2");
-    }
-    if (rc) return rc;
+    int rc = (kind == 0) ? plan_fwd(&p, sms, passes, M, N, K, a, b, bias, act, out)
+           : (kind == 1) ? plan_dgrad(&p, sms, passes, M, N, K, a, b, h, out)
+                         : plan_wgrad(&p, sms, passes, M, N, K, slices, a, b, partial);
+    if (rc || (rc = allow_gemm_smem({p.kind}))) return rc;
     return launch_gemm(p, static_cast<cudaStream_t>(stream));
 }
-
 
 int dn_ppo_create(const dn_ppo_config* cfg, int device, float* params, float* grads, float* exp_avg, float* exp_avg_sq, float* step,
                   dn_ppo** out) {
@@ -580,29 +686,20 @@ int dn_ppo_create(const dn_ppo_config* cfg, int device, float* params, float* gr
         return dn_internal_fail(DN_EINVAL, "dn_ppo_create: the last hidden layer may be at most 512 wide");
     if (cfg->precision != DN_MLP_BF16X3 && cfg->precision != DN_MLP_BF16) return dn_internal_fail(DN_EINVAL, "dn_ppo_create: unknown precision");
     if (cfg->world_size < 1) return dn_internal_fail(DN_EINVAL, "dn_ppo_create: world_size must be >= 1");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return dn_internal_fail(DN_ECUDA, "dn_ppo_create: no CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) return dn_internal_fail(DN_EINVAL, "dn_ppo_create: bad device index");
-    PPO_CUDA(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    PPO_CUDA(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) return dn_internal_fail(DN_ECUDA, "dn_ppo_create: the update kernels are sm_100a only (tcgen05 / TMEM / TMA)");
+    int sms = 0, rc;
+    if ((rc = open_device("dn_ppo_create", "the update kernels", device, &sms))) return rc;
 
     dn_ppo* h = new dn_ppo();
-    h->cfg = *cfg;
-    h->device = device;
-    h->passes = (cfg->precision == DN_MLP_BF16X3) ? 3 : 1;
-    h->sms = prop.multiProcessorCount;
-    g_num_sms = h->sms;
-    h->max_rows = cfg->max_rows;
-    h->params = params; h->grads = grads; h->exp_avg = exp_avg; h->exp_avg_sq = exp_avg_sq; h->step = step;
-    const long long R = h->max_rows;
-    const int A = cfg->act_dim;
-    int rc = DN_OK;
     auto bail = [&](int code) { dn_ppo_destroy(h); return code; };
-    if ((rc = dev_alloc(h, &h->x, 2 * R * XPAD))) return bail(rc);
-    if ((rc = setup_net(h, h->pi, cfg->n_pi, cfg->pi_hidden, cfg->pi_w_off, cfg->pi_b_off))) return bail(rc);
-    if ((rc = setup_net(h, h->vf, cfg->n_vf, cfg->vf_hidden, cfg->vf_w_off, cfg->vf_b_off))) return bail(rc);
+    h->cfg = *cfg;
+    h->grads = grads; h->exp_avg = exp_avg; h->exp_avg_sq = exp_avg_sq; h->step = step;
+    const long long R = cfg->max_rows;
+    const int A = cfg->act_dim;
+    if ((rc = init_core(h, device, sms, cfg->precision, cfg->max_rows, params))) return bail(rc);
+    if ((rc = setup_net(h, h->pi, cfg->n_pi, cfg->pi_hidden, cfg->pi_w_off, cfg->pi_b_off, true))) return bail(rc);
+    if ((rc = setup_net(h, h->vf, cfg->n_vf, cfg->vf_hidden, cfg->vf_w_off, cfg->vf_b_off, true))) return bail(rc);
+    h->pi.w_off[cfg->n_pi] = cfg->pi_w_off[cfg->n_pi]; h->pi.b_off[cfg->n_pi] = cfg->pi_b_off[cfg->n_pi];    // index L: the heads
+    h->vf.w_off[cfg->n_vf] = cfg->vf_w_off[cfg->n_vf]; h->vf.b_off[cfg->n_vf] = cfg->vf_b_off[cfg->n_vf];
     if ((rc = dev_alloc(h, &h->m_act, R * A)) || (rc = dev_alloc(h, &h->m_logp, R)) || (rc = dev_alloc(h, &h->m_val, R)) ||
         (rc = dev_alloc(h, &h->m_adv, R)) || (rc = dev_alloc(h, &h->m_ret, R)))
         return bail(rc);
@@ -629,6 +726,7 @@ int dn_ppo_create(const dn_ppo_config* cfg, int device, float* params, float* gr
         const Net* nets[2] = {&h->pi, &h->vf};
         if ((rc = build_plane_table(h, nets, 2, cfg->obs_dim))) return bail(rc);
     }
+    if ((rc = allow_gemm_smem({K_FWD, K_DGRAD, K_WGRAD})) || (rc = setup_heads(h, std::max(npi, nvf)))) return bail(rc);
     if ((rc = ensure_rows(h, h->max_rows, true))) return bail(rc);
     if ((rc = dn_ppo_sync_weights(h, nullptr))) return bail(rc);
     PPO_CUDA(cudaStreamSynchronize(nullptr));
@@ -641,12 +739,9 @@ int dn_ppo_destroy(dn_ppo* h) {
     cudaSetDevice(h->device);
     for (void* p : h->comm_opened) cudaIpcCloseMemHandle(p);
     if (h->comm_base) cudaFree(h->comm_base);
-    for (void* p : h->allocs) cudaFree(p);
     if (h->mirror) cudaFreeHost(h->mirror);
     if (h->segs_dev) cudaFree(h->segs_dev);
     if (h->seg_of_block_dev) cudaFree(h->seg_of_block_dev);
-    if (h->psegs_dev) cudaFree(h->psegs_dev);
-    if (h->pseg_of_block_dev) cudaFree(h->pseg_of_block_dev);
     delete h;
     return DN_OK;
 }
@@ -715,9 +810,7 @@ int dn_ppo_allreduce(dn_ppo* h, void* stream) {
 
 int dn_ppo_sync_weights(dn_ppo* h, void* stream) {
     if (!h) return dn_internal_fail(DN_EINVAL, "dn_ppo_sync_weights: null handle");
-    planes_kernel<<<h->plane_blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(h->psegs_dev, h->pseg_of_block_dev, h->params, h->passes > 1);
-    PPO_CUDA(cudaGetLastError());
-    return DN_OK;
+    return refresh_planes(h, static_cast<cudaStream_t>(stream));
 }
 
 int dn_ppo_begin_update(dn_ppo* h, void* stream) {
@@ -797,8 +890,8 @@ int dn_ppo_minibatch_apply(dn_ppo* h, void* stream) {
     adam_kernel<<<std::min<long long>((n + 255) / 256, 4 * h->sms), 256, 0, st>>>(a);
     PPO_CUDA(cudaGetLastError());
     // the planes are refreshed unconditionally (a stopped step leaves the parameters, hence the planes, unchanged)
-    planes_kernel<<<h->plane_blocks, 256, 0, st>>>(h->psegs_dev, h->pseg_of_block_dev, h->params, h->passes > 1);
-    PPO_CUDA(cudaGetLastError());
+    int rc;
+    if ((rc = refresh_planes(h, st))) return rc;
     ctrl_commit_kernel<<<1, 32, 0, st>>>(h->ctrl, h->grads, n, h->step, h->norm_partial, a.inv_world, h->mirror_dev);
     PPO_CUDA(cudaGetLastError());
     return DN_OK;
@@ -828,10 +921,10 @@ int dn_ppo_poll(dn_ppo* h, int32_t* early_stop, int32_t* minibatches, int32_t* o
 
 int dn_ppo_forward(dn_ppo* h, const float* obs, int32_t rows, float* mean, float* value, void* stream) {
     if (!h || !obs || !mean || !value) return dn_internal_fail(DN_EINVAL, "dn_ppo_forward: null argument");
-    if (rows < 1 || rows > h->max_rows) return dn_internal_fail(DN_EINVAL, "dn_ppo_forward: rows must be within max_rows");
+    int rc;
+    if ((rc = check_rows(h, "dn_ppo_forward", rows))) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int rows_pad = (rows + BM - 1) / BM * BM;
-    int rc;
     if ((rc = ensure_rows(h, rows_pad, false))) return rc;
     if ((rc = run_gather(h, obs, nullptr, nullptr, rows, false, st))) return rc;
     if ((rc = run_forward_chain(h, st))) return rc;
@@ -849,11 +942,10 @@ int dn_ppo_act(dn_ppo* h, const float* obs, int32_t rows, const dn_ppo_sample* s
     if (!s->deterministic && !s->counter) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: a sampling call needs the device counter (null counter)");
     if (s->row_id_offset < 0) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: row_id_offset must be >= 0");
     if (!(s->low <= s->high)) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: low must not exceed high (and neither may be NaN)");
-    if (rows < 1) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: rows must be within max_rows");
-    if (rows > h->max_rows) return dn_internal_fail(DN_EINVAL, "dn_ppo_act: rows must be within max_rows");
+    int rc;
+    if ((rc = check_rows(h, "dn_ppo_act", rows))) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int rows_pad = (rows + BM - 1) / BM * BM;
-    int rc;
     if ((rc = ensure_rows(h, rows_pad, false))) return rc;
     if ((rc = run_gather(h, obs, nullptr, nullptr, rows, false, st))) return rc;
     if ((rc = run_forward_chain(h, st))) return rc;
@@ -865,48 +957,21 @@ int dn_ppo_act(dn_ppo* h, const float* obs, int32_t rows, const dn_ppo_sample* s
     a.seed = s->seed; a.row_id_offset = s->row_id_offset; a.low = s->low; a.high = s->high;
     const int head_blocks = std::min(std::max((rows + HEAD_WARPS - 1) / HEAD_WARPS, 1), h->head_blocks_max);
     if ((rc = run_head(h, a, head_blocks, st))) return rc;
-    if (!s->deterministic) {
-        counter_advance_kernel<<<1, 32, 0, st>>>(reinterpret_cast<long long*>(s->counter));
-        PPO_CUDA(cudaGetLastError());
-    }
-    return DN_OK;
+    return s->deterministic ? DN_OK : advance_counter(s->counter, st);
 }
 
 int dn_ppo_buffer(dn_ppo* h, const char* name, void** ptr, int64_t* elems) {
     if (!h || !name || !ptr || !elems) return dn_internal_fail(DN_EINVAL, "dn_ppo_buffer: null argument");
-    const long long R = h->max_rows;
-    std::string s(name);
-    if (s == "x") { *ptr = h->x; *elems = 2 * R * XPAD; return DN_OK; }
-    if (s.size() >= 5 && (s.compare(0, 3, "pi.") == 0 || s.compare(0, 3, "vf.") == 0)) {
-        Net& net = (s[0] == 'p') ? h->pi : h->vf;
-        const int l = s.back() - '0';
-        const std::string kind = s.substr(3, s.size() - 4);
-        if (l >= 1 && l <= net.L) {
-            if (kind == "h") { *ptr = net.h[l]; *elems = 2 * R * net.n[l]; return DN_OK; }
-            if (kind == "dz") { *ptr = net.dz[l]; *elems = 2 * R * net.n[l]; return DN_OK; }
-            if (kind == "w") { *ptr = net.w[l]; *elems = 2LL * net.n[l] * net.n[l - 1]; return DN_OK; }
-        }
-    }
+    const std::string s(name);
+    if (s == "x") { *ptr = h->x; *elems = 2LL * h->max_rows * XPAD; return DN_OK; }
+    const bool pi = s.compare(0, 3, "pi.") == 0, vf = s.compare(0, 3, "vf.") == 0;
+    if ((pi || vf) && find_planes(h, pi ? h->pi : h->vf, s.substr(3), ptr, elems)) return DN_OK;
     return dn_internal_fail(DN_EINVAL, "dn_ppo_buffer: unknown buffer name");
 }
 
 }  // extern "C"
 
-// ====================================================================================================================
-// the SAC actor (include/dnsac.h): the latent ReLU layers on the forward contraction above, then sac_head_kernel
-// ====================================================================================================================
-struct dn_sac_actor {
-    dn_sac_actor_config cfg;
-    int device = 0, passes = 3, sms = 148;
-    int max_rows = 0, cur_rows = -1;
-    const float* params = nullptr;
-    __nv_bfloat16* x = nullptr;
-    Net net;                          // h, w and fwd of the latent layers (the training buffers stay unallocated)
-    float *mu = nullptr, *log_std = nullptr;
-    PlaneSeg* psegs_dev = nullptr; int* pseg_of_block_dev = nullptr; int plane_blocks = 0;
-    std::vector<void*> allocs;
-};
-
+// ---- the SAC actor (include/dnsac.h) ----
 namespace {
 
 int sac_check_config(const dn_sac_actor_config* c) {
@@ -933,39 +998,24 @@ int sac_check_config(const dn_sac_actor_config* c) {
 
 int sac_ensure_rows(dn_sac_actor* h, int rows_pad) {
     if (rows_pad == h->cur_rows) return DN_OK;
-    Net& net = h->net;
     int rc;
-    for (int l = 1; l <= net.L; ++l)
-        if ((rc = plan_fwd(&net.fwd[l], h->passes, h->max_rows, net.n[l], net.n[l - 1], net.h[l - 1], net.w[l], h->params + net.b_off[l - 1], 2,
-                           net.h[l], rows_pad)))
-            return rc;
+    if ((rc = plan_forward(h, h->net, rows_pad, 2))) return rc;
     h->cur_rows = rows_pad;
     return DN_OK;
 }
 
-template <int ACT, int NP>
-int launch_sac_head(const dnsac::SacHeadArgs& a, int blocks, cudaStream_t st) {
-    dnsac::sac_head_kernel<ACT, NP><<<blocks, HEAD_WARPS * 32, 2 * ACT * a.n * sizeof(float), st>>>(a);
-    PPO_CUDA(cudaGetLastError());
-    return DN_OK;
-}
-
-template <int ACT>
-int run_sac_head_np(const dnsac::SacHeadArgs& a, int blocks, cudaStream_t st) {
-    const int np = a.n / 64;                              // widths are multiples of 128
-    if (np <= 2) return launch_sac_head<ACT, 2>(a, blocks, st);
-    if (np <= 4) return launch_sac_head<ACT, 4>(a, blocks, st);
-    return launch_sac_head<ACT, 8>(a, blocks, st);
-}
-
-int run_sac_head(int act_dim, const dnsac::SacHeadArgs& a, int blocks, cudaStream_t st) {
-    switch (act_dim) {
-        case 1: return run_sac_head_np<1>(a, blocks, st);
-        case 2: return run_sac_head_np<2>(a, blocks, st);
-        case 3: return run_sac_head_np<3>(a, blocks, st);
-        case 4: return run_sac_head_np<4>(a, blocks, st);
-        default: return dn_internal_fail(DN_EINVAL, "dn_sac_act: act_dim must be 1..4");
-    }
+// the SAC head for act_dim 1..4 and the last hidden width
+SacHeadKernel sac_head_for(int act_dim, int width) {
+    return with_np(width, [&](auto np) -> SacHeadKernel {
+        constexpr int NP = decltype(np)::value;
+        switch (act_dim) {
+            case 1: return dnsac::sac_head_kernel<1, NP>;
+            case 2: return dnsac::sac_head_kernel<2, NP>;
+            case 3: return dnsac::sac_head_kernel<3, NP>;
+            case 4: return dnsac::sac_head_kernel<4, NP>;
+            default: return nullptr;
+        }
+    });
 }
 
 }  // namespace
@@ -977,38 +1027,22 @@ int dn_sac_actor_create(const dn_sac_actor_config* cfg, int device, const float*
     *out = nullptr;
     int rc;
     if ((rc = sac_check_config(cfg))) return rc;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return dn_internal_fail(DN_ECUDA, "dn_sac_actor_create: no CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_create: bad device index");
-    PPO_CUDA(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    PPO_CUDA(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) return dn_internal_fail(DN_ECUDA, "dn_sac_actor_create: the kernels are sm_100a only (tcgen05 / TMEM / TMA)");
+    int sms = 0;
+    if ((rc = open_device("dn_sac_actor_create", "the kernels", device, &sms))) return rc;
 
     dn_sac_actor* h = new dn_sac_actor();
-    h->cfg = *cfg;
-    h->device = device;
-    h->passes = (cfg->precision == DN_MLP_BF16X3) ? 3 : 1;
-    h->sms = prop.multiProcessorCount;
-    g_num_sms = h->sms;
-    h->max_rows = cfg->max_rows;
-    h->params = params;
-    const long long R = h->max_rows;
     auto bail = [&](int code) { dn_sac_actor_destroy(h); return code; };
-    Net& net = h->net;
-    net.L = cfg->n_hidden;
-    net.n[0] = XPAD;
-    if ((rc = dev_alloc(h, &h->x, 2 * R * XPAD))) return bail(rc);
-    net.h[0] = h->x;
-    for (int l = 1; l <= net.L; ++l) {
-        net.n[l] = cfg->hidden[l - 1];
-        net.w_off[l - 1] = cfg->w_off[l - 1];
-        net.b_off[l - 1] = cfg->b_off[l - 1];
-        if ((rc = dev_alloc(h, &net.h[l], 2 * R * net.n[l])) || (rc = dev_alloc(h, &net.w[l], 2LL * net.n[l] * net.n[l - 1]))) return bail(rc);
-    }
+    h->cfg = *cfg;
+    h->head = sac_head_for(cfg->act_dim, cfg->hidden[cfg->n_hidden - 1]);
+    const long long R = cfg->max_rows;
+    // (the actor only reads the parameters)
+    if ((rc = init_core(h, device, sms, cfg->precision, cfg->max_rows, const_cast<float*>(params))) ||
+        (rc = setup_net(h, h->net, cfg->n_hidden, cfg->hidden, cfg->w_off, cfg->b_off, false)))
+        return bail(rc);
     if ((rc = dev_alloc(h, &h->mu, R * cfg->act_dim)) || (rc = dev_alloc(h, &h->log_std, R * cfg->act_dim))) return bail(rc);
-    const Net* nets[1] = {&net};
+    const Net* nets[1] = {&h->net};
     if ((rc = build_plane_table(h, nets, 1, cfg->obs_dim))) return bail(rc);
+    if ((rc = allow_gemm_smem({K_FWD_RELU}))) return bail(rc);
     if ((rc = sac_ensure_rows(h, h->max_rows))) return bail(rc);
     if ((rc = dn_sac_actor_sync_weights(h, nullptr))) return bail(rc);
     PPO_CUDA(cudaStreamSynchronize(nullptr));
@@ -1019,18 +1053,13 @@ int dn_sac_actor_create(const dn_sac_actor_config* cfg, int device, const float*
 int dn_sac_actor_destroy(dn_sac_actor* h) {
     if (!h) return DN_OK;
     cudaSetDevice(h->device);
-    for (void* p : h->allocs) cudaFree(p);
-    if (h->psegs_dev) cudaFree(h->psegs_dev);
-    if (h->pseg_of_block_dev) cudaFree(h->pseg_of_block_dev);
     delete h;
     return DN_OK;
 }
 
 int dn_sac_actor_sync_weights(dn_sac_actor* h, void* stream) {
     if (!h) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_sync_weights: null handle");
-    planes_kernel<<<h->plane_blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(h->psegs_dev, h->pseg_of_block_dev, h->params, h->passes > 1);
-    PPO_CUDA(cudaGetLastError());
-    return DN_OK;
+    return refresh_planes(h, static_cast<cudaStream_t>(stream));
 }
 
 int dn_sac_act(dn_sac_actor* h, const float* obs, int32_t rows, const dn_sac_sample* s, float* action, float* log_prob, void* stream) {
@@ -1039,21 +1068,18 @@ int dn_sac_act(dn_sac_actor* h, const float* obs, int32_t rows, const dn_sac_sam
         return dn_internal_fail(DN_EINVAL, "dn_sac_act: mode must be DN_SAC_SAMPLE, DN_SAC_DETERMINISTIC or DN_SAC_UNIFORM");
     if (s->mode != DN_SAC_DETERMINISTIC && !s->counter) return dn_internal_fail(DN_EINVAL, "dn_sac_act: a drawing call needs the device counter (null counter)");
     if (s->row_id_offset < 0) return dn_internal_fail(DN_EINVAL, "dn_sac_act: row_id_offset must be >= 0");
-    if (rows < 1) return dn_internal_fail(DN_EINVAL, "dn_sac_act: rows must be within max_rows");
-    if (rows > h->max_rows) return dn_internal_fail(DN_EINVAL, "dn_sac_act: rows must be within max_rows");
+    int rc;
+    if ((rc = check_rows(h, "dn_sac_act", rows))) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const long long* counter = reinterpret_cast<const long long*>(s->counter);
-    int rc;
     if (s->mode == DN_SAC_UNIFORM) {
         dnsac::sac_uniform_kernel<<<(rows + 255) / 256, 256, 0, st>>>(rows, h->cfg.act_dim, counter, s->seed, s->row_id_offset, action, log_prob);
         PPO_CUDA(cudaGetLastError());
     } else {
         if ((rc = sac_ensure_rows(h, (rows + BM - 1) / BM * BM))) return rc;
         GatherArgs g;
-        gather_obs_args(g, obs, rows, h->cfg.obs_dim, h->x, h->max_rows, h->passes);
-        if ((rc = launch_gather(g, st))) return rc;
-        for (int l = 1; l <= h->net.L; ++l)
-            if ((rc = launch_gemm(h->net.fwd[l], st))) return rc;
+        gather_obs_args(g, h, obs, rows, h->cfg.obs_dim);
+        if ((rc = launch_gather(g, st)) || (rc = launch_forward(h->net, st))) return rc;
         const Net& net = h->net;
         const int n = net.n[net.L];
         dnsac::SacHeadArgs a;
@@ -1067,31 +1093,20 @@ int dn_sac_act(dn_sac_actor* h, const float* obs, int32_t rows, const dn_sac_sam
         a.counter = (s->mode == DN_SAC_SAMPLE) ? counter : nullptr;
         a.seed = s->seed; a.row_id_offset = s->row_id_offset;
         const int blocks = std::min((rows + HEAD_WARPS - 1) / HEAD_WARPS, 3 * h->sms);
-        if ((rc = run_sac_head(c.act_dim, a, blocks, st))) return rc;
-    }
-    if (s->mode != DN_SAC_DETERMINISTIC) {
-        counter_advance_kernel<<<1, 32, 0, st>>>(reinterpret_cast<long long*>(s->counter));
+        h->head<<<blocks, HEAD_WARPS * 32, 2 * c.act_dim * n * sizeof(float), st>>>(a);
         PPO_CUDA(cudaGetLastError());
     }
-    return DN_OK;
+    return (s->mode == DN_SAC_DETERMINISTIC) ? DN_OK : advance_counter(s->counter, st);
 }
 
 int dn_sac_actor_buffer(dn_sac_actor* h, const char* name, void** ptr, int64_t* elems) {
     if (!h || !name || !ptr || !elems) return dn_internal_fail(DN_EINVAL, "dn_sac_actor_buffer: null argument");
     const long long R = h->max_rows;
-    const Net& net = h->net;
-    std::string s(name);
+    const std::string s(name);
     if (s == "x") { *ptr = h->x; *elems = 2 * R * XPAD; return DN_OK; }
     if (s == "mu") { *ptr = h->mu; *elems = R * h->cfg.act_dim; return DN_OK; }
     if (s == "log_std") { *ptr = h->log_std; *elems = R * h->cfg.act_dim; return DN_OK; }
-    if (s.size() == 2 && (s[0] == 'h' || s[0] == 'w')) {
-        const int l = s[1] - '0';
-        if (l >= 1 && l <= net.L) {
-            if (s[0] == 'h') { *ptr = net.h[l]; *elems = 2 * R * net.n[l]; }
-            else { *ptr = net.w[l]; *elems = 2LL * net.n[l] * net.n[l - 1]; }
-            return DN_OK;
-        }
-    }
+    if (find_planes(h, h->net, s, ptr, elems)) return DN_OK;
     return dn_internal_fail(DN_EINVAL, "dn_sac_actor_buffer: unknown buffer name");
 }
 

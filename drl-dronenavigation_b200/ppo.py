@@ -23,6 +23,9 @@ import torch
 import torch.distributed as dist
 from torch import nn
 
+from ._fused import Handle, flat_views, offsets, sm100, widths_ok
+from ._fused import world as _world
+
 
 @dataclass
 class PPOConfig:
@@ -185,38 +188,30 @@ def compute_gae(rewards, values, dones, last_values, gamma, lam):
     return adv, ret
 
 
-def _world():
-    return dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
-
-
-class FusedUpdate:
+class FusedUpdate(Handle):
     """ctypes face of the dn_ppo handle (include/dnppo.h): the body of PPO.train's minibatch loop and the policy forward
     as hand-written sm_100a kernels on ONE flat FP32 parameter vector.  The torch ``Parameter`` s of the policy, their
     ``.grad`` s and the Adam moments are views into the flat buffers this object hands to the library, so checkpoints,
     the eager torch path and the kernels all see the same memory."""
 
+    ABI = "dn_ppo"
+
     @staticmethod
     def shapes_ok(pi_arch, vf_arch, obs_dim: int, act_dim: int) -> bool:
         """The shapes dn_ppo_create accepts: 1..4 hidden layers per network, every hidden width a multiple of 128 between 128
         and 512 (the column-sum accumulator of the bias gradients holds 512 columns), 1 <= obs_dim <= 64, act_dim in (1, 3, 4)."""
-        widths = tuple(pi_arch) + tuple(vf_arch)
-        return (1 <= len(pi_arch) <= 4 and 1 <= len(vf_arch) <= 4 and all(w % 128 == 0 and 128 <= w <= 512 for w in widths)
-                and 1 <= obs_dim <= 64 and act_dim in (1, 3, 4))
+        return widths_ok(pi_arch, obs_dim) and widths_ok(vf_arch, obs_dim) and act_dim in (1, 3, 4)
 
     @staticmethod
     def supported(cfg: "PPOConfig", obs_dim: int, act_dim: int, device) -> bool:
-        dev = torch.device(device)
-        if dev.type != "cuda" or torch.cuda.get_device_capability(dev)[0] != 10:
-            return False
-        return FusedUpdate.shapes_ok(cfg.pi_arch, cfg.vf_arch, obs_dim, act_dim)
+        return sm100(device) and FusedUpdate.shapes_ok(cfg.pi_arch, cfg.vf_arch, obs_dim, act_dim)
 
     def __init__(self, learner: "PPOLearner", max_rows: int):
-        from . import _lib as L
-        self.L, self.lib = L, L.lib()
+        super().__init__(learner.device)
+        L = self.L
         self.learner = learner
         cfg, dev = learner.cfg, learner.device
         pol = learner.policy
-        self.device = dev
         self.max_rows = int(-(-max_rows // 128) * 128)
         n = learner.n_params
         f = dict(dtype=torch.float32, device=dev)
@@ -224,22 +219,17 @@ class FusedUpdate:
         self.exp_avg, self.exp_avg_sq = torch.zeros(n, **f), torch.zeros(n, **f)
         self.step = torch.zeros((), **f)
         # re-seat parameters (and the Adam state) as views of the flat vectors
-        offs = {}
-        off = 0
+        ps, offs = list(pol.parameters()), offsets(pol.named_parameters())
         with torch.no_grad():
-            for name, p in pol.named_parameters():
-                k = p.numel()
-                self.params[off:off + k].copy_(p.detach().reshape(-1))
-                p.data = self.params[off:off + k].view_as(p)
+            for p, v, m, m2 in zip(ps, flat_views(self.params, ps), flat_views(self.exp_avg, ps), flat_views(self.exp_avg_sq, ps)):
+                v.copy_(p.detach())
+                p.data = v
                 old = learner.opt.state.get(p)
                 if old:                                  # keep the moments of an optimiser that has already stepped / was loaded
-                    self.exp_avg[off:off + k].copy_(old["exp_avg"].reshape(-1))
-                    self.exp_avg_sq[off:off + k].copy_(old["exp_avg_sq"].reshape(-1))
+                    m.copy_(old["exp_avg"])
+                    m2.copy_(old["exp_avg_sq"])
                     self.step.copy_(torch.as_tensor(old["step"], dtype=torch.float32).reshape(()))
-                learner.opt.state[p] = {"step": self.step, "exp_avg": self.exp_avg[off:off + k].view_as(p),
-                                        "exp_avg_sq": self.exp_avg_sq[off:off + k].view_as(p)}
-                offs[name] = off
-                off += k
+                learner.opt.state[p] = {"step": self.step, "exp_avg": m, "exp_avg_sq": m2}
         c = L.dn_ppo_config()
         c.abi_version = L.DN_ABI_VERSION
         c.obs_dim, c.act_dim, c.max_rows = pol.pi[0].in_features, pol.log_std.numel(), self.max_rows
@@ -261,31 +251,9 @@ class FusedUpdate:
         for l in range(c.n_vf + 1):
             c.vf_w_off[l], c.vf_b_off[l] = offs[f"vf.{2 * l}.weight"], offs[f"vf.{2 * l}.bias"]
         c.log_std_off, c.n_params = offs["log_std"], n
-        self.cfg_c = c
-        self.handle = C.c_void_p()
-        with torch.cuda.device(dev):
-            torch.cuda.synchronize(dev)
-            L.check(self.lib.dn_ppo_create(C.byref(c), dev.index or 0, self.params.data_ptr(), learner._flat.data_ptr(), self.exp_avg.data_ptr(),
-                                           self.exp_avg_sq.data_ptr(), self.step.data_ptr(), C.byref(self.handle)), "dn_ppo_create")
+        self._create(c, self.params.data_ptr(), learner._flat.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
+                     self.step.data_ptr())
         self.launches = 0
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def close(self):
-        if getattr(self, "handle", None):
-            self.lib.dn_ppo_destroy(self.handle)
-            self.handle = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:  # noqa: BLE001
-            pass
-
-    def sync_weights(self):
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_ppo_sync_weights(self.handle, self._stream()), "dn_ppo_sync_weights")
 
     def forward(self, obs: torch.Tensor):
         """(mean [n, act_dim], value [n]) with the kernels and arithmetic of the update."""
@@ -293,9 +261,8 @@ class FusedUpdate:
         n = obs.shape[0]
         mean = torch.empty(n, self.cfg_c.act_dim, dtype=torch.float32, device=self.device)
         value = torch.empty(n, dtype=torch.float32, device=self.device)
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_ppo_sync_weights(self.handle, self._stream()), "dn_ppo_sync_weights")
-            self.L.check(self.lib.dn_ppo_forward(self.handle, obs.data_ptr(), n, mean.data_ptr(), value.data_ptr(), self._stream()), "dn_ppo_forward")
+        self.sync_weights()
+        self.call("dn_ppo_forward", obs.data_ptr(), n, mean.data_ptr(), value.data_ptr())
         return mean, value
 
     def act(self, obs: torch.Tensor, sample, action: torch.Tensor = None, clipped_action: torch.Tensor = None,
@@ -315,25 +282,21 @@ class FusedUpdate:
         for t, shape in ((obs, (n, self.cfg_c.obs_dim)), (action, (n, A)), (clipped_action, (n, A)), (log_prob, (n,)), (value, (n,))):
             if t.dtype != torch.float32 or t.device != dev or not t.is_contiguous() or tuple(t.shape) != shape:
                 raise ValueError(f"dn_ppo_act: expected a contiguous float32 tensor of shape {shape} on {self.device}")
-        with torch.cuda.device(self.device):
-            if sync:
-                self.L.check(self.lib.dn_ppo_sync_weights(self.handle, self._stream()), "dn_ppo_sync_weights")
-            self.L.check(self.lib.dn_ppo_act(self.handle, obs.data_ptr(), n, C.byref(sample), action.data_ptr(), clipped_action.data_ptr(),
-                                             log_prob.data_ptr(), value.data_ptr(), self._stream()), "dn_ppo_act")
+        if sync:
+            self.sync_weights()
+        self.call("dn_ppo_act", obs.data_ptr(), n, C.byref(sample), action.data_ptr(), clipped_action.data_ptr(), log_prob.data_ptr(),
+                  value.data_ptr())
         return action, clipped_action, log_prob, value
 
     def begin_update(self):
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_ppo_sync_weights(self.handle, self._stream()), "dn_ppo_sync_weights")
-            self.L.check(self.lib.dn_ppo_begin_update(self.handle, self._stream()), "dn_ppo_begin_update")
+        self.sync_weights()
+        self.call("dn_ppo_begin_update")
 
     def minibatch_grad(self, ro, idx: torch.Tensor):
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_ppo_minibatch_grad(self.handle, C.byref(ro), idx.data_ptr(), idx.numel(), self._stream()), "dn_ppo_minibatch_grad")
+        self.call("dn_ppo_minibatch_grad", C.byref(ro), idx.data_ptr(), idx.numel())
 
     def minibatch_apply(self):
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_ppo_minibatch_apply(self.handle, self._stream()), "dn_ppo_minibatch_apply")
+        self.call("dn_ppo_minibatch_apply")
 
     comm_ready = False
 
@@ -367,8 +330,7 @@ class FusedUpdate:
         return self.comm_ready
 
     def allreduce(self):
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_ppo_allreduce(self.handle, self._stream()), "dn_ppo_allreduce")
+        self.call("dn_ppo_allreduce")
 
     def poll(self):
         a, b, c = C.c_int32(), C.c_int32(), C.c_int32()
@@ -377,23 +339,12 @@ class FusedUpdate:
 
     def stats(self):
         st = self.L.dn_ppo_stats()
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_ppo_get_stats(self.handle, C.byref(st), self._stream()), "dn_ppo_get_stats")
+        self.call("dn_ppo_get_stats", C.byref(st))
         return st
 
     def buffer(self, name: str, rows: int, cols: int):
         """Test hook: FP32 reconstruction (hi + lo) of the first `rows` rows of an internal BF16 plane pair."""
-        ptr, elems = C.c_void_p(), C.c_int64()
-        self.L.check(self.lib.dn_ppo_buffer(self.handle, name.encode(), C.byref(ptr), C.byref(elems)), "dn_ppo_buffer")
-        n = elems.value
-
-        class _Arr:      # __cuda_array_interface__ view of the library's allocation
-            pass
-        a = _Arr()
-        a.__cuda_array_interface__ = {"shape": (n,), "typestr": "<i2", "data": (ptr.value, False), "version": 2}
-        raw = torch.as_tensor(a, device=self.device).view(torch.bfloat16)
-        full_rows = n // 2 // cols
-        planes = raw.view(2, full_rows, cols)[:, :rows]
+        planes = self._raw_buffer(name, "<i2").view(torch.bfloat16).view(2, -1, cols)[:, :rows]
         return planes[0].float() + (planes[1].float() if self.learner.cfg.mlp_precision == "bf16x3" else 0.0)
 
 
@@ -416,10 +367,8 @@ class PPOLearner:
         # (one extra element: the fused update carries this rank's KL early-stop vote through the same all-reduce)
         self._bucket = torch.zeros(self.n_params + 1, device=self.device)
         self._flat = self._bucket[:self.n_params]
-        off = 0
-        for p in self.params:
-            p.grad = self._flat[off:off + p.numel()].view_as(p)
-            off += p.numel()
+        for p, g in zip(self.params, flat_views(self._flat, self.params)):
+            p.grad = g
         self.n_updates = 0
         self.allreduce_calls = 0
         self.obs_dim, self.act_dim = obs_dim, act_dim

@@ -25,6 +25,9 @@ import torch
 import torch.distributed as dist
 from torch import nn
 
+from ._fused import Handle, flat_views, offsets, sm100, widths_ok
+from ._fused import world as _world
+
 LOG_STD_MIN, LOG_STD_MAX = -20.0, 2.0      # SB3 sac/policies.py
 
 
@@ -101,20 +104,14 @@ class Critics(nn.Module):
         return [q(x).squeeze(-1) for q in self.qs]
 
 
-def _world():
-    return dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
-
-
 class _FlatGrads:
     """All gradients of a parameter list as views into ONE tensor (one all-reduce per optimiser step)."""
 
     def __init__(self, params, device):
         self.params = list(params)
         self.flat = torch.zeros(sum(p.numel() for p in self.params), device=device)
-        off = 0
-        for p in self.params:
-            p.grad = self.flat[off:off + p.numel()].view_as(p)
-            off += p.numel()
+        for p, g in zip(self.params, flat_views(self.flat, self.params)):
+            p.grad = g
         self.calls = 0
 
     def zero(self):
@@ -218,25 +215,25 @@ class ReplayBuffer:
         return flat(self.obs)[idx], flat(self.act)[idx], flat(self.rew)[idx], flat(self.next_obs)[idx], flat(self.done)[idx]
 
 
-class FusedSACActor:
+class FusedSACActor(Handle):
     """ctypes face of the dn_sac_actor handle (include/dnsac.h): SB3's Actor.forward with sampling as sm_100a kernels (the
     latent ReLU layers on the tcgen05 contraction, heads and sampler in one CUDA-core kernel) on ONE flat FP32 parameter
     vector.  The actor's ``Parameter`` s are views into that vector (:meth:`flatten`, before the optimisers are built), so
     the torch gradient step, state dicts and checkpoints all see the memory the kernels read."""
 
+    ABI = "dn_sac_actor"
+
     @staticmethod
     def shapes_ok(arch, obs_dim: int, act_dim: int) -> bool:
         """The shapes dn_sac_actor_create accepts: 1..4 hidden layers, every width a multiple of 128 between 128 and 512,
         1 <= obs_dim <= 64, 1 <= act_dim <= 4."""
-        arch = tuple(arch)
-        return 1 <= len(arch) <= 4 and all(w % 128 == 0 and 128 <= w <= 512 for w in arch) and 1 <= obs_dim <= 64 and 1 <= act_dim <= 4
+        return widths_ok(arch, obs_dim) and 1 <= act_dim <= 4
 
     @staticmethod
     def check_supported(arch, obs_dim: int, act_dim: int, device) -> None:
-        dev = torch.device(device)
-        if dev.type != "cuda" or torch.cuda.get_device_capability(dev)[0] != 10:
+        if not sm100(device):
             raise RuntimeError(f"rollout_impl='fused' runs the SAC actor on sm_100a kernels: needs a compute-capability-10 CUDA device, "
-                               f"got {dev}")
+                               f"got {torch.device(device)}")
         if not FusedSACActor.shapes_ok(arch, obs_dim, act_dim):
             raise RuntimeError(f"rollout_impl='fused': pi_arch={tuple(arch)}, obs_dim={obs_dim}, act_dim={act_dim} is not a shape "
                                "dn_sac_actor_create accepts (1..4 hidden layers, widths multiples of 128 between 128 and 512, "
@@ -247,23 +244,18 @@ class FusedSACActor:
         """Re-seats the actor's parameters (latent layers, mu, log_std, SB3's order) as views of one new flat vector, values unchanged."""
         ps = list(actor.parameters())
         flat = torch.cat([p.detach().reshape(-1) for p in ps])
-        off = 0
-        for p in ps:
-            p.data = flat[off:off + p.numel()].view_as(p)
-            off += p.numel()
+        for p, v in zip(ps, flat_views(flat, ps)):
+            p.data = v
         return flat
 
     def __init__(self, actor: "Actor", flat: torch.Tensor, max_rows: int):
-        from . import _lib as L
-        self.L, self.lib = L, L.lib()
-        self.device, self.flat = flat.device, flat
+        super().__init__(flat.device)
+        L, self.flat = self.L, flat
         self.max_rows = int(-(-max_rows // 128) * 128)
-        offs, off = {}, 0
+        offs = offsets(actor.named_parameters())
         for name, p in actor.named_parameters():
-            if p.data_ptr() != flat.data_ptr() + 4 * off:
+            if p.data_ptr() != flat.data_ptr() + 4 * offs[name]:
                 raise RuntimeError(f"FusedSACActor: {name} is not a view of the flat parameter vector (FusedSACActor.flatten first)")
-            offs[name] = off
-            off += p.numel()
         arch = [m.out_features for m in actor.latent if isinstance(m, nn.Linear)]
         c = L.dn_sac_actor_config()
         c.abi_version = L.DN_ABI_VERSION
@@ -276,30 +268,7 @@ class FusedSACActor:
         c.mu_w_off, c.mu_b_off = offs["mu.weight"], offs["mu.bias"]
         c.log_std_w_off, c.log_std_b_off = offs["log_std.weight"], offs["log_std.bias"]
         c.n_params = flat.numel()
-        self.cfg_c = c
-        self.handle = C.c_void_p()
-        with torch.cuda.device(self.device):
-            torch.cuda.synchronize(self.device)
-            L.check(self.lib.dn_sac_actor_create(C.byref(c), self.device.index or 0, flat.data_ptr(), C.byref(self.handle)),
-                    "dn_sac_actor_create")
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def close(self):
-        if getattr(self, "handle", None):
-            self.lib.dn_sac_actor_destroy(self.handle)
-            self.handle = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:  # noqa: BLE001
-            pass
-
-    def sync_weights(self):
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_sac_actor_sync_weights(self.handle, self._stream()), "dn_sac_actor_sync_weights")
+        self._create(c, flat.data_ptr())
 
     def act(self, obs: torch.Tensor, sample, action: torch.Tensor = None, log_prob: torch.Tensor = None):
         """dn_sac_act on `obs` [n, obs_dim]: action [n, act_dim] (and log_prob [n] when given).  `sample` is an
@@ -310,23 +279,14 @@ class FusedSACActor:
         for t, shape in ((obs, (n, self.cfg_c.obs_dim)), (action, (n, A))) + (((log_prob, (n,)),) if log_prob is not None else ()):
             if t.dtype != torch.float32 or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape:
                 raise ValueError(f"dn_sac_act: expected a contiguous float32 tensor of shape {shape} on {self.device}")
-        with torch.cuda.device(self.device):
-            self.L.check(self.lib.dn_sac_act(self.handle, obs.data_ptr(), n, C.byref(sample), action.data_ptr(),
-                                             None if log_prob is None else log_prob.data_ptr(), self._stream()), "dn_sac_act")
+        self.call("dn_sac_act", obs.data_ptr(), n, C.byref(sample), action.data_ptr(), None if log_prob is None else log_prob.data_ptr())
         return action
 
     def buffer(self, name: str, rows: int) -> torch.Tensor:
         """Test hook: the first `rows` rows of an internal buffer in FP32: "h1".."h4" (hi + lo of the BF16 planes of that
         hidden layer), "mu", "log_std" (as the last non-uniform dn_sac_act left them)."""
-        ptr, elems = C.c_void_p(), C.c_int64()
-        self.L.check(self.lib.dn_sac_actor_buffer(self.handle, name.encode(), C.byref(ptr), C.byref(elems)), "dn_sac_actor_buffer")
-        n, planes = elems.value, name not in ("mu", "log_std")
-
-        class _Arr:      # __cuda_array_interface__ view of the library's allocation
-            pass
-        a = _Arr()
-        a.__cuda_array_interface__ = {"shape": (n,), "typestr": "<i2" if planes else "<f4", "data": (ptr.value, False), "version": 2}
-        raw = torch.as_tensor(a, device=self.device)
+        planes = name not in ("mu", "log_std")
+        raw = self._raw_buffer(name, "<i2" if planes else "<f4")
         if not planes:
             return raw.view(self.max_rows, -1)[:rows].clone()
         p = raw.view(torch.bfloat16).view(2, self.max_rows, -1)[:, :rows]

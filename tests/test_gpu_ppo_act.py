@@ -200,3 +200,35 @@ def test_trainer_with_the_fused_rollout_learns_to_reduce_value_loss():
     assert tr._rollout_graph is not None and int(tr.draw_counter.item()) == 4 * 16
     assert np.isfinite([o["value_loss"] for o in outs]).all() and outs[-1]["value_loss"] < outs[0]["value_loss"]
     env.close()
+
+
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two visible GPUs")
+def test_handles_on_two_devices_of_one_process_compute_the_same():
+    """A PPO handle and a SAC actor on device 1, then on device 0, from the same parameters; dn_ppo_forward and dn_sac_act
+    (deterministic) run on device 1 first.  What a handle sets up for its kernels (the contraction's shared-memory limit, the
+    SM count that sizes its grids) belongs to its own device, so device 0 runs too and gives the same bits."""
+    from drl_dronenavigation_b200 import _lib
+    from drl_dronenavigation_b200.ppo import PPOConfig, PPOLearner
+    from drl_dronenavigation_b200.sac import SACConfig, SACLearner
+    learners = {}
+    for d in (1, 0):
+        ppo = PPOLearner(13, 4, PPOConfig(pi_arch=(256, 128), vf_arch=(256, 128), update_impl="fused"), device=f"cuda:{d}")
+        sac = SACLearner(13, 4, SACConfig(pi_arch=(256, 256), rollout_impl="fused"), device=f"cuda:{d}")
+        if d == 0:
+            with torch.no_grad():
+                for a, b in zip(list(ppo.policy.parameters()) + list(sac.actor.parameters()),
+                                list(learners[1][0].policy.parameters()) + list(learners[1][1].actor.parameters())):
+                    a.copy_(b.to(a.device))
+        learners[d] = (ppo, sac, ppo.ensure_fused(4096), sac.ensure_fused_actor(4096))
+    obs = torch.randn(1000, 13, generator=torch.Generator().manual_seed(5)) * 2
+    s = _lib.dn_sac_sample()
+    s.seed, s.row_id_offset, s.counter, s.mode = 77, 0, None, _lib.DN_SAC_DETERMINISTIC
+    out = {}
+    for d in (1, 0):
+        _, _, fu, fa = learners[d]
+        o = obs.to(f"cuda:{d}")
+        mean, value = fu.forward(o)
+        out[d] = [t.cpu() for t in (mean, value, fa.act(o, s))]
+    for a, b in zip(out[1], out[0]):
+        assert torch.equal(a, b)
+    assert out[0][2].abs().max() > 0
