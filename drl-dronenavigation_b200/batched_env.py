@@ -188,7 +188,7 @@ class BatchedDroneEnv:
     def host_buffers(self, with_episode_info: bool = False):
         """dn_host_buffers: the handle's pinned host slab as numpy views (``actions`` to write, the rest to read) plus the
         ``dn_step_io`` of their pointers.  ``step_host(io)`` / ``step_host_async(io)`` with that io replay one captured graph
-        (one H2D DMA, the fused kernel, one D2H DMA) -- the lowest-latency way to step from the host."""
+        (one H2D DMA, the fused kernel, one D2H DMA) instead of a kernel that reads and writes host memory over PCIe."""
         io = L.dn_step_io()
         L.check(self._lib.dn_host_buffers(self._handle, int(bool(with_episode_info)), C.byref(io)), "dn_host_buffers")
         N, D = self.num_envs, self.obs_dim
@@ -207,7 +207,8 @@ class BatchedDroneEnv:
         return io, bufs
 
     def step_host_async(self, host_io) -> None:
-        """dn_step_host_async (buffers of :meth:`host_buffers` only): returns once the step is launched."""
+        """dn_step_host_async (buffers of :meth:`host_buffers`, or pinned, device-mapped ones): returns once the step is launched.
+        Until :meth:`step_host_wait`, every other call on the handle raises."""
         L.check(self._lib.dn_step_host_async(self._handle, C.byref(host_io)), "dn_step_host_async")
 
     def step_host_wait(self) -> None:

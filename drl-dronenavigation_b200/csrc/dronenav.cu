@@ -585,10 +585,49 @@ __global__ void state_xfer_kernel(const __grid_constant__ Params P, const __grid
 // ===========================================================================
 using dn::Params;
 
+// Every step_kernel instantiation, [physics & 3][MULTI] for one (normalize_obs, full) pair; dn_create keeps the two a handle
+// launches.
+using StepKernel = void (*)(dn::Params, dn::StepIO, int, int);
+template <bool NORM, bool FULL>
+const StepKernel kStepKernels[4][2] = {
+    {dn::step_kernel<0, NORM, false, FULL>, dn::step_kernel<0, NORM, true, FULL>},
+    {dn::step_kernel<1, NORM, false, FULL>, dn::step_kernel<1, NORM, true, FULL>},
+    {dn::step_kernel<2, NORM, false, FULL>, dn::step_kernel<2, NORM, true, FULL>},
+    {dn::step_kernel<3, NORM, false, FULL>, dn::step_kernel<3, NORM, true, FULL>}};
+
+// Byte offsets of the host-call buffers, each at 256-byte alignment:
+//   actions | obs | reward | found_targets | done | [episode_return | episode_length | terminal_obs] | completion word
+// Everything after the actions is one contiguous range [obs, word + 4): the slab moves its outputs with a single D2H copy.
+struct IoLayout { size_t act, obs, rew, fnd, done, epr, epl, term, word, bytes; bool episode; };
+
+static IoLayout io_layout(size_t N, size_t D, bool episode) {
+    IoLayout L = {};
+    L.episode = episode;
+    auto take = [&L](size_t b) { const size_t at = L.bytes; L.bytes += (b + 255) & ~static_cast<size_t>(255); return at; };
+    L.act = take(N * 16); L.obs = take(N * D * 4); L.rew = take(N * 4); L.fnd = take(N * 4); L.done = take(N);
+    if (episode) { L.epr = take(N * 4); L.epl = take(N * 4); L.term = take(N * D * 4); }
+    L.word = take(4);
+    return L;
+}
+
+static dn_step_io io_at(const IoLayout& L, char* b) {
+    dn_step_io io;
+    io.actions = reinterpret_cast<const float*>(b + L.act); io.obs = reinterpret_cast<float*>(b + L.obs);
+    io.reward = reinterpret_cast<float*>(b + L.rew); io.found_targets = reinterpret_cast<int32_t*>(b + L.fnd);
+    io.done = reinterpret_cast<uint8_t*>(b + L.done);
+    io.episode_return = L.episode ? reinterpret_cast<float*>(b + L.epr) : nullptr;
+    io.episode_length = L.episode ? reinterpret_cast<int32_t*>(b + L.epl) : nullptr;
+    io.terminal_obs = L.episode ? reinterpret_cast<float*>(b + L.term) : nullptr;
+    return io;
+}
+
+enum class InFlight { None, Slab, ZeroCopy };   // which dn_step_host_async step dn_step_host_wait has to wait for
+
 struct dn_env {
     Params P;
     int device;
     int normalize_obs;
+    StepKernel step_one, step_many;   // this handle's step_kernel: one step per launch (MULTI = false) | dn_step_many
     void* state_mem;
     float4* d_targets;
     float4* d_segs;
@@ -597,37 +636,32 @@ struct dn_env {
     int n_slots;
     int64_t launches;
     int sms;                // multiprocessor count of the device
-    int full;               // 1: any optional feature is on (random spawn, another reward family, reward wrappers) -> FULL kernels
     float d0;
-    // dn_step_host staging (allocated on first use)
+    // host-buffer calls (allocated on first use)
     cudaStream_t host_stream;
-    void* stage;            // device: actions | obs | terminal_obs | reward | ep_return | found | ep_length | done
+    void* stage;            // device staging of the pageable path: IoLayout with the episode outputs
     dn_step_io host_seen;   // last host io whose pointers were classified
     dn_step_io host_mapped; // device aliases of those pointers when all of them are pinned + mapped (UVA)
     int host_direct;        // 1: the kernel reads / writes the caller's pinned buffers directly (zero copy)
     const void* ptr_cache_h[32]; void* ptr_cache_d[32]; int ptr_cache_n; unsigned ptr_cache_next;   // pinned + mapped pointers seen so far
+    InFlight in_flight;     // the dn_step_host_async step that has not been waited for
     // dn_host_buffers: handle-owned pinned slab + device slab, stepped by replaying one captured graph
     char* slab_h; char* slab_d;
-    size_t slab_out_off, slab_out_bytes, slab_seq_off;   // outputs [slab_out_off, +slab_out_bytes) incl. the completion word
+    IoLayout slab;
     dn_step_io slab_io_h, slab_io_d;
     cudaGraphExec_t slab_exec;
-    int slab_pending;       // a graph launch whose completion word has not been consumed yet
-    int no_pdl;             // launch_step: plain launch (inside the slab graph the predecessor is a copy node)
-    long long graph_replays;
     // zero-copy host call: completion word in pinned host memory, written by the last CTA of the step kernel
     unsigned int* zc_flag_h; unsigned int* zc_flag_d; unsigned int* zc_counter; unsigned int zc_seq;
-    int zc_signal;          // launch_step: pass the completion word to the kernel (set around the zero-copy launch only)
     // resident step server (dn_host_server): a dn_step_many kernel that stays on the GPU and takes one host command per step
     int srv_idle_us;        // > 0: dn_step_host on pinned + mapped buffers goes through the server
     int srv_alive;          // a server kernel has been launched on srv_stream and has not been seen to finish
-    int srv_launch;         // launch_step: fill the server fields of StepIO (set around the server launch only)
     cudaStream_t srv_stream;
     unsigned long long* srv_doorbell_h; unsigned long long* srv_doorbell_d;   // pinned + mapped
     unsigned long long* srv_word_h;     // pinned staging word for the initial value of srv_cmd
     unsigned long long* srv_cmd;        // device
     unsigned int srv_seq;   // sequence number of the last command (16 bits, never 0)
     dn_step_io srv_io;      // mapped output pointers the running server writes
-    long long srv_launches, srv_steps;
+    long long srv_residencies, srv_steps;
 };
 
 static thread_local std::string g_err;
@@ -657,7 +691,20 @@ struct DeviceGuard {   // switches the calling thread to the handle's device onl
 
 extern "C" {
 
-static int srv_quiesce(dn_env* env);     // stops the resident step server (if one is running) before anything else touches the state
+// Every call that touches the handle's state goes through here first.  It refuses while a dn_step_host_async step has not been
+// waited for (that step still runs on the handle's stream against the same state), then stops the resident step server if one
+// is running -- unless `stop_server` is false (dn_step_host on the server path).
+static int quiesce(dn_env* env, const char* who, bool stop_server = true) {
+    if (env->in_flight != InFlight::None)
+        return fail(DN_EINVAL, std::string(who) + ": a dn_step_host_async step has not been waited for (dn_step_host_wait)");
+    if (!stop_server || !env->srv_alive) return DN_OK;
+    DeviceGuard guard(env->device);
+    env->srv_seq = (env->srv_seq % 0xFFFFu) + 1u;
+    *reinterpret_cast<volatile unsigned long long*>(env->srv_doorbell_h) = static_cast<unsigned long long>(env->srv_seq) << 48;   // pointer 0: quit
+    env->srv_alive = 0;
+    DN_CUDA(cudaStreamSynchronize(env->srv_stream));
+    return DN_OK;
+}
 
 int dn_abi_version(void) { return DN_ABI_VERSION; }
 const char* dn_last_error(void) { return g_err.c_str(); }
@@ -697,12 +744,18 @@ int dn_create(const dn_config* cfg, int device, dn_env** out) {
     std::memset(e, 0, sizeof(*e));
     e->device = device;
     e->normalize_obs = cfg->normalize_obs ? 1 : 0;
-    e->full = (cfg->spawn_mode != DN_SPAWN_FIXED || rw.mode != dn::RW_WAYPOINT || rw.proj_w != 0.0f || cfg->normalize_reward ||
-               cfg->clip_reward > 0.0 || cfg->act_type >= DN_ACT_PID) ? 1 : 0;
     Params& P = e->P;
     const int N = cfg->num_envs, T = cfg->num_targets;
     std::vector<float4> h_t, h_s;
     dn::host::fill_params(*cfg, rw, P, h_t, h_s, e->d0);
+    {   // FULL kernels when any optional feature is on (random spawn, another reward family, reward wrappers, PID actions)
+        const bool full = cfg->spawn_mode != DN_SPAWN_FIXED || rw.mode != dn::RW_WAYPOINT || rw.proj_w != 0.0f ||
+                          cfg->normalize_reward || cfg->clip_reward > 0.0 || cfg->act_type >= DN_ACT_PID;
+        const StepKernel (&ks)[4][2] = e->normalize_obs ? (full ? kStepKernels<true, true> : kStepKernels<true, false>)
+                                                        : (full ? kStepKernels<false, true> : kStepKernels<false, false>);
+        e->step_one = ks[P.physics & 3][0];
+        e->step_many = ks[P.physics & 3][1];
+    }
 
     auto cleanup = [&](int code, const std::string& msg) {
         if (e->state_mem) cudaFree(e->state_mem);
@@ -768,8 +821,10 @@ int dn_create(const dn_config* cfg, int device, dn_env** out) {
 
 int dn_destroy(dn_env* env) {
     if (!env) return DN_OK;
-    srv_quiesce(env);
     DeviceGuard guard(env->device);
+    if (env->in_flight != InFlight::None) cudaStreamSynchronize(env->host_stream);
+    env->in_flight = InFlight::None;
+    quiesce(env, "dn_destroy");
     if (env->srv_stream) cudaStreamDestroy(env->srv_stream);
     if (env->srv_doorbell_h) cudaFreeHost(env->srv_doorbell_h);
     if (env->srv_cmd) cudaFree(env->srv_cmd);
@@ -778,7 +833,6 @@ int dn_destroy(dn_env* env) {
     if (env->stage) cudaFree(env->stage);
     if (env->zc_flag_h) cudaFreeHost(env->zc_flag_h);
     if (env->zc_counter) cudaFree(env->zc_counter);
-    if (env->slab_pending) cudaStreamSynchronize(env->host_stream);
     if (env->slab_exec) cudaGraphExecDestroy(env->slab_exec);
     if (env->slab_h) cudaFreeHost(env->slab_h);
     if (env->slab_d) cudaFree(env->slab_d);
@@ -793,7 +847,7 @@ int64_t dn_launch_count(const dn_env* env) { return env ? env->launches : 0; }
 
 int dn_reset(dn_env* env, const uint8_t* mask, float* obs_out, void* stream) {
     if (!env) return fail(DN_EINVAL, "dn_reset: null handle");
-    { const int rq = srv_quiesce(env); if (rq != DN_OK) return rq; }
+    { const int rq = quiesce(env, "dn_reset"); if (rq != DN_OK) return rq; }
     DeviceGuard guard(env->device);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int N = env->P.n;
@@ -804,28 +858,26 @@ int dn_reset(dn_env* env, const uint8_t* mask, float* obs_out, void* stream) {
     return DN_OK;
 }
 
-static int launch_step(dn_env* env, const dn_step_io* io, int num_steps, int per_step, void* stream) {
+// The argument checks of the step calls and the dn_step_io -> dn::StepIO conversion; the completion word and the server
+// fields are left empty for the caller to fill in.
+static int step_io(const dn_env* env, const dn_step_io* io, int num_steps, dn::StepIO& k) {
     if (!env || !io) return fail(DN_EINVAL, "dn_step: null argument");
     if (!io->actions || !io->obs || !io->reward || !io->done) return fail(DN_EINVAL, "dn_step: actions/obs/reward/done are required");
     if (num_steps <= 0) return fail(DN_EINVAL, "dn_step_many: num_steps must be > 0");
     if (reinterpret_cast<uintptr_t>(io->actions) & 15u) return fail(DN_EINVAL, "dn_step: actions must be 16-byte aligned");
-    DeviceGuard guard(env->device);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    dn::StepIO k;
+    k = dn::StepIO{};
     k.actions = reinterpret_cast<const float4*>(io->actions);
     k.obs = io->obs; k.reward = io->reward; k.done = io->done; k.terminal_obs = io->terminal_obs;
     k.found_targets = io->found_targets; k.episode_return = io->episode_return; k.episode_length = io->episode_length;
-    k.done_counter = nullptr; k.host_flag = nullptr; k.seq = 0u;
-    if (env->zc_signal && num_steps == 1) { k.done_counter = env->zc_counter; k.host_flag = env->zc_flag_d; k.seq = env->zc_seq; }
-    k.srv_doorbell = nullptr; k.srv_cmd = nullptr; k.srv_word0 = 0ull; k.srv_idle_us = 0u;
-    if (env->srv_launch) {
-        k.done_counter = env->zc_counter; k.host_flag = env->zc_flag_d;
-        k.srv_doorbell = env->srv_doorbell_d; k.srv_cmd = env->srv_cmd; k.srv_word0 = *env->srv_word_h;
-        k.srv_idle_us = static_cast<unsigned int>(env->srv_idle_us);
-    }
+    return DN_OK;
+}
+
+// One launch of the handle's step kernel: the single-step one for num_steps == 1, the dn_step_many one otherwise.  `pdl`: the
+// caller allows a programmatic dependent launch (not inside the slab graph, whose predecessor is a copy node, nor for the server).
+static int launch_step(dn_env* env, dn::StepIO k, int num_steps, int per_step, cudaStream_t st, bool pdl) {
+    DeviceGuard guard(env->device);
     const int N = env->P.n;
     const dim3 grid((N + dn::kBlock - 1) / dn::kBlock), block(dn::kBlock);
-    const int phys = env->P.physics & 3;
     // Programmatic dependent launch: the step kernel may be scheduled while the previous kernel of the stream is still
     // running (its CTAs trigger at entry); it then waits (griddepcontrol.wait, before its first global access) until that
     // kernel has completed and flushed.  Back-to-back steps -- plain or replayed from a CUDA graph -- thereby hide
@@ -839,27 +891,10 @@ static int launch_step(dn_env* env, const dn_step_io* io, int num_steps, int per
     // two consecutive small grids each get SMs of their own.  With mid-size grids (0.3 - 1 wave) the early-resident
     // CTAs of the next step pile up on the SMs that had free slots, and the step then runs unbalanced (measured:
     // 65 536 envs 7.7 -> 9.8 us, 16 384 envs with drag / ground effect 7.4 -> 9.1 us per replayed step).
-    lc.attrs = attr; lc.numAttrs = (!env->no_pdl && !env->srv_launch && static_cast<int>(grid.x) * 2 <= env->sms) ? 1 : 0;
+    lc.attrs = attr; lc.numAttrs = (pdl && static_cast<int>(grid.x) * 2 <= env->sms) ? 1 : 0;
     k.pdl_prefetch = static_cast<int>(lc.numAttrs);
-    cudaError_t lerr = cudaSuccess;
-#define DN_LAUNCH(PH, NO)                                                                                              \
-    do {                                                                                                               \
-        if (env->full) {                                                                                               \
-            if (num_steps == 1) lerr = cudaLaunchKernelEx(&lc, dn::step_kernel<PH, NO, false, true>, env->P, k, 1, 1); \
-            else lerr = cudaLaunchKernelEx(&lc, dn::step_kernel<PH, NO, true, true>, env->P, k, num_steps, per_step);  \
-        } else {                                                                                                       \
-            if (num_steps == 1) lerr = cudaLaunchKernelEx(&lc, dn::step_kernel<PH, NO, false, false>, env->P, k, 1, 1); \
-            else lerr = cudaLaunchKernelEx(&lc, dn::step_kernel<PH, NO, true, false>, env->P, k, num_steps, per_step); \
-        }                                                                                                              \
-    } while (0)
-    if (env->normalize_obs) {
-        switch (phys) { case 0: DN_LAUNCH(0, true); break; case 1: DN_LAUNCH(1, true); break;
-                        case 2: DN_LAUNCH(2, true); break; default: DN_LAUNCH(3, true); break; }
-    } else {
-        switch (phys) { case 0: DN_LAUNCH(0, false); break; case 1: DN_LAUNCH(1, false); break;
-                        case 2: DN_LAUNCH(2, false); break; default: DN_LAUNCH(3, false); break; }
-    }
-#undef DN_LAUNCH
+    const cudaError_t lerr = num_steps == 1 ? cudaLaunchKernelEx(&lc, env->step_one, env->P, k, 1, 1)
+                                            : cudaLaunchKernelEx(&lc, env->step_many, env->P, k, num_steps, per_step);
     DN_CUDA(lerr);
     DN_CUDA(cudaGetLastError());
     env->launches += 1;
@@ -867,13 +902,17 @@ static int launch_step(dn_env* env, const dn_step_io* io, int num_steps, int per
 }
 
 int dn_step(dn_env* env, const dn_step_io* io, void* stream) {
-    { const int rq = srv_quiesce(env); if (rq != DN_OK) return rq; }
-    return launch_step(env, io, 1, 1, stream);
+    dn::StepIO k;
+    int rc = step_io(env, io, 1, k);
+    if (rc == DN_OK) rc = quiesce(env, "dn_step");
+    return rc != DN_OK ? rc : launch_step(env, k, 1, 1, static_cast<cudaStream_t>(stream), true);
 }
 
 int dn_step_many(dn_env* env, const dn_step_io* io, int num_steps, int per_step_outputs, void* stream) {
-    { const int rq = srv_quiesce(env); if (rq != DN_OK) return rq; }
-    return launch_step(env, io, num_steps, per_step_outputs ? 1 : 0, stream);
+    dn::StepIO k;
+    int rc = step_io(env, io, num_steps, k);
+    if (rc == DN_OK) rc = quiesce(env, "dn_step_many");
+    return rc != DN_OK ? rc : launch_step(env, k, num_steps, per_step_outputs ? 1 : 0, static_cast<cudaStream_t>(stream), true);
 }
 
 // Zero-copy classification: if every buffer is pinned host memory mapped into the device address space (torch /
@@ -926,30 +965,32 @@ static int ensure_completion_word(dn_env* env) {
 
 // One launch of the step kernel on the mapped host buffers; the kernel announces completion through the completion word.
 static int zero_copy_launch(dn_env* env) {
-    const int rw = ensure_completion_word(env);
-    if (rw != DN_OK) return rw;
-    env->zc_seq += 1; if (env->zc_seq == 0u) env->zc_seq = 1u; env->zc_signal = 1;
+    dn::StepIO k;
+    int rc = ensure_completion_word(env);
+    if (rc == DN_OK) rc = step_io(env, &env->host_mapped, 1, k);
+    if (rc != DN_OK) return rc;
+    env->zc_seq += 1; if (env->zc_seq == 0u) env->zc_seq = 1u;
     // the word is shared with the resident server (its own sequence numbers): never start a wait on a stale equal value
     if (*reinterpret_cast<volatile unsigned int*>(env->zc_flag_h) == env->zc_seq) *reinterpret_cast<volatile unsigned int*>(env->zc_flag_h) = 0u;
-    const int rc = launch_step(env, &env->host_mapped, 1, 1, env->host_stream);
-    env->zc_signal = 0;
-    return rc;
+    k.done_counter = env->zc_counter; k.host_flag = env->zc_flag_d; k.seq = env->zc_seq;
+    return launch_step(env, k, 1, 1, env->host_stream, true);
+}
+
+// Spins until the pinned completion word holds `want`.  Every 2^16 spins it looks at the stream, so that a failed launch, or a
+// step that finished without writing the word, ends in an error instead of an endless spin.
+static int wait_word(dn_env* env, const volatile uint32_t* word, uint32_t want, cudaStream_t st, const char* who, const char* message) {
+    for (uint32_t spins = 0; *word != want;) {
+        if ((++spins & 0xFFFFu) != 0u) continue;
+        DeviceGuard guard(env->device);
+        const cudaError_t e = cudaStreamQuery(st);
+        if (e != cudaErrorNotReady && *word != want)
+            return fail(DN_ECUDA, std::string(who) + ": " + (e == cudaSuccess ? message : cudaGetErrorString(e)));
+    }
+    return DN_OK;
 }
 
 static int zero_copy_wait(dn_env* env) {
-    volatile unsigned int* flag = env->zc_flag_h;
-    const unsigned int want = env->zc_seq;
-    uint32_t spins = 0;
-    while (*flag != want) {
-        if ((++spins & 0xFFFFu) == 0u) {           // a failed launch must end in an error, not in an endless spin
-            const cudaError_t e = cudaStreamQuery(env->host_stream);
-            if (e != cudaErrorNotReady && *flag != want) {
-                if (e == cudaSuccess) return fail(DN_ECUDA, "dn_step_host: the step finished without writing the completion word");
-                return fail(DN_ECUDA, std::string("dn_step_host: ") + cudaGetErrorString(e));
-            }
-        }
-    }
-    return DN_OK;
+    return wait_word(env, env->zc_flag_h, env->zc_seq, env->host_stream, "dn_step_host", "the step finished without writing the completion word");
 }
 
 // ---------------------------------------------------------------------------------------------------------------------------
@@ -957,18 +998,8 @@ static int zero_copy_wait(dn_env* env) {
 // completion hand-off: tools/e2e_breakdown.py).  With dn_host_server(env, idle_us) the step kernel (the dn_step_many variant:
 // state in registers, stored every step) stays resident instead: the host writes the step's actions, rings a doorbell word in
 // pinned memory and polls the completion word; the kernel leaves by itself after `idle_us` without a command and is launched
-// again by the next dn_step_host.  Every other call that touches the handle's state stops the server first (srv_quiesce).
+// again by the next dn_step_host.  Every other call that touches the handle's state stops the server first (quiesce).
 // ---------------------------------------------------------------------------------------------------------------------------
-static int srv_quiesce(dn_env* env) {
-    if (!env || !env->srv_alive) return DN_OK;
-    DeviceGuard guard(env->device);
-    env->srv_seq = (env->srv_seq % 0xFFFFu) + 1u;
-    *reinterpret_cast<volatile unsigned long long*>(env->srv_doorbell_h) = static_cast<unsigned long long>(env->srv_seq) << 48;   // pointer 0: quit
-    env->srv_alive = 0;
-    DN_CUDA(cudaStreamSynchronize(env->srv_stream));
-    return DN_OK;
-}
-
 static int srv_start(dn_env* env, unsigned int seq_done) {
     if (!env->srv_stream) {
         DN_CUDA(cudaStreamCreateWithFlags(&env->srv_stream, cudaStreamNonBlocking));
@@ -985,12 +1016,16 @@ static int srv_start(dn_env* env, unsigned int seq_done) {
     DN_CUDA(cudaMemcpyAsync(env->srv_cmd, env->srv_word_h, 8, cudaMemcpyHostToDevice, env->srv_stream));
     dn_step_io io = env->srv_io;
     io.actions = reinterpret_cast<const float*>(env->srv_doorbell_d);   // placeholder (16-byte aligned); the commands carry the real pointer
-    env->srv_launch = 1;
-    const int rc = launch_step(env, &io, 0x7fffffff, 0, env->srv_stream);
-    env->srv_launch = 0;
+    dn::StepIO k;
+    int rc = step_io(env, &io, 0x7fffffff, k);
+    if (rc != DN_OK) return rc;
+    k.done_counter = env->zc_counter; k.host_flag = env->zc_flag_d;
+    k.srv_doorbell = env->srv_doorbell_d; k.srv_cmd = env->srv_cmd; k.srv_word0 = *env->srv_word_h;
+    k.srv_idle_us = static_cast<unsigned int>(env->srv_idle_us);
+    rc = launch_step(env, k, 0x7fffffff, 0, env->srv_stream, false);
     if (rc != DN_OK) return rc;
     env->srv_alive = 1;
-    env->srv_launches += 1;
+    env->srv_residencies += 1;
     return DN_OK;
 }
 
@@ -1000,7 +1035,7 @@ static int srv_step(dn_env* env) {
     if (reinterpret_cast<uintptr_t>(m.actions) >> 48) return fail(DN_EINVAL, "dn_step_host: device pointer does not fit the doorbell word");
     dn_step_io outs = m; outs.actions = nullptr;
     if (env->srv_alive && std::memcmp(&outs, &env->srv_io, sizeof(outs)) != 0) {      // other output buffers: new residency
-        const int rq = srv_quiesce(env);
+        const int rq = quiesce(env, "dn_step_host");
         if (rq != DN_OK) return rq;
     }
     const int rw = ensure_completion_word(env);
@@ -1039,7 +1074,7 @@ static int srv_step(dn_env* env) {
 int dn_host_server(dn_env* env, int idle_us) {
     if (!env) return fail(DN_EINVAL, "dn_host_server: null handle");
     if (idle_us < 0 || idle_us > 1000000) return fail(DN_EINVAL, "dn_host_server: idle_us must be in [0, 1000000]");
-    const int rq = srv_quiesce(env);
+    const int rq = quiesce(env, "dn_host_server");
     if (rq != DN_OK) return rq;
     // every CTA of the resident grid must fit on the device at once (they wait for each other's commands)
     const int grid = (env->P.n + dn::kBlock - 1) / dn::kBlock;
@@ -1050,58 +1085,40 @@ int dn_host_server(dn_env* env, int idle_us) {
 
 int dn_host_server_stats(dn_env* env, int64_t* residencies, int64_t* steps) {
     if (!env) return fail(DN_EINVAL, "dn_host_server_stats: null handle");
-    if (residencies) *residencies = env->srv_launches;
+    if (residencies) *residencies = env->srv_residencies;
     if (steps) *steps = env->srv_steps;
+    return DN_OK;
+}
+
+static int ensure_host_stream(dn_env* env) {
+    if (!env->host_stream) DN_CUDA(cudaStreamCreateWithFlags(&env->host_stream, cudaStreamNonBlocking));
     return DN_OK;
 }
 
 int dn_host_buffers(dn_env* env, int with_episode_info, dn_step_io* out) {
     if (!env || !out) return fail(DN_EINVAL, "dn_host_buffers: null argument");
-    { const int rq = srv_quiesce(env); if (rq != DN_OK) return rq; }
+    { const int rq = quiesce(env, "dn_host_buffers"); if (rq != DN_OK) return rq; }
     DeviceGuard guard(env->device);
-    if (!env->host_stream) DN_CUDA(cudaStreamCreateWithFlags(&env->host_stream, cudaStreamNonBlocking));
-    if (env->slab_h && (env->slab_io_h.terminal_obs != nullptr) != (with_episode_info != 0)) {
-        if (env->slab_pending) return fail(DN_EINVAL, "dn_host_buffers: a step is pending");
+    { const int rs = ensure_host_stream(env); if (rs != DN_OK) return rs; }
+    if (env->slab_h && env->slab.episode != (with_episode_info != 0)) {
         if (env->slab_exec) { cudaGraphExecDestroy(env->slab_exec); env->slab_exec = nullptr; }
         cudaFreeHost(env->slab_h); cudaFree(env->slab_d);
         env->slab_h = env->slab_d = nullptr;
     }
     if (!env->slab_h) {
-        const size_t N = env->P.n, D = env->P.obs_dim;
-        auto up = [](size_t b) { return (b + 255) & ~static_cast<size_t>(255); };
-        size_t o = 0;
-        const size_t o_act = o; o += up(N * 16);
-        const size_t o_obs = o; o += up(N * D * 4);
-        const size_t o_rew = o; o += up(N * 4);
-        const size_t o_fnd = o; o += up(N * 4);
-        const size_t o_done = o; o += up(N);
-        size_t o_epr = 0, o_epl = 0, o_term = 0;
-        if (with_episode_info) {
-            o_epr = o; o += up(N * 4);
-            o_epl = o; o += up(N * 4);
-            o_term = o; o += up(N * D * 4);
-        }
-        const size_t o_seq = o; o += 256;
+        const IoLayout L = io_layout(env->P.n, env->P.obs_dim, with_episode_info != 0);
         void* hp = nullptr; void* dp = nullptr;
-        DN_CUDA(cudaHostAlloc(&hp, o, cudaHostAllocDefault));
-        cudaError_t ce = cudaMalloc(&dp, o);
+        DN_CUDA(cudaHostAlloc(&hp, L.bytes, cudaHostAllocDefault));
+        cudaError_t ce = cudaMalloc(&dp, L.bytes);
         if (ce != cudaSuccess) { cudaFreeHost(hp); return fail(DN_ENOMEM, std::string("dn_host_buffers: cudaMalloc: ") + cudaGetErrorString(ce)); }
-        std::memset(hp, 0, o);
-        DN_CUDA(cudaMemset(dp, 0, o));
+        std::memset(hp, 0, L.bytes);
+        DN_CUDA(cudaMemset(dp, 0, L.bytes));
         const uint32_t one = 1;                        // the completion word: constant 1 on the device, cleared on the host before a launch
-        DN_CUDA(cudaMemcpy(static_cast<char*>(dp) + o_seq, &one, 4, cudaMemcpyHostToDevice));
+        DN_CUDA(cudaMemcpy(static_cast<char*>(dp) + L.word, &one, 4, cudaMemcpyHostToDevice));
         env->slab_h = static_cast<char*>(hp); env->slab_d = static_cast<char*>(dp);
-        env->slab_out_off = o_obs; env->slab_out_bytes = o_seq + 4 - o_obs; env->slab_seq_off = o_seq;
-        auto fill = [&](dn_step_io& io, char* b) {
-            io.actions = reinterpret_cast<const float*>(b + o_act); io.obs = reinterpret_cast<float*>(b + o_obs);
-            io.reward = reinterpret_cast<float*>(b + o_rew); io.found_targets = reinterpret_cast<int32_t*>(b + o_fnd);
-            io.done = reinterpret_cast<uint8_t*>(b + o_done);
-            io.episode_return = with_episode_info ? reinterpret_cast<float*>(b + o_epr) : nullptr;
-            io.episode_length = with_episode_info ? reinterpret_cast<int32_t*>(b + o_epl) : nullptr;
-            io.terminal_obs = with_episode_info ? reinterpret_cast<float*>(b + o_term) : nullptr;
-        };
-        fill(env->slab_io_h, env->slab_h);
-        fill(env->slab_io_d, env->slab_d);
+        env->slab = L;
+        env->slab_io_h = io_at(L, env->slab_h);
+        env->slab_io_d = io_at(L, env->slab_d);
     }
     *out = env->slab_io_h;
     return DN_OK;
@@ -1109,34 +1126,33 @@ int dn_host_buffers(dn_env* env, int with_episode_info, dn_step_io* out) {
 
 int dn_step_host_async(dn_env* env, const dn_step_io* h) {
     if (!env || !h) return fail(DN_EINVAL, "dn_step_host_async: null argument");
-    if (env->slab_pending) return fail(DN_EINVAL, "dn_step_host_async: the previous step has not been waited for");
-    { const int rq = srv_quiesce(env); if (rq != DN_OK) return rq; }
+    { const int rq = quiesce(env, "dn_step_host_async"); if (rq != DN_OK) return rq; }
+    DeviceGuard guard(env->device);
     if (!env->slab_h || std::memcmp(h, &env->slab_io_h, sizeof(*h)) != 0) {
         // caller-owned buffers: only the zero-copy form (pinned + mapped) can be left in flight
         if (!h->actions || !h->obs || !h->reward || !h->done) return fail(DN_EINVAL, "dn_step_host_async: actions/obs/reward/done are required");
-        DeviceGuard guard(env->device);
-        if (!env->host_stream) DN_CUDA(cudaStreamCreateWithFlags(&env->host_stream, cudaStreamNonBlocking));
-        const int rc = host_classify(env, h);
+        int rc = ensure_host_stream(env);
+        if (rc == DN_OK) rc = host_classify(env, h);
         if (rc != DN_OK) return rc;
         if (!env->host_direct)
             return fail(DN_EINVAL, "dn_step_host_async: needs pinned, device-mapped host buffers or the buffers dn_host_buffers returned");
-        const int rl = zero_copy_launch(env);
-        if (rl != DN_OK) return rl;
-        env->slab_pending = 2;
+        rc = zero_copy_launch(env);
+        if (rc != DN_OK) return rc;
+        env->in_flight = InFlight::ZeroCopy;
         return DN_OK;
     }
-    DeviceGuard guard(env->device);
     cudaStream_t st = env->host_stream;
     if (!env->slab_exec) {
         // capture once: H2D(actions) -> fused step kernel -> D2H(outputs + completion word)
+        dn::StepIO k;
+        int rc = step_io(env, &env->slab_io_d, 1, k);
+        if (rc != DN_OK) return rc;
         cudaGraph_t graph = nullptr;
         DN_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
         cudaError_t ce = cudaMemcpyAsync(env->slab_d, env->slab_h, static_cast<size_t>(env->P.n) * 16, cudaMemcpyHostToDevice, st);
-        env->no_pdl = 1;
-        const int rc = (ce == cudaSuccess) ? launch_step(env, &env->slab_io_d, 1, 1, st) : DN_ECUDA;
-        env->no_pdl = 0;
+        rc = (ce == cudaSuccess) ? launch_step(env, k, 1, 1, st, false) : DN_ECUDA;
         if (ce == cudaSuccess && rc == DN_OK)
-            ce = cudaMemcpyAsync(env->slab_h + env->slab_out_off, env->slab_d + env->slab_out_off, env->slab_out_bytes, cudaMemcpyDeviceToHost, st);
+            ce = cudaMemcpyAsync(env->slab_h + env->slab.obs, env->slab_d + env->slab.obs, env->slab.word + 4 - env->slab.obs, cudaMemcpyDeviceToHost, st);
         cudaError_t ce2 = cudaStreamEndCapture(st, &graph);
         if (rc != DN_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
         if (ce != cudaSuccess || ce2 != cudaSuccess) {
@@ -1148,37 +1164,21 @@ int dn_step_host_async(dn_env* env, const dn_step_io* h) {
         if (ce != cudaSuccess) { env->slab_exec = nullptr; return fail(DN_ECUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce)); }
         env->launches -= 1;                            // the captured launch is counted per replay below
     }
-    *reinterpret_cast<volatile uint32_t*>(env->slab_h + env->slab_seq_off) = 0u;
+    *reinterpret_cast<volatile uint32_t*>(env->slab_h + env->slab.word) = 0u;
     DN_CUDA(cudaGraphLaunch(env->slab_exec, st));
-    env->slab_pending = 1;
+    env->in_flight = InFlight::Slab;
     env->launches += 1;
-    env->graph_replays += 1;
     return DN_OK;
 }
 
 int dn_step_host_wait(dn_env* env) {
     if (!env) return fail(DN_EINVAL, "dn_step_host_wait: null handle");
-    if (!env->slab_pending) return DN_OK;
-    if (env->slab_pending == 2) {
-        env->slab_pending = 0;
-        return zero_copy_wait(env);
-    }
-    volatile uint32_t* seq = reinterpret_cast<volatile uint32_t*>(env->slab_h + env->slab_seq_off);
-    // the D2H copy writes the completion word last; poll it, and look at the stream now and then so that a failed
-    // launch ends in an error instead of an endless spin
-    uint32_t spins = 0;
-    while (*seq == 0u) {
-        if ((++spins & 0xFFFFu) == 0u) {
-            DeviceGuard guard(env->device);
-            const cudaError_t e = cudaStreamQuery(env->host_stream);
-            if (e != cudaErrorNotReady && *seq == 0u) {
-                env->slab_pending = 0;
-                if (e == cudaSuccess) return fail(DN_ECUDA, "dn_step_host_wait: the graph finished without setting the completion word");
-                return fail(DN_ECUDA, std::string("dn_step_host_wait: ") + cudaGetErrorString(e));
-            }
-        }
-    }
-    env->slab_pending = 0;
+    const InFlight f = env->in_flight;
+    env->in_flight = InFlight::None;
+    if (f == InFlight::ZeroCopy) return zero_copy_wait(env);
+    if (f == InFlight::Slab)                           // the graph's D2H copy writes the device's constant 1 to the word last
+        return wait_word(env, reinterpret_cast<volatile uint32_t*>(env->slab_h + env->slab.word), 1u, env->host_stream,
+                         "dn_step_host_wait", "the graph finished without setting the completion word");
     return DN_OK;
 }
 
@@ -1190,47 +1190,38 @@ int dn_step_host(dn_env* env, const dn_step_io* h) {
         return rc != DN_OK ? rc : dn_step_host_wait(env);
     }
     DeviceGuard guard(env->device);
-    if (!env->host_stream) DN_CUDA(cudaStreamCreateWithFlags(&env->host_stream, cudaStreamNonBlocking));
-    {
-        const int rc = host_classify(env, h);
-        if (rc != DN_OK) return rc;
-    }
-    if (env->host_direct && env->srv_idle_us > 0) return srv_step(env);
-    {
-        const int rq = srv_quiesce(env);
-        if (rq != DN_OK) return rq;
-    }
+    int rc = ensure_host_stream(env);
+    if (rc == DN_OK) rc = host_classify(env, h);
+    const bool server = env->host_direct && env->srv_idle_us > 0;
+    if (rc == DN_OK) rc = quiesce(env, "dn_step_host", !server);
+    if (rc != DN_OK) return rc;
+    if (server) return srv_step(env);
     if (env->host_direct) {
-        const int rc = zero_copy_launch(env);
+        rc = zero_copy_launch(env);
         return rc != DN_OK ? rc : zero_copy_wait(env);
     }
     const size_t N = env->P.n, D = env->P.obs_dim;
-    const size_t a256 = 255;
-    auto up = [&](size_t b) { return (b + a256) & ~a256; };
-    const size_t o_act = 0, o_obs = o_act + up(N * 16), o_term = o_obs + up(N * D * 4), o_rew = o_term + up(N * D * 4);
-    const size_t o_epr = o_rew + up(N * 4), o_fnd = o_epr + up(N * 4), o_epl = o_fnd + up(N * 4), o_done = o_epl + up(N * 4);
-    if (!env->stage) DN_CUDA(cudaMalloc(&env->stage, o_done + up(N)));
+    const IoLayout L = io_layout(N, D, true);
+    if (!env->stage) DN_CUDA(cudaMalloc(&env->stage, L.bytes));
     char* d = static_cast<char*>(env->stage);
     cudaStream_t st = env->host_stream;
-    DN_CUDA(cudaMemcpyAsync(d + o_act, h->actions, N * 16, cudaMemcpyHostToDevice, st));
-    dn_step_io io;
-    io.actions = reinterpret_cast<const float*>(d + o_act);
-    io.obs = reinterpret_cast<float*>(d + o_obs);
-    io.reward = reinterpret_cast<float*>(d + o_rew);
-    io.done = reinterpret_cast<uint8_t*>(d + o_done);
-    io.terminal_obs = h->terminal_obs ? reinterpret_cast<float*>(d + o_term) : nullptr;
-    io.found_targets = h->found_targets ? reinterpret_cast<int32_t*>(d + o_fnd) : nullptr;
-    io.episode_return = h->episode_return ? reinterpret_cast<float*>(d + o_epr) : nullptr;
-    io.episode_length = h->episode_length ? reinterpret_cast<int32_t*>(d + o_epl) : nullptr;
-    const int rc = launch_step(env, &io, 1, 1, st);
+    DN_CUDA(cudaMemcpyAsync(d + L.act, h->actions, N * 16, cudaMemcpyHostToDevice, st));
+    dn_step_io io = io_at(L, d);
+    if (!h->terminal_obs) io.terminal_obs = nullptr;
+    if (!h->found_targets) io.found_targets = nullptr;
+    if (!h->episode_return) io.episode_return = nullptr;
+    if (!h->episode_length) io.episode_length = nullptr;
+    dn::StepIO k;
+    rc = step_io(env, &io, 1, k);
+    if (rc == DN_OK) rc = launch_step(env, k, 1, 1, st, true);
     if (rc != DN_OK) return rc;
-    DN_CUDA(cudaMemcpyAsync(h->obs, d + o_obs, N * D * 4, cudaMemcpyDeviceToHost, st));
-    DN_CUDA(cudaMemcpyAsync(h->reward, d + o_rew, N * 4, cudaMemcpyDeviceToHost, st));
-    DN_CUDA(cudaMemcpyAsync(h->done, d + o_done, N, cudaMemcpyDeviceToHost, st));
-    if (h->found_targets) DN_CUDA(cudaMemcpyAsync(h->found_targets, d + o_fnd, N * 4, cudaMemcpyDeviceToHost, st));
-    if (h->terminal_obs) DN_CUDA(cudaMemcpyAsync(h->terminal_obs, d + o_term, N * D * 4, cudaMemcpyDeviceToHost, st));
-    if (h->episode_return) DN_CUDA(cudaMemcpyAsync(h->episode_return, d + o_epr, N * 4, cudaMemcpyDeviceToHost, st));
-    if (h->episode_length) DN_CUDA(cudaMemcpyAsync(h->episode_length, d + o_epl, N * 4, cudaMemcpyDeviceToHost, st));
+    DN_CUDA(cudaMemcpyAsync(h->obs, io.obs, N * D * 4, cudaMemcpyDeviceToHost, st));
+    DN_CUDA(cudaMemcpyAsync(h->reward, io.reward, N * 4, cudaMemcpyDeviceToHost, st));
+    DN_CUDA(cudaMemcpyAsync(h->done, io.done, N, cudaMemcpyDeviceToHost, st));
+    if (h->found_targets) DN_CUDA(cudaMemcpyAsync(h->found_targets, io.found_targets, N * 4, cudaMemcpyDeviceToHost, st));
+    if (h->terminal_obs) DN_CUDA(cudaMemcpyAsync(h->terminal_obs, io.terminal_obs, N * D * 4, cudaMemcpyDeviceToHost, st));
+    if (h->episode_return) DN_CUDA(cudaMemcpyAsync(h->episode_return, io.episode_return, N * 4, cudaMemcpyDeviceToHost, st));
+    if (h->episode_length) DN_CUDA(cudaMemcpyAsync(h->episode_length, io.episode_length, N * 4, cudaMemcpyDeviceToHost, st));
     DN_CUDA(cudaStreamSynchronize(st));
     return DN_OK;
 }
@@ -1260,7 +1251,7 @@ int dn_gae(const float* rewards, const float* values, const uint8_t* done, const
 
 static int state_xfer(dn_env* env, const dn_state_view* v, bool set, void* stream) {
     if (!env || !v) return fail(DN_EINVAL, "dn_get/set_state: null argument");
-    { const int rq = srv_quiesce(env); if (rq != DN_OK) return rq; }
+    { const int rq = quiesce(env, set ? "dn_set_state" : "dn_get_state"); if (rq != DN_OK) return rq; }
     DeviceGuard guard(env->device);
     dn::StateView V;
     V.pos = v->pos; V.quat = v->quat; V.vel = v->vel; V.rpy_rates = v->rpy_rates; V.ang_v = v->ang_v;
@@ -1282,7 +1273,7 @@ int dn_set_state(dn_env* env, const dn_state_view* view, void* stream) { return 
 
 int dn_episode_stats(dn_env* env, dn_stats* host_out, int clear, void* stream) {
     if (!env || !host_out) return fail(DN_EINVAL, "dn_episode_stats: null argument");
-    { const int rq = srv_quiesce(env); if (rq != DN_OK) return rq; }
+    { const int rq = quiesce(env, "dn_episode_stats"); if (rq != DN_OK) return rq; }
     DeviceGuard guard(env->device);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     dn::Stats h;

@@ -7,8 +7,10 @@
 ``step_wait`` contract with the worker's auto-reset semantics
 (``terminal_observation``, ``TimeLimit.truncated``, Monitor's ``episode`` dict,
 ``found_targets``), but one kernel launch per vector step instead of N processes.
-Host buffers are pinned; every ``step`` is H2D(actions) -> kernel -> D2H(results) on
-the environment's stream.
+Host buffers are pinned.  By default (``host_path="zero_copy"``) every ``step`` is one
+kernel launch that reads the actions from and writes the results to those buffers over
+PCIe; ``host_path="slab"`` copies them with one H2D and one D2H DMA around the kernel, and
+``host_path="server"`` keeps the kernel resident between steps.
 """
 from __future__ import annotations
 

@@ -228,7 +228,7 @@ int dn_step_many(dn_env* env, const dn_step_io* io, int num_steps, int per_step_
  * makes; staging buffers and the stream belong to the handle. */
 int dn_step_host(dn_env* env, const dn_step_io* host_io);
 
-/* The lowest-latency form of the host-buffer call: the HANDLE owns one pinned host slab laid out
+/* The host-buffer call on handle-owned buffers, moved by DMA: the HANDLE owns one pinned host slab laid out
  *   actions | obs | reward | found_targets | done | [episode_return | episode_length | terminal_obs]
  * and a device slab of the same layout.  dn_host_buffers fills `out` with HOST pointers into that slab (write actions
  * there, read results there: no copy on either side); `with_episode_info` = 0 leaves the three bracketed outputs NULL.
@@ -236,7 +236,8 @@ int dn_step_host(dn_env* env, const dn_step_io* host_io);
  * one H2D DMA of the actions, the fused kernel, one D2H DMA of the contiguous outputs (whose last word is the completion
  * flag the host waits on) -- instead of a kernel that reads and writes host memory over PCIe word by word plus a poll of the
  * stream.  dn_step_host_async returns as soon as the graph is launched, dn_step_host_wait when the results are in the slab
- * (SB3 VecEnv.step_async / step_wait).  Any other pointer set takes the paths described above. */
+ * (SB3 VecEnv.step_async / step_wait).  Any other pointer set takes the paths described above; dn_step_host_async accepts only
+ * the zero-copy one.  Until dn_step_host_wait has returned, every other call on the handle fails with DN_EINVAL. */
 int dn_host_buffers(dn_env* env, int with_episode_info, dn_step_io* out);
 int dn_step_host_async(dn_env* env, const dn_step_io* host_io);
 int dn_step_host_wait(dn_env* env);

@@ -295,6 +295,47 @@ def test_step_host_slab_graph_path_equals_device_step(N, with_info):
         e.close()
 
 
+@pytest.mark.parametrize("form", ["zero_copy", "slab"])
+def test_step_host_async_in_flight_refuses_other_calls(form):
+    """While a dn_step_host_async step has not been waited for, it still runs against the handle's state: every other call that
+    touches that state refuses -- the resident server path of dn_step_host included -- and after dn_step_host_wait the handle
+    equals one stepped with dn_step on the same actions."""
+    from drl_dronenavigation_b200 import _lib as L
+    N, D, T = 777, 13, 6
+    envs = [_make("circle", N, 8)[0] for _ in range(2)]
+    for e in envs:
+        e.reset()
+    pin = lambda *s, dtype: torch.empty(*s, dtype=dtype).pin_memory()
+    h = dict(actions=pin(N, 4, dtype=torch.float32), obs=pin(N, D, dtype=torch.float32), reward=pin(N, dtype=torch.float32),
+             done=pin(N, dtype=torch.uint8), found_targets=pin(N, dtype=torch.int32))
+    io_pin = envs[1]._make_io(h["actions"], h["obs"], h["reward"], h["done"], found=h["found_targets"])
+    if form == "slab":
+        io, b = envs[1].host_buffers()
+    else:
+        io, b = io_pin, {k: v.numpy() for k, v in h.items()}
+    envs[1].host_server(2000)
+    acts = _actions("saturating", T, N, seed=8)
+    a_dev = torch.from_numpy(acts[0]).cuda()
+    for t in range(T):
+        o, r, d, f = envs[0].step(torch.from_numpy(acts[t]).cuda())
+        b["actions"][...] = acts[t]
+        envs[1].step_host_async(io)
+        for call in (lambda: envs[1].step_host(io_pin), lambda: envs[1].step(a_dev), envs[1].reset, envs[1].get_state,
+                     envs[1].episode_stats):
+            with pytest.raises(L.DroneNavError, match="not been waited"):
+                call()
+        envs[1].step_host_wait()
+        for name, dev_t in (("obs", o), ("reward", r), ("done", d), ("found_targets", f)):
+            np.testing.assert_array_equal(b[name], dev_t.cpu().numpy(), err_msg=f"{name} t={t}")
+    sa, sb = envs[0].get_state(), envs[1].get_state()
+    for k in sa:
+        assert torch.equal(sa[k], sb[k]), k
+    assert envs[1].episode_stats() == envs[0].episode_stats()
+    assert envs[1].host_server_stats()["steps"] == 0
+    for e in envs:
+        e.close()
+
+
 @pytest.mark.parametrize("N,norm,idle_us", [(777, False, 2000), (4096, True, 2000), (12, True, 50), (1, False, 2000)])
 def test_step_host_resident_server_equals_device_step(N, norm, idle_us):
     """dn_host_server: the RESIDENT step kernel (dn_step_many variant, one host doorbell per step) == dn_step launch by launch --
