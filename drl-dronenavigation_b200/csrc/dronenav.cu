@@ -120,14 +120,18 @@ __device__ __forceinline__ void prefetch_l2(const void* p) {
 // their finished episodes to it, and dn_episode_stats reduces the slots.  (A first version used one
 // atomicAdd per warp per counter on 7 GLOBAL addresses; with ~12 % of the envs finishing per step
 // that serialised in L2 and doubled the step time at 4 Mi envs.)
-struct BlockAcc { float ret; int len, fnd, eps_suc, cra_tru; };   // eps|suc and cra|tru packed 16:16 (<= 65535 steps per launch)
+// eps|suc and cra|tru are packed 16:16.  A lane adds at most one episode per step, and the multi-step kernel flushes and
+// clears its accumulator every kStatsFlushSteps steps, so every half stays below 2^15: the low halves never carry into the
+// high ones and the arithmetic shift of a high half never sees a sign bit, whatever num_steps is.
+struct BlockAcc { float ret; int len, fnd, eps_suc, cra_tru; };
+constexpr int kStatsFlushSteps = 32767;
 
 __device__ __forceinline__ int warp_sum(int v) { return __reduce_add_sync(0xffffffffu, v); }
 
 // ---- Monitor statistics: warp shuffle -> this CTA's slot.  Only the (up to 4) warps of one CTA ever
 // touch a slot, so these reductions do not contend; integer sums are exact and the float returns are
 // added as doubles (exact for any realistic count), so the totals do not depend on arrival order.
-// (per-lane counts are < 2^16 per launch, so a warp's packed 16:16 sums need the two halves summed apart)
+// (per-lane counts are < 2^15 between flushes, so a warp's packed 16:16 sums need the two halves summed apart)
 __device__ __forceinline__ void flush_stats(const Params& P, const BlockAcc& acc, const int tid) {
     const int eps_w = warp_sum(acc.eps_suc & 0xffff);
     if (eps_w != 0) {                              // warp-uniform
@@ -326,6 +330,11 @@ step_kernel(const __grid_constant__ Params P, const __grid_constant__ StepIO io,
                 }
             }
         }
+        if (MULTI && !srv && (t + 1) % kStatsFlushSteps == 0) {
+            // t is the same for every thread, so the warp collectives of flush_stats stay convergent
+            flush_stats(P, acc, tid);
+            acc = BlockAcc{0.f, 0, 0, 0, 0};
+        }
         if (MULTI && srv) {
             // the step is complete for the host when every CTA's stores (bulk stores of the observation rows included) are
             // visible system-wide: count this CTA done; the last one writes the step's sequence number to the pinned word
@@ -445,7 +454,7 @@ __global__ void reset_kernel(const __grid_constant__ Params P, const uint8_t* ma
         if (P.spawn_mode == DN_SPAWN_LINE) spawn_line(P, i, s.ep_count, s.px, s.py, s.pz);
         else spawn_midpoint(P, i, s.ep_count, s.px, s.py, s.pz, roll);
         P.spawn[i] = make_float4(s.px, s.py, s.pz, static_cast<float>(roll));
-        if (P.aux && P.rw.mode == RW_REACHING) { float4 ax = P.aux[i]; ax.x = s.px; ax.y = s.py; ax.z = s.pz; P.aux[i] = ax; }
+        if (P.aux && P.rw.mode == RW_REACHING) reaching_travel_after_spawn(P, i, s.px, s.py, s.pz);
         const float4 t0 = target_at(P, roll);
         const float dx = s.px - t0.x, dy = s.py - t0.y, dz = s.pz - t0.z;
         D0 = sqrtf(dx * dx + dy * dy + dz * dz);
@@ -569,8 +578,11 @@ __global__ void state_xfer_kernel(const __grid_constant__ Params P, const __grid
         }
     }
     if (SET) {
-        if (V.quat) {   // resetBasePositionAndOrientation -> read-back returns a unit quaternion
-            const float inv = rsqrtf(s.qx * s.qx + s.qy * s.qy + s.qz * s.qz + s.qw * s.qw);
+        // resetBasePositionAndOrientation -> read-back returns a unit quaternion.  One that is already unit to FP32 precision
+        // (every quaternion dn_get_state returns) is kept bit for bit, so that a get / set round trip clones the state exactly.
+        const float q2 = s.qx * s.qx + s.qy * s.qy + s.qz * s.qz + s.qw * s.qw;
+        if (V.quat && fabsf(q2 - 1.0f) > 4e-6f) {
+            const float inv = rsqrtf(q2);
             s.qx *= inv; s.qy *= inv; s.qz *= inv; s.qw *= inv;
         }
         s.bits = (static_cast<uint32_t>(idx) << kIdxShift) | (jf ? kJustFoundBit : 0u) | (static_cast<uint32_t>(steps) & kStepsMask);

@@ -172,7 +172,8 @@ typedef struct dn_state_view {
     float*    last_rpm_sum;   /* [N]    sum(last_clipped_action) (drag only, BaseAviary.py:429,442) */
     double*   obs_rms;        /* [N,2*obs_dim+1] FP64 mean | var | count, the dtype of the reference's RunningMeanStd
                                  (normalize.py:10-47); only if normalize_obs */
-    float*    aux;            /* [N,4] _current_position.xyz | last travel with DN_REWARD_REACHING; PBDroneEnv._last_action with
+    float*    aux;            /* [N,4] _current_position.xyz | last travel with DN_REWARD_REACHING (with a random spawn mode
+                                 _last_position.xyz | last travel); PBDroneEnv._last_action with
                                  DN_REWARD_BOOTSTRAPPED / DN_REWARD_CHAMP; absent otherwise */
     float*    rew_rms;        /* [N,4] returns | mean | var | count (normalize.py:100-147); only if normalize_reward */
     float*    spawn;          /* [N,4] INIT_XYZS[0] of the current episode | target roll; only with a random spawn mode */

@@ -54,6 +54,14 @@ def upload_oracle_state(gpu_env, workers):
     gpu_env.set_state(st)
 
 
+def return_sum_bound(abs_sum, n_terms, max_per_lane):
+    """|return_sum - FP64 sum| bound of the Monitor statistics (dn_episode_stats) over `n_terms` finished episodes whose
+    returns have absolute sum `abs_sum`.  A lane adds its finished episodes (at most `max_per_lane` between two flushes) one
+    after another in FP32, a warp adds its 32 lanes in a 5-level shuffle tree, and the warp sums are added as FP64:
+    (k - 1 + 5) u sum|r| with u = 2^-24, plus 2^-53 sum|r| per FP64 addition.  dn_step has k = 1."""
+    return (max_per_lane - 1 + 5) * 2.0 ** -24 * abs_sum + (n_terms + 1) * 2.0 ** -53 * abs_sum
+
+
 def _np(x):
     return x.detach().cpu().numpy() if hasattr(x, "detach") else np.asarray(x)
 

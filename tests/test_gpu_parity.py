@@ -175,16 +175,35 @@ def test_single_step_random_states_all_branches():
     assert total.near_ties <= 8
 
 
-@pytest.mark.parametrize("kw", [{}, {"normalize_obs": True, "normalize_reward": True, "clip_reward": 10.0},
-                                {"reward_id": 4, "random_spawn": "midpoint", "seed": 77}, {"reward_id": 5, "random_spawn": "line", "seed": 78},
-                                {"reward_id": 3, "physics": "PYB_GND_DRAG_DW"},
-                                {"act": "VEL"}, {"act": "PID", "drone_model": "CF2P", "physics": "PYB_GND"}, {"act": "RPM", "drone_model": "RACE"},
-                                {"reward_id": 8, "random_spawn": "line", "seed": 79}, {"reward_id": 9, "normalize_reward": True}],
-                         ids=["default", "wrappers", "reaching_midpoint", "progress_line", "her_drag_gnd", "vel", "cf2p_pid_gnd", "race_rpm",
-                              "bootstrapped_line", "champ_normrew"])
-def test_step_many_matches_repeated_step(kw):
+STEP_MANY_CONFIGS = [
+    ("default", {}), ("wrappers", {"normalize_obs": True, "normalize_reward": True, "clip_reward": 10.0}),
+    ("reaching_midpoint", {"reward_id": 4, "random_spawn": "midpoint", "seed": 77}),
+    ("progress_line", {"reward_id": 5, "random_spawn": "line", "seed": 78}), ("her_drag_gnd", {"reward_id": 3, "physics": "PYB_GND_DRAG_DW"}),
+    ("vel", {"act": "VEL"}), ("cf2p_pid_gnd", {"act": "PID", "drone_model": "CF2P", "physics": "PYB_GND"}),
+    ("race_rpm", {"act": "RPM", "drone_model": "RACE"}), ("bootstrapped_line", {"reward_id": 8, "random_spawn": "line", "seed": 79}),
+    ("champ_normrew", {"reward_id": 9, "normalize_reward": True}),
+]
+# N = 1000: every step's observation rows start 16-byte aligned (bulk TMA store); N = 777 with obs_dim 13: three steps in
+# four start misaligned, and every warp of such a step takes the per-element store.  The first id of each configuration
+# (N = 1000, per-step outputs) keeps its plain name.
+STEP_MANY_CASES = [pytest.param(kw, N, per_step, id=name if (N, per_step) == (1000, True) else
+                                f"{name}-n{N}-{'per_step' if per_step else 'last_step'}")
+                   for name, kw in STEP_MANY_CONFIGS for N in (1000, 777) for per_step in (True, False)]
+def bits_equal(a, b):
+    """Bit-for-bit equality of two tensors (NaN payloads included)."""
+    if a.dtype.is_floating_point:
+        a, b = a.view(torch.int32), b.view(torch.int32)
+    return torch.equal(a, b)
+
+
+@pytest.mark.parametrize("kw,N,per_step", STEP_MANY_CASES)
+def test_step_many_matches_repeated_step(kw, N, per_step):
     """dn_step_many (T steps, state in registers) is bit-identical to T dn_step launches -- also with the fused
-    wrappers, the optional planes (aux / spawn / reward statistics) and the physics add-ons in play."""
+    wrappers, the optional planes (aux / spawn / reward statistics) and the physics add-ons in play, all eight outputs passed.
+    per_step_outputs = 1: every output [T, N, ...], the terminal observation and the episode outputs on the finished rows.
+    per_step_outputs = 0: only the last step's outputs, the episode outputs only on the rows finished at that step, sentinels
+    everywhere else.  The Monitor counts are equal; the return sums are within parity_utils.return_sum_bound of the FP64
+    sum of the returns dn_step emitted (k = 1 for dn_step, k = the most episodes of one env for the one flush of dn_step_many)."""
     from drl_dronenavigation_b200 import Physics
     from drl_dronenavigation_b200.enums import ActionType, DroneModel
     kw = dict(kw)
@@ -196,20 +215,50 @@ def test_step_many_matches_repeated_step(kw):
         kw["drone_model"] = getattr(DroneModel, kw["drone_model"])
     norm = kw.pop("normalize_obs", False)
     track = "reaching" if "random_spawn" in kw else "circle"
-    envA, _ = _make(track, 1000, 8, normalize_obs=norm, **kw)
-    envB, _ = _make(track, 1000, 8, normalize_obs=norm, **kw)
+    envA, _ = _make(track, N, 8, normalize_obs=norm, **kw)
+    envB, _ = _make(track, N, 8, normalize_obs=norm, **kw)
     envA.reset(); envB.reset()
-    T = 40
-    acts = torch.from_numpy(_actions("saturating", T, 1000, seed=11)).to(envA.device)
-    outs = envB.step_many(acts, per_step_outputs=True)
+    T, D, dev = 40, envA.obs_dim, envA.device
+    acts = torch.from_numpy(_actions("saturating", T, N, seed=11)).to(dev)
+    lead = (T,) if per_step else ()
+    nan = float("nan")
+    outs = dict(obs=torch.full((*lead, N, D), nan, device=dev), terminal_obs=torch.full((*lead, N, D), nan, device=dev),
+                reward=torch.full((*lead, N), nan, device=dev), done=torch.full((*lead, N), 255, dtype=torch.uint8, device=dev),
+                found_targets=torch.full((*lead, N), -1, dtype=torch.int32, device=dev),
+                episode_return=torch.full((*lead, N), nan, device=dev),
+                episode_length=torch.full((*lead, N), -1, dtype=torch.int32, device=dev))
+    envB.step_many(acts, per_step_outputs=per_step, out=outs)
+    ep_ret, ep_count = [], torch.zeros(N, dtype=torch.int64, device=dev)
     for t in range(T):
         o, r, d, f = envA.step(acts[t])
-        assert torch.equal(o, outs["obs"][t]) and torch.equal(r, outs["reward"][t])
-        assert torch.equal(d, outs["done"][t]) and torch.equal(f, outs["found_targets"][t])
+        done = d != 0
+        ep_ret.append(envA.episode_return[done].double())
+        ep_count += done
+        if per_step:
+            got = {k: v[t] for k, v in outs.items()}
+        elif t == T - 1:
+            got = outs
+        else:
+            continue
+        assert bits_equal(o, got["obs"]) and bits_equal(r, got["reward"]), t
+        assert torch.equal(d, got["done"]) and torch.equal(f, got["found_targets"]), t
+        assert bits_equal(envA.terminal_obs[done], got["terminal_obs"][done]), t
+        assert bits_equal(envA.episode_return[done], got["episode_return"][done]), t
+        assert torch.equal(envA.episode_length[done], got["episode_length"][done]), t
+        if not per_step:                                     # rows not finished at the last step keep the sentinels
+            assert bool(torch.isnan(got["terminal_obs"][~done]).all()) and bool(torch.isnan(got["episode_return"][~done]).all())
+            assert bool((got["episode_length"][~done] == -1).all())
     sa, sb = envA.get_state(), envB.get_state()
     for k in sa:
-        assert torch.equal(sa[k], sb[k]), k
-    assert envA.episode_stats()["episodes"] == envB.episode_stats()["episodes"] > 0
+        assert bits_equal(sa[k], sb[k]), k
+    stA, stB = envA.episode_stats(), envB.episode_stats()
+    for k in ("episodes", "length_sum", "found_targets", "successes", "crashes", "truncations"):
+        assert stA[k] == stB[k], (k, stA, stB)
+    assert stA["episodes"] == int(ep_count.sum()) > 0
+    ep_ret = torch.cat(ep_ret)
+    ref, abs_sum, n = float(ep_ret.sum()), float(ep_ret.abs().sum()), ep_ret.numel()
+    assert abs(stA["return_sum"] - ref) <= PU.return_sum_bound(abs_sum, n, 1), (stA["return_sum"], ref)
+    assert abs(stB["return_sum"] - ref) <= PU.return_sum_bound(abs_sum, n, int(ep_count.max())), (stB["return_sum"], ref)
     envA.close(); envB.close()
 
 
