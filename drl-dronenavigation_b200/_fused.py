@@ -1,5 +1,6 @@
-"""Torch plumbing shared by the ctypes faces of the library's MLP handles: ``ppo.FusedUpdate`` (include/dnppo.h) and
-``sac.FusedSACActor`` (include/dnsac.h).  Kept apart from ``_lib`` so that the ctypes binding does not import torch."""
+"""Torch plumbing shared by the PPO and SAC learners: the ctypes faces of the library's MLP handles (``ppo.FusedUpdate``,
+include/dnppo.h, and ``sac.FusedSACActor``, include/dnsac.h) and the CUDA-graph capture of the update steps and of the trainers'
+collection phases.  Kept apart from ``_lib`` so that the ctypes binding does not import torch."""
 from __future__ import annotations
 
 import ctypes as C
@@ -43,6 +44,58 @@ def widths_ok(arch, obs_dim: int) -> bool:
     and 512, and 1 <= obs_dim <= 64 (one padded 64-column k-block)."""
     arch = tuple(arch)
     return 1 <= len(arch) <= 4 and all(w % 128 == 0 and 128 <= w <= 512 for w in arch) and 1 <= obs_dim <= 64
+
+
+def capture_graphs(stages, warmup, tensors, optimizers, device) -> list:
+    """One CUDA graph per callable of `stages`, all from one shared memory pool (a stage may consume tensors an earlier stage
+    produced), captured after ``warmup()`` has run on a side stream (lazy kernel loading, allocator, library workspaces,
+    optimiser state).  The warm-up takes real steps, so afterwards every tensor of `tensors` and the state of every optimiser
+    of `optimizers` is put back bit for bit, in place (the graphs bake those pointers in); optimiser state the warm-up
+    created ends zeroed, which is a fresh Adam state.  Every rank of a data-parallel job must run the same warm-up."""
+    opt_state = lambda: [v for o in optimizers for st in o.state.values() for v in st.values() if torch.is_tensor(v)]
+    saved = [(t, t.detach().clone()) for t in list(tensors) + opt_state()]
+    side = torch.cuda.Stream(device=device)
+    side.wait_stream(torch.cuda.current_stream(device))
+    quiet = getattr(torch.autograd.graph, "set_warn_on_accumulate_grad_stream_mismatch", None)
+    if quiet is not None:        # the gradient buckets were created on the current stream, the warm-up runs on a side stream: intended
+        quiet(False)
+    with torch.cuda.stream(side):
+        warmup()
+    torch.cuda.current_stream(device).wait_stream(side)
+    with torch.no_grad():
+        for v in opt_state():
+            v.zero_()
+        for t, s in saved:
+            t.copy_(s)
+    pool = torch.cuda.graph_pool_handle()
+    graphs = []
+    for stage in stages:
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g, pool=pool):
+            stage()
+        graphs.append(g)
+    return graphs
+
+
+class PhaseGraph:
+    """A phase of a trainer (a callable that issues the same launches every time) run from a CUDA graph: the first call launches
+    it (loading every kernel), the next call captures and replays it, later calls with the same key replay.  A new key captures
+    again, without another launched call.  A call with ``enabled`` false launches."""
+
+    def __init__(self):
+        self.key, self.graph, self.warm = None, None, False
+
+    def run(self, enabled: bool, key, phase) -> None:
+        if not (enabled and self.warm):
+            phase()
+            self.warm = True
+            return
+        if self.graph is None or self.key != key:
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                phase()
+            self.key, self.graph = key, g
+        self.graph.replay()
 
 
 class Handle:

@@ -296,16 +296,9 @@ def load_sb3_sac_zip(path: str, learner, load_optimizer: bool = False, strict: b
                 with torch.no_grad():
                     learner.log_ent_coef.copy_(pv["log_ent_coef"].reshape(learner.log_ent_coef.shape).to(learner.log_ent_coef.device))
         if load_optimizer:
-            for member, opt in (("actor.optimizer.pth", learner.actor_opt), ("critic.optimizer.pth", learner.critic_opt),
-                                ("ent_coef_optimizer.pth", learner.ent_opt)):
-                if member in names:
-                    st = torch.load(io.BytesIO(zf.read(member)), map_location="cpu", weights_only=False)
-                    own = opt.state_dict()
-                    if len(st.get("state", {})) in (0, len(own["param_groups"][0]["params"])):
-                        own["state"] = st.get("state", {})
-                        opt.load_state_dict(own)
-            if hasattr(learner, "_graphs"):
-                learner._graphs = None            # optimiser state tensors were re-created: captured CUDA graphs must be rebuilt
+            members = {"actor": "actor.optimizer.pth", "critic": "critic.optimizer.pth", "ent_coef": "ent_coef_optimizer.pth"}
+            learner.load_optimizer_state({name: torch.load(io.BytesIO(zf.read(m)), map_location="cpu", weights_only=False)
+                                          for name, m in members.items() if m in names})
         data = {}
         if "data" in names:
             try:

@@ -23,7 +23,7 @@ import torch
 import torch.distributed as dist
 from torch import nn
 
-from ._fused import Handle, flat_views, offsets, sm100, widths_ok
+from ._fused import Handle, PhaseGraph, capture_graphs, flat_views, offsets, sm100, widths_ok
 from ._fused import world as _world
 
 
@@ -356,7 +356,7 @@ class PPOLearner:
         self.cfg, self.device = cfg, torch.device(device)
         torch.manual_seed(cfg.seed)                     # same seed on every rank -> identical initial parameters
         self.policy = ActorCritic(obs_dim, act_dim, cfg).to(self.device)
-        self._graphs = None                             # (shape key, graph A, graph B, static tensors); built lazily
+        self._graphs = None                             # (key, graphs, static tensors) of the update in use; built lazily
         self.use_graph = bool(cfg.cuda_graph) and self.device.type == "cuda"
         self.opt = torch.optim.Adam(self.policy.parameters(), lr=cfg.learning_rate, eps=cfg.adam_eps,
                                     capturable=self.use_graph)
@@ -395,9 +395,13 @@ class PPOLearner:
                 torch.cuda.synchronize(self.device)
                 self.fused.close()
             self.fused = FusedUpdate(self, rows)
-            self._graphs = None            # parameters were re-seated: graphs of the torch path are stale
-            self._fused_graphs = None
+            self.drop_graphs()             # parameters and Adam state were re-seated
         return self.fused
+
+    def drop_graphs(self) -> None:
+        """Forgets the captured update graphs (the next update captures again).  Called by everything that replaces a tensor
+        the graphs point to."""
+        self._graphs = None
 
     def forward(self, obs):
         """(mean, value) of the policy: fused kernels when available, else the torch modules."""
@@ -455,14 +459,13 @@ class PPOLearner:
             # the ~25 kernels of a minibatch step replayed from CUDA graphs (one for the gradient half, one for the apply half; a
             # single one when there is no all-reduce in between): removes the launch gaps between the short dependent kernels.
             # Graphs bake pointers in, so the rollout is staged in static tensors and the minibatch indices in a static buffer.
-            fg = self._fused_graphs
-            key = (B, mb, obs.shape[1], actions.shape[1], world, peer)
-            if fg is None or fg["key"] != key or fg["fu"] is not fu:
-                fg = self._capture_fused(fu, key)
-            for dst, src in zip(fg["static"], (obs, actions, old_logp, old_values, advantages, returns)):
+            key = ("fused", B, mb, obs.shape[1], actions.shape[1], world, peer)
+            if self._graphs is None or self._graphs[0] != key:
+                self._capture_fused(fu, key)
+            _, graphs, (static, idx) = self._graphs
+            for dst, src in zip(static, (obs, actions, old_logp, old_values, advantages, returns)):
                 dst.copy_(src)
-            keep = list(fg["static"])
-            graphs = fg
+            keep = list(static)
         else:
             keep = [t.contiguous().float() for t in (obs, actions, old_logp, old_values, advantages, returns)]
         ro.obs, ro.actions, ro.old_log_prob, ro.old_values, ro.advantages, ro.returns = [t.data_ptr() for t in keep]
@@ -480,13 +483,13 @@ class PPOLearner:
             keep.append(perm)
             for k in range(n_mb):
                 if graphs is not None:
-                    graphs["idx"].copy_(perm[k * mb:(k + 1) * mb])
-                    graphs["grad"].replay()              # one rank, or peer all-reduce: the whole step
+                    idx.copy_(perm[k * mb:(k + 1) * mb])
+                    graphs[0].replay()                   # one rank, or peer all-reduce: the whole step
                     if world > 1:
                         self.allreduce_calls += 1
                         if not peer:
                             dist.all_reduce(self._bucket, op=dist.ReduceOp.SUM)
-                            graphs["apply"].replay()
+                            graphs[1].replay()
                 else:
                     fu.minibatch_grad(ro, perm[k * mb:(k + 1) * mb])
                     if world > 1:
@@ -516,46 +519,32 @@ class PPOLearner:
                 "optimizer_steps": st.optimizer_steps, "early_stop": bool(st.early_stop), "launched_minibatches": launched,
                 "grad_norm": st.last_grad_norm, "std": float(self.policy.log_std.detach().exp().mean()), "impl": "fused/" + cfg.mlp_precision}
 
-    _fused_graphs = None
-
     def _capture_fused(self, fu: FusedUpdate, key):
-        """CUDA graphs of the fused minibatch step for rollouts of `key` = (B, mb, D, A, world, peer).  One graph for the whole step
-        with one rank or with the peer-memory all-reduce (three kernels of the library between the halves); with ncclAllReduce the
-        collective sits between two graphs."""
-        B, mb, D, A, world, peer = key
+        """CUDA graphs of the fused minibatch step for rollouts of `key` = ("fused", B, mb, D, A, world, peer).  One graph for the
+        whole step with one rank or with the peer-memory all-reduce (three kernels of the library between the halves); with
+        ncclAllReduce the collective sits between two graphs."""
+        _, B, mb, D, A, world, peer = key
         dev = self.device
         f = dict(dtype=torch.float32, device=dev)
         static = [torch.zeros(B, D, **f), torch.zeros(B, A, **f), torch.zeros(B, **f), torch.zeros(B, **f), torch.zeros(B, **f), torch.zeros(B, **f)]
         idx = torch.arange(mb, dtype=torch.long, device=dev)
         ro = fu.L.dn_ppo_rollout()
         ro.obs, ro.actions, ro.old_log_prob, ro.old_values, ro.advantages, ro.returns = [t.data_ptr() for t in static]
-        # warm-up outside the capture (lazy kernel loading, launch attributes, plans for `mb` rows): one gradient half on zeros, then
-        # an apply half that is a no-op because the early-stop vote in the bucket's extra element is forced to "stop"
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):
-            fu.begin_update()
+
+        def step():
             fu.minibatch_grad(ro, idx)
             if world > 1 and peer:
-                fu.allreduce()                 # (every rank captures at the same point of the program: the peers answer)
-            self._bucket[-1] = 1.0
-            fu.minibatch_apply()
-            fu.begin_update()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        torch.cuda.synchronize(dev)
-        g_grad, g_apply = torch.cuda.CUDAGraph(), None
-        with torch.cuda.graph(g_grad):
-            fu.minibatch_grad(ro, idx)
-            if world > 1 and peer:
-                fu.allreduce()
+                fu.allreduce()                 # (every rank warms up and captures at the same point of the program: the peers answer)
             if world == 1 or peer:
                 fu.minibatch_apply()
-        if world > 1 and not peer:
-            g_apply = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g_apply):
-                fu.minibatch_apply()
-        self._fused_graphs = {"key": key, "fu": fu, "static": static, "idx": idx, "ro": ro, "grad": g_grad, "apply": g_apply}
-        return self._fused_graphs
+        stages = (step,) if world == 1 or peer else (step, fu.minibatch_apply)
+
+        def warmup():                          # lazy kernel loading, launch attributes, plans for `mb` rows: one step on zeros
+            fu.begin_update()
+            for stage in stages:
+                stage()
+        graphs = capture_graphs(stages, warmup, (fu.params, fu.exp_avg, fu.exp_avg_sq, fu.step), (), dev)
+        self._graphs = (key, graphs, (static, idx))
 
     # ---- the only collective: one flat bucket per optimiser step (between backward and clip, sb3_ppo.py:291-293)
     def _allreduce_grads(self, approx_kl=None) -> bool:
@@ -607,10 +596,11 @@ class PPOLearner:
         self._flat.mul_(torch.clamp(self.cfg.max_grad_norm / (norm + 1e-6), max=1.0))
         self.opt.step()
 
-    def _capture(self, B, mb, D, A):
-        """Two CUDA graphs per minibatch step: [gather -> forward -> losses -> backward] and [clip -> Adam], split
-        where the gradient all-reduce (and the KL early-stop decision of sb3_ppo.py:283-287) sits.  The eager
-        loop is CPU-bound (~200 small kernels per minibatch); replay makes it one launch per half."""
+    def _capture(self, key):
+        """Two CUDA graphs per minibatch step for rollouts of `key` = ("torch", B, mb, D, A): [gather -> forward -> losses ->
+        backward] and [clip -> Adam], split where the gradient all-reduce (and the KL early-stop decision of sb3_ppo.py:283-287)
+        sits.  The eager loop is CPU-bound (~200 small kernels per minibatch); replay makes it one launch per half."""
+        _, B, mb, D, A = key
         dev = self.device
         f = dict(dtype=torch.float32, device=dev)
         st = dict(obs=torch.zeros(B, D, **f), act=torch.zeros(B, A, **f), logp=torch.zeros(B, **f), val=torch.zeros(B, **f),
@@ -621,46 +611,15 @@ class PPOLearner:
             i = st["idx"]
             kl = self._forward_backward(st["obs"][i], st["act"][i], st["logp"][i], st["val"][i], st["adv"][i], st["ret"][i], st["acc"])
             st["kl"].copy_(kl)
-        # warm-up on a side stream (allocator, cuBLAS workspaces, Adam state) with the real parameters saved around it
-        saved = [p.detach().clone() for p in self.params]
-        opt_state = None
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        if hasattr(torch.autograd.graph, "set_warn_on_accumulate_grad_stream_mismatch"):
-            # the gradient buckets were created on the current stream, the warm-up runs on a side stream: intended
-            torch.autograd.graph.set_warn_on_accumulate_grad_stream_mismatch(False)
-        with torch.cuda.stream(side):
+
+        def warmup():                          # allocator, cuBLAS workspaces, Adam state
             st["idx"].copy_(torch.arange(mb, device=dev) % B)
             st["obs"].normal_(); st["act"].uniform_(-1, 1); st["adv"].normal_(); st["ret"].normal_()
             for _ in range(3):
                 half_a()
                 self._clip_and_step()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        ga, gb = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-        with torch.cuda.graph(ga):
-            half_a()
-        with torch.cuda.graph(gb):
-            self._clip_and_step()
-        # undo the warm-up: parameters and the Adam moments / step counters back to their pre-capture values
-        with torch.no_grad():
-            for p, q in zip(self.params, saved):
-                p.copy_(q)
-            for p in self.params:
-                stt = self.opt.state[p]
-                stt["exp_avg"].zero_(); stt["exp_avg_sq"].zero_(); stt["step"].zero_()
-            if self._pending_opt_state is not None:
-                self._restore_opt(self._pending_opt_state)
-        self._graphs = ((B, mb, D, A), ga, gb, st)
-
-    _pending_opt_state = None
-
-    def _snapshot_opt(self):
-        return [{k: v.clone() for k, v in self.opt.state[p].items() if torch.is_tensor(v)} for p in self.params if p in self.opt.state]
-
-    def _restore_opt(self, snap):
-        for p, sn in zip(self.params, snap):
-            for k, v in sn.items():
-                self.opt.state[p][k].copy_(v)
+        graphs = capture_graphs((half_a, self._clip_and_step), warmup, self.params, (self.opt,), dev)
+        self._graphs = (key, graphs, st)
 
     def update(self, obs, actions, old_logp, old_values, advantages, returns, generator=None) -> Dict[str, float]:
         """PPO.train (sb3_ppo.py:190-316) on flat [B, ...] tensors of this rank's rollout."""
@@ -678,11 +637,10 @@ class PPOLearner:
         n_mb = B // mb
         graphed = self.use_graph and obs.is_cuda
         if graphed:
-            key = (B, mb, obs.shape[1], actions.shape[1])
+            key = ("torch", B, mb, obs.shape[1], actions.shape[1])
             if self._graphs is None or self._graphs[0] != key:
-                self._pending_opt_state = self._snapshot_opt() if len(self.opt.state) > 0 else None
-                self._capture(*key)
-            _, ga, gb, st = self._graphs
+                self._capture(key)
+            _, (ga, gb), st = self._graphs
             st["obs"].copy_(obs); st["act"].copy_(actions); st["logp"].copy_(old_logp); st["val"].copy_(old_values)
             st["adv"].copy_(advantages); st["ret"].copy_(returns)
             acc = st["acc"].zero_()
@@ -735,7 +693,7 @@ class PPOLearner:
         own = self.opt.state_dict()
         own["state"] = state
         self.opt.load_state_dict(own)
-        self._graphs = None      # load_state_dict re-creates the state tensors: captured CUDA graphs must be rebuilt
+        self.drop_graphs()       # load_state_dict re-creates the state tensors
 
     def flat_parameters(self) -> torch.Tensor:
         return torch.cat([p.detach().reshape(-1) for p in self.params])
@@ -765,8 +723,8 @@ class PPOTrainer:
         self.low, self.high = -1.0, 1.0           # Box(-1, 1) with normalize_actions (PBDroneEnv.py:230-236)
         if cfg.rollout_impl not in ("torch", "fused"):
             raise ValueError(f"rollout_impl={cfg.rollout_impl!r}")
-        self.rollout_graph = bool(cfg.cuda_graph)
-        self._rollout_graph = None
+        self.rollout_graph = bool(cfg.cuda_graph)           # replay the T-step loop of the fused rollout from a CUDA graph
+        self._rollout_phase = PhaseGraph()                  # that graph, keyed by the handle the loop calls
         if cfg.rollout_impl == "fused":
             if self.learner.fused is None:
                 raise RuntimeError("rollout_impl='fused' needs the fused PPO handle (update_impl 'fused' or 'auto' on a compute-capability-10 "
@@ -815,7 +773,12 @@ class PPOTrainer:
         self.b_term[t].copy_(env.terminal_obs)
         self.obs.copy_(env.obs)
 
-    def _collect_rollouts_fused(self, graph: Optional[bool] = None):
+    @property
+    def _rollout_graph(self) -> Optional[torch.cuda.CUDAGraph]:
+        """The captured graph of the fused rollout (None until one was captured)."""
+        return self._rollout_phase.graph
+
+    def _collect_rollouts_fused(self):
         """collect_rollouts on dn_ppo_act.  The T-step loop is one CUDA graph, captured at the second rollout (the first one, launched
         step by step, loads every kernel) and replayed from then on; between its first and last step the host does not wait.  The
         policy is fixed during a rollout, so the truncation bootstrap of SB3's collect_rollouts (V(terminal_obs) of episodes that
@@ -825,22 +788,12 @@ class PPOTrainer:
         from . import _lib as L
         env, pol, cfg = self.env, self.learner, self.cfg
         fu = pol.fused
-        graph = self.rollout_graph if graph is None else graph
         fu.sync_weights()                       # the planes the loop reads (the loop itself does not refresh them)
-        g = self._rollout_graph
-        if graph and g is not None and g[0] is fu:
-            g[1].replay()
-        elif graph and getattr(self, "_rollout_warm", False):
-            cg = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(cg):
-                for t in range(self.T):
-                    self._rollout_step(fu, t)
-            self._rollout_graph = (fu, cg)
-            cg.replay()
-        else:
+
+        def rollout():
             for t in range(self.T):
                 self._rollout_step(fu, t)
-            self._rollout_warm = True
+        self._rollout_phase.run(self.rollout_graph, fu, rollout)
         # deferred bootstrap of truncated episodes
         D = env.obs_dim
         idx = (self.b_done.reshape(-1) == L.DN_DONE_TRUNCATED).nonzero().squeeze(1)

@@ -25,7 +25,7 @@ import torch
 import torch.distributed as dist
 from torch import nn
 
-from ._fused import Handle, flat_views, offsets, sm100, widths_ok
+from ._fused import Handle, PhaseGraph, capture_graphs, flat_views, offsets, sm100, widths_ok
 from ._fused import world as _world
 
 LOG_STD_MIN, LOG_STD_MAX = -20.0, 2.0      # SB3 sac/policies.py
@@ -140,16 +140,25 @@ class ReplayBuffer:
         self.done = torch.empty(self.cap, num_envs, **f)        # 1 only for true terminations (timeouts excluded)
 
     def add(self, obs, next_obs, act, rew, done_bits, terminal_obs):
-        p = self.pos
-        finished = done_bits != 0
-        self.obs[p].copy_(obs)
-        # the VecEnv returns the RESET observation on done; the transition's successor is the terminal observation
-        self.next_obs[p].copy_(torch.where(finished.unsqueeze(-1), terminal_obs, next_obs))
-        self.act[p].copy_(act)
-        self.rew[p].copy_(rew)
-        self.done[p].copy_(((done_bits & 1) != 0).to(torch.float32))      # DN_DONE_TERMINATED; truncated-only -> bootstrap
-        self.pos = (p + 1) % self.cap
+        self.write(self.pos, obs, next_obs, act, rew, done_bits, terminal_obs)
+        self.pos = (self.pos + 1) % self.cap
         self.full = self.full or self.pos == 0
+
+    def write(self, row, obs, next_obs, act, rew, done_bits, terminal_obs):
+        """One step of transitions into `row`: a host integer, or a one-element int64 device tensor (a CUDA graph can replay
+        the write at a slot that moves).  Leaves ``pos`` / ``full`` alone."""
+        def put(t, v):
+            # index_copy_, not t[row] = v: the advanced-index assignment made fused collection phases 3-5 % longer (B200, 1000 W)
+            if torch.is_tensor(row):
+                t.index_copy_(0, row, v.unsqueeze(0))
+            else:
+                t[row].copy_(v)
+        put(self.obs, obs)
+        # the VecEnv returns the RESET observation on done; the transition's successor is the terminal observation
+        put(self.next_obs, torch.where((done_bits != 0).unsqueeze(-1), terminal_obs, next_obs))
+        put(self.act, act)
+        put(self.rew, rew)
+        put(self.done, ((done_bits & 1) != 0).to(torch.float32))          # DN_DONE_TERMINATED; truncated-only -> bootstrap
 
     def __len__(self):
         return (self.cap if self.full else self.pos) * self.N
@@ -314,7 +323,7 @@ class SACLearner:
         lr = cfg.learning_rate
         # (the Polyak decision is baked into the captured graph, so replay is only used with target_update_interval == 1)
         self.use_graph = bool(cfg.cuda_graph) and self.device.type == "cuda" and cfg.target_update_interval == 1
-        self._graphs = None
+        self._graphs = None                                 # (key, graphs, static tensors, stage outputs); built lazily
         self.actor_opt = torch.optim.Adam(self.actor.parameters(), lr=lr, capturable=self.use_graph)
         self.critic_opt = torch.optim.Adam(self.critic.parameters(), lr=lr, capturable=self.use_graph)
         self.ent_opt = torch.optim.Adam([self.log_ent_coef], lr=lr, capturable=self.use_graph)
@@ -338,6 +347,23 @@ class SACLearner:
                 self.fused_actor.close()
             self.fused_actor = FusedSACActor(self.actor, self.actor_flat, max_rows)
         return self.fused_actor
+
+    def drop_graphs(self) -> None:
+        """Forgets the captured gradient-step graphs (the next update captures again).  Called by everything that replaces a
+        tensor the graphs point to."""
+        self._graphs = None
+
+    def load_optimizer_state(self, state: Dict[str, dict]) -> None:
+        """Adam states by optimiser: "actor", "critic" and "ent_coef" map to torch optimiser state dicts such as SB3's
+        ``actor.optimizer.pth``, ``critic.optimizer.pth`` and ``ent_coef_optimizer.pth``.  An optimiser that is not named keeps
+        its own state, and so does one whose given state covers some but not all of its parameters."""
+        for name, opt in (("actor", self.actor_opt), ("critic", self.critic_opt), ("ent_coef", self.ent_opt)):
+            if name in state:
+                own, st = opt.state_dict(), state[name].get("state", {})
+                if len(st) in (0, len(own["param_groups"][0]["params"])):
+                    own["state"] = st
+                    opt.load_state_dict(own)
+        self.drop_graphs()      # load_state_dict re-creates the state tensors
 
     # ---- one gradient step of SB3's SAC.train, in three stages around the two gradient all-reduces -----------------
     def _stage_critic(self, obs, act, rew, next_obs, done, eps_pi, eps_next, out):
@@ -383,46 +409,24 @@ class SACLearner:
         f = dict(dtype=torch.float32, device=dev)
         st = dict(obs=torch.zeros(B, D, **f), act=torch.zeros(B, A, **f), rew=torch.zeros(B, **f), next_obs=torch.zeros(B, D, **f),
                   done=torch.zeros(B, **f), eps_pi=torch.zeros(B, A, **f), eps_next=torch.zeros(B, A, **f), out=torch.zeros(4, **f))
-        nets = list(self.actor.parameters()) + list(self.critic.parameters()) + list(self.critic_target.parameters()) + [self.log_ent_coef]
-        saved = [p.detach().clone() for p in nets]
-        snap = [[{k: v.clone() for k, v in o.state[p].items() if torch.is_tensor(v)} if p in o.state else None
-                 for g in o.param_groups for p in g["params"]] for o in (self.actor_opt, self.critic_opt, self.ent_opt)]
-        keep = {}
+        keep = {}                                            # stage 1's outputs, stage 2's inputs
 
-        def run_all():
+        def critic():
             keep["a"], keep["l"], keep["e"] = self._stage_critic(st["obs"], st["act"], st["rew"], st["next_obs"], st["done"],
                                                                  st["eps_pi"], st["eps_next"], st["out"])
+
+        def actor():
             self._stage_actor(st["obs"], keep["a"], keep["l"], keep["e"], st["out"])
-            self._stage_finish()
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        if hasattr(torch.autograd.graph, "set_warn_on_accumulate_grad_stream_mismatch"):
-            # the gradient buckets were created on the current stream, the warm-up runs on a side stream: intended
-            torch.autograd.graph.set_warn_on_accumulate_grad_stream_mismatch(False)
-        with torch.cuda.stream(side):
+        stages = (critic, actor, self._stage_finish)
+
+        def warmup():
             st["obs"].normal_(); st["next_obs"].normal_(); st["act"].uniform_(-1, 1); st["eps_pi"].normal_(); st["eps_next"].normal_()
             for _ in range(3):
-                run_all()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        g1, g2, g3 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-        pool = torch.cuda.graph_pool_handle()                # stage 2 consumes tensors stage 1 produced: one shared pool
-        with torch.cuda.graph(g1, pool=pool):
-            keep["a"], keep["l"], keep["e"] = self._stage_critic(st["obs"], st["act"], st["rew"], st["next_obs"], st["done"],
-                                                                 st["eps_pi"], st["eps_next"], st["out"])
-        with torch.cuda.graph(g2, pool=pool):
-            self._stage_actor(st["obs"], keep["a"], keep["l"], keep["e"], st["out"])
-        with torch.cuda.graph(g3, pool=pool):
-            self._stage_finish()
-        with torch.no_grad():                                # undo the warm-up: parameters, targets, Adam state
-            for p, q in zip(nets, saved):
-                p.copy_(q)
-            for o, sn in zip((self.actor_opt, self.critic_opt, self.ent_opt), snap):
-                ps = [p for g in o.param_groups for p in g["params"]]
-                for p, old in zip(ps, sn):
-                    for k, v in o.state[p].items():
-                        if torch.is_tensor(v):
-                            v.copy_(old[k]) if old is not None else v.zero_()
-        self._graphs = ((B, D, A), g1, g2, g3, st, keep)
+                for stage in stages:
+                    stage()
+        nets = list(self.actor.parameters()) + list(self.critic.parameters()) + list(self.critic_target.parameters()) + [self.log_ent_coef]
+        graphs = capture_graphs(stages, warmup, nets, (self.actor_opt, self.critic_opt, self.ent_opt), dev)
+        self._graphs = ((B, D, A), graphs, st, keep)
 
     def update(self, batch, generator=None) -> Dict[str, torch.Tensor]:
         """One gradient step of SB3's SAC.train on a sampled batch (obs, act, rew, next_obs, done)."""
@@ -431,7 +435,7 @@ class SACLearner:
         if self.use_graph and obs.is_cuda:
             if self._graphs is None or self._graphs[0] != (B, D, A):
                 self._capture(B, D, A)
-            _, g1, g2, g3, st, _ = self._graphs
+            _, (g1, g2, g3), st, _ = self._graphs
             st["obs"].copy_(obs); st["act"].copy_(act); st["rew"].copy_(rew); st["next_obs"].copy_(next_obs); st["done"].copy_(done)
             st["eps_pi"].normal_(generator=generator); st["eps_next"].normal_(generator=generator)
             g1.replay()
@@ -468,8 +472,8 @@ class SACTrainer:
         self.buffer = ReplayBuffer(cfg.buffer_size, env.num_envs, env.obs_dim, 4, self.dev)
         self.obs = env.reset().clone()
         self.total_steps = 0
-        self.collect_graph = bool(cfg.cuda_graph)
-        self._collect_graph, self._collect_warm = None, False
+        self.collect_graph = bool(cfg.cuda_graph)           # replay the sampled phases of the fused collection from a CUDA graph
+        self._collect_phase = PhaseGraph()                  # that graph, keyed by the phase length
         if cfg.rollout_impl == "fused":
             from . import _lib as L
             self.fused = self.learner.ensure_fused_actor(env.num_envs)
@@ -502,26 +506,26 @@ class SACTrainer:
 
     def _collect_step(self, mode: int):
         """One env step of a fused phase: dn_sac_act on the current observation, env.step, the replay write at the device-side
-        slot (ReplayBuffer.add's arithmetic with torch ops), slot + 1.  Nothing here waits for the host."""
-        env, buf, s = self.env, self.buffer, self.slot
+        slot, slot + 1.  Nothing here waits for the host."""
+        env, buf = self.env, self.buffer
         self.fused.act(self.obs, self.samplers[mode], self.action)
         env.step(self.action)
-        buf.obs.index_copy_(0, s, self.obs.unsqueeze(0))
-        buf.next_obs.index_copy_(0, s, torch.where((env.done != 0).unsqueeze(-1), env.terminal_obs, env.obs).unsqueeze(0))
-        buf.act.index_copy_(0, s, self.action.unsqueeze(0))
-        buf.rew.index_copy_(0, s, env.reward.unsqueeze(0))
-        buf.done.index_copy_(0, s, ((env.done & 1) != 0).to(torch.float32).unsqueeze(0))
-        s.add_(1).remainder_(buf.cap)
+        buf.write(self.slot, self.obs, env.obs, self.action, env.reward, env.done, env.terminal_obs)
+        self.slot.add_(1).remainder_(buf.cap)
         self.obs.copy_(env.obs)
 
-    def _collect_fused(self, n_steps: int, graph: Optional[bool] = None):
+    @property
+    def _collect_graph(self) -> Optional[torch.cuda.CUDAGraph]:
+        """The captured graph of the fused collection (None until one was captured)."""
+        return self._collect_phase.graph
+
+    def _collect_fused(self, n_steps: int):
         """collect() on dn_sac_act.  A phase with a step before learning_starts runs launch by launch (uniform actions for those
         steps, as SB3's action_space.sample()).  Every later phase is ONE CUDA graph -- weight refresh, then n_steps x (act,
         env.step, replay write) -- captured at the second such phase (the first, launched, loads every kernel) and replayed from
         then on.  The host keeps ReplayBuffer.pos / full by arithmetic; the slot tensor is set from pos before every phase."""
         from . import _lib as L
         cfg, buf = self.cfg, self.buffer
-        graph = self.collect_graph if graph is None else graph
         per_step = self.env.num_envs * _world()
         self.slot.fill_(buf.pos)
         if self.total_steps < cfg.learning_starts:
@@ -529,22 +533,11 @@ class SACTrainer:
             for k in range(n_steps):
                 self._collect_step(L.DN_SAC_UNIFORM if self.total_steps + k * per_step < cfg.learning_starts else L.DN_SAC_SAMPLE)
         else:
-            g = self._collect_graph
-            if graph and g is not None and g[0] == n_steps:
-                g[1].replay()
-            elif graph and self._collect_warm:
-                cg = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(cg):
-                    self.fused.sync_weights()
-                    for _ in range(n_steps):
-                        self._collect_step(L.DN_SAC_SAMPLE)
-                self._collect_graph = (n_steps, cg)
-                cg.replay()
-            else:
+            def phase():
                 self.fused.sync_weights()
                 for _ in range(n_steps):
                     self._collect_step(L.DN_SAC_SAMPLE)
-                self._collect_warm = True
+            self._collect_phase.run(self.collect_graph, n_steps, phase)
         for _ in range(n_steps):
             buf.pos = (buf.pos + 1) % buf.cap
             buf.full = buf.full or buf.pos == 0

@@ -172,6 +172,81 @@ def test_sac_update_cuda_graph_equals_eager():
     torch.testing.assert_close(res[True][2], res[False][2], rtol=1e-3, atol=1e-5)
 
 
+def test_ppo_update_graphs_follow_an_optimizer_load():
+    """A graphed learner that has already captured its minibatch step loads another learner's parameters and Adam state:
+    load_state_dict re-creates the state tensors the graphs pointed to, so the next update must capture again and take the
+    steps an eager learner takes from the same state (the tolerances of the graph-vs-eager test above)."""
+    import copy
+    from drl_dronenavigation_b200.ppo import PPOConfig, PPOLearner
+    g = torch.Generator(device="cuda").manual_seed(0)
+    B = 8192
+    obs, act = torch.randn(B, 13, device="cuda", generator=g), torch.rand(B, 4, device="cuda", generator=g) * 2 - 1
+    adv, ret = torch.randn(B, device="cuda", generator=g), torch.randn(B, device="cuda", generator=g)
+    cfg = lambda graph: PPOConfig(batch_size=1024, n_epochs=3, target_kl=None, cuda_graph=graph, matmul_precision="fp32", update_impl="torch")
+    src = PPOLearner(13, 4, cfg(False), device="cuda")
+    with torch.no_grad():
+        v, logp, _ = src.policy.evaluate(obs, act)
+    src.update(obs, act, logp, v, adv, ret, generator=torch.Generator(device="cuda").manual_seed(1))
+    state = src.opt.state_dict()["state"]
+    res = {}
+    for graph in (False, True):
+        L = PPOLearner(13, 4, cfg(graph), device="cuda")
+        if graph:
+            L.update(obs, act, logp, v, adv, ret, generator=torch.Generator(device="cuda").manual_seed(2))     # captured
+        L.policy.load_state_dict(src.policy.state_dict())
+        L.load_optimizer_state(copy.deepcopy(state))
+        p0 = L.flat_parameters().clone()
+        r = L.update(obs, act, logp, v, adv, ret, generator=torch.Generator(device="cuda").manual_seed(3))
+        res[graph] = (p0, L.flat_parameters().clone(), r, float(L.opt.state[L.params[0]]["step"]))
+    assert torch.equal(res[False][0], res[True][0])
+    assert res[True][3] == res[False][3] == 48.0                      # 24 loaded steps + 24 taken on the loaded state
+    d = (res[True][1] - res[False][1]).abs()
+    moved = (res[False][1] - res[False][0]).abs()
+    print("graph-vs-eager after a load: max", float(d.max()), "mean", float(d.mean()), "mean movement", float(moved.mean()))
+    assert float(d.mean()) < 0.02 * float(moved.mean()) and float(d.max()) < 2e-3
+    for k in ("policy_gradient_loss", "value_loss", "approx_kl", "clip_fraction"):
+        assert abs(res[True][2][k] - res[False][2][k]) < 1e-3, k
+
+
+def test_sac_update_graphs_follow_an_archive_load(tmp_path):
+    """A graphed SAC learner that has already captured its gradient step loads an SB3 archive with its optimisers; its next steps
+    must be those of an eager learner loaded from the same archive (the tolerances of the graph-vs-eager test above)."""
+    from drl_dronenavigation_b200.checkpoint import load_sb3_zip, save_sb3_sac_zip
+    from drl_dronenavigation_b200.sac import SACConfig, SACLearner
+    g = torch.Generator(device="cuda").manual_seed(0)
+    B = 1024
+    batches = [(torch.randn(B, 13, device="cuda", generator=g), torch.rand(B, 4, device="cuda", generator=g) * 2 - 1,
+                torch.randn(B, device="cuda", generator=g), torch.randn(B, 13, device="cuda", generator=g),
+                (torch.rand(B, device="cuda", generator=g) < 0.1).float()) for _ in range(6)]
+    gen = lambda k: torch.Generator(device="cuda").manual_seed(10 + k)
+    src = SACLearner(13, 4, SACConfig(cuda_graph=False, matmul_precision="fp32", seed=7), device="cuda")
+    for k, b in enumerate(batches[:5]):
+        src.update(b, generator=gen(k))
+    path = save_sb3_sac_zip(str(tmp_path / "src.zip"), src)
+    res = {}
+    for graph in (False, True):
+        L = SACLearner(13, 4, SACConfig(cuda_graph=graph, matmul_precision="fp32"), device="cuda")
+        if graph:
+            for k, b in enumerate(batches[:2]):                      # captured
+                L.update(b, generator=gen(20 + k))
+        load_sb3_zip(path, L, load_optimizer=True)
+        p0 = L.flat_parameters().clone()
+        outs = [L.update(b, generator=gen(30 + k)) for k, b in enumerate(batches[2:])]
+        tgt = torch.cat([p.reshape(-1) for p in L.critic_target.parameters()])
+        steps = [float(o.state[p]["step"]) for o in (L.actor_opt, L.critic_opt, L.ent_opt) for p in o.state]
+        res[graph] = (p0, L.flat_parameters().clone(), tgt.clone(), [{k: float(v) for k, v in o.items()} for o in outs], steps)
+    assert torch.equal(res[False][0], res[True][0])
+    assert res[True][4] == res[False][4] == [9.0] * len(res[False][4])    # 5 loaded steps + 4 taken on the loaded state
+    for a, b in zip(res[True][3], res[False][3]):
+        for k in ("critic_loss", "actor_loss", "ent_coef", "ent_coef_loss"):
+            assert abs(a[k] - b[k]) <= 1e-3 * max(1.0, abs(b[k])), (k, a[k], b[k])
+    moved = (res[False][1] - res[False][0]).abs().mean()
+    d = (res[True][1] - res[False][1]).abs()
+    print("sac graph-vs-eager after a load: max", float(d.max()), "mean", float(d.mean()), "mean movement", float(moved))
+    assert float(d.mean()) < 0.02 * float(moved) and float(d.max()) < 2e-3
+    torch.testing.assert_close(res[True][2], res[False][2], rtol=1e-3, atol=1e-5)
+
+
 def test_fast_linear_matches_nn_linear():
     """FastLinear (GEMV bias gradient, input width padded to a multiple of 8) against plain nn.Linear in FP32: same
     outputs and the same gradients for input, weight and bias, for the first-layer (13 -> 512) and a square layer."""
